@@ -2,6 +2,10 @@
 """bench.py — CoPER-ConvE hot-path throughput on B200 (contract: see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--shape S] [--prec P] [--impl ours|reference]
+                    [--dump-outputs DIR]
+
+Every GPU workload block times exactly K steps after max(W, 3) warm-up steps (the first two calls of a step run eager and
+capture its CUDA graph).
 
 A "step" = one full training step of the hot path over one synthetic batch of B (e1, rel) queries with
 1-N labels: lookups -> conv -> fused CPG-FC -> 1-N scorer + label-smoothed BCE -> backward -> global-norm
@@ -192,13 +196,13 @@ def reference_arm(args, shape, B, scaling, workload):
     """`--impl reference`: the reference's CPU implementation of the path (oracle port, kind "port") on all host cores,
     exactly W warm-up + K timed steps, on the configuration our own arm labels.  Shapes whose dense fp32 [B, N] labels
     and logits do not fit a bounded CPU step (synth-10m: 2 x 20 GB per step) are timed on an entity SLICE and
-    extrapolated linearly in N (the scorer, loss, gradient and optimizer all stream N rows); the slice is stated."""
+    extrapolated linearly in N (the scorer, loss, gradient and optimizer all stream N rows); the slice is stated.
+    --steps sets the timed train steps only: the eval batches (2 to 8) and the small slice's train steps (K // 2, at
+    least 2) are counts of their own, stated in `sample`."""
     from coper_b200 import synthetic
     s = synthetic.SHAPES[shape]
     N = s["num_ent"]
     K, W = args.steps, args.warmup
-    if shape == "toy":
-        K, W = min(K, 3), min(W, 1)
     slice_n = None
     if N > 400_000:
         slice_n = 1 << 18                                  # 262 144 rows: ~1 s per CPU step
@@ -285,10 +289,35 @@ def working_set_mb(s, B):
     return int((3 * N * d * 4 + 3 * dr * F * d * 4 + B * N * 4 + 4 * B * F * 4) / 1e6)
 
 
+DUMP_MAX_ELEMS = 1 << 19       # per array: larger outputs are dumped as a fixed, seeded sample of this many elements
+
+
+def host_output(t):
+    """A device output as float32 (float64 stays float64; integers become exact float64), sampled if large."""
+    import torch
+    t = t.detach()
+    if t.numel() > DUMP_MAX_ELEMS:
+        idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_MAX_ELEMS))
+        t = t.reshape(-1)[torch.as_tensor(idx, device=t.device)]
+    a = t.cpu().numpy()
+    return a.astype(np.float64 if a.dtype in (np.float64, np.int64, np.int32) else np.float32)
+
+
+def write_outputs(out_dir, outputs):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > 64 << 20:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the 64 MB cap" % total)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure(ctx, shape, prec, K, W, peaks, *, sharded=False, dp=False, e2e=True, breakdown=True, graphs_multi=True,
-            overlap=True):
+            overlap=True, outputs=None):
     """One workload: device-resident train / eval throughput, end-to-end numbers and the per-stage rooflines.
-    sharded=False builds a single-GPU model on this rank (no collectives) even inside a multi-rank job."""
+    sharded=False builds a single-GPU model on this rank (no collectives) even inside a multi-rank job.
+    outputs (a dict) receives, as host arrays, what the last timed train step and eval batch returned: the loss, the
+    model state after the update (variables, optimizer slots, batch-norm statistics) and the filtered ranks."""
     torch = ctx.torch
     from coper_b200 import synthetic
     from coper_b200.models import ConvE, EntityShard
@@ -305,8 +334,22 @@ def measure(ctx, shape, prec, K, W, peaks, *, sharded=False, dp=False, e2e=True,
     host = synthetic.make_batches(s["num_ent"], s["num_rel"], B, n_batches, seed=1)
     devb = [{k: torch.as_tensor(v).cuda() for k, v in hb.items()} for hb in host]
     coll = world > 1
-    train_ms, train_launches = ctx.timed(model, lambda i: model.train_step(devb[i % n_batches]), K, W, coll)
-    eval_ms, eval_launches = ctx.timed(model, lambda i: model.filtered_ranks(devb[i % n_batches]), K, W, coll)
+    last = {}
+
+    def train(i):
+        last["loss"] = model.train_step(devb[i % n_batches])
+
+    def evaluate(i):
+        last["rank"], last["n_equal"] = model.filtered_ranks(devb[i % n_batches])
+    train_ms, train_launches = ctx.timed(model, train, K, W, coll)
+    if outputs is not None:
+        outputs["train_loss"] = host_output(last["loss"])
+        for k, t in model.state_dict().items():
+            if k != "seed_dev":                  # a uint64 hash seed, not a computed value
+                outputs["state__" + k.replace("/", "__")] = host_output(t)
+    eval_ms, eval_launches = ctx.timed(model, evaluate, K, W, coll)
+    if outputs is not None:
+        outputs["eval_rank"], outputs["eval_n_equal"] = host_output(last["rank"]), host_output(last["n_equal"])
     nnz = float(np.mean([hb["e2_multi_col"].shape[0] for hb in host]))
     h2d = int(B * 8 * 2 + (B + 1) * 4 + nnz * 4)
     out = {
@@ -516,6 +559,11 @@ def main():
     ap.add_argument("--no-overlap", action="store_true",
                     help="data-parallel: all-reduce the whole gradient bucket at the end of the backward pass instead "
                          "of overlapping the generator-weight gradient with the conv backward")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the headline workload, write what its last train step and eval "
+                         "batch computed as DIR/<name>.npy (float32 / float64; arrays above %d elements as a fixed "
+                         "seeded sample; N > 1: rank 0's entity rows) so that two builds can be compared on the same "
+                         "inputs" % DUMP_MAX_ELEMS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -556,10 +604,13 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
+    outputs = {} if args.dump_outputs and rank == 0 else None
     head, model, host = measure(ctx, shape, prec, K, W, peaks, sharded=True, dp=dp, e2e=True,
                                 breakdown=not args.no_breakdown, graphs_multi=not args.no_graph_multi,
-                                overlap=not args.no_overlap)
+                                overlap=not args.no_overlap, outputs=outputs)
     clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     n_batches = len(host)
 
     alt = sampled = cpu = None
@@ -615,15 +666,14 @@ def main():
         model = None
         if extra:
             # ---- every other named configuration of BASELINE.json on one GPU (parity-tested at full size in tests/)
-            Kc, Wc = max(5, min(K, 10)), max(3, min(W, 5))
             for other in ("fb15k-237", "nell-995", "yago3-10", "synth-10m"):
                 if other == shape:
                     continue
                 try:
-                    blk, m_o, _ = measure(ctx, other, "bf16" if other == "synth-10m" else "fp16x3", Kc, Wc, peaks,
+                    blk, m_o, _ = measure(ctx, other, "bf16" if other == "synth-10m" else "fp16x3", K, W, peaks,
                                           e2e=True, breakdown=not args.no_breakdown)
                     blk.pop("_B")
-                    blk["steps"], blk["warmup"] = Kc, Wc
+                    blk["steps"], blk["warmup"] = K, W
                     configs[other] = blk
                     _free(ctx, m_o)
                 except Exception as exc:           # one failing extra block must not take the headline down
@@ -644,7 +694,6 @@ def main():
         _free(ctx, model)
         model = None
         if extra:
-            Kc, Wc = max(5, min(K, 10)), max(3, min(W, 5))
             # ---- the data-parallel WN18RR weak-scaling numbers (global batch N * 512), all ranks
             try:
                 weak, m_w, _ = measure(ctx, "wn18rr", "fp16x3", K, W, peaks, sharded=True, dp=True, e2e=True,
@@ -659,10 +708,10 @@ def main():
             torch.cuda.synchronize()
             if rank == 0:
                 try:
-                    base, m_b, _ = measure(ctx, shape, prec, Kc, Wc, peaks, sharded=False, e2e=False, breakdown=False)
+                    base, m_b, _ = measure(ctx, shape, prec, K, W, peaks, sharded=False, e2e=False, breakdown=False)
                     base = {"n_gpus": 1, "value": base["value"], "unit": base["unit"], "ms_per_step": base["ms_per_step"],
                             "eval_value": base["eval"]["value"], "eval_ms_per_batch": base["eval"]["ms_per_batch"],
-                            "steps": Kc, "warmup": Wc,
+                            "steps": K, "warmup": W,
                             "note": "same workload, single GPU, measured by rank 0 in this run; strong-scaling ratio = "
                                     "value / (n_gpus * strong_scaling_base.value)"}
                     _free(ctx, m_b)

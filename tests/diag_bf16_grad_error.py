@@ -3,7 +3,9 @@
 pattern (the bf16 forward flips units whose pre-activation lies within rounding of zero; each flip moves that element
 of dy by the full common part of dq, which dominates the max-norm error of (a)).
 Lives under tests/ because it uses the oracle (only tests/, smoke() and bench.py's CPU legs may)."""
-import sys; sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE)); sys.path.insert(0, HERE)
 import numpy as np, torch
 from oracle import conve_oracle as O
 import test_gpu_model as T
