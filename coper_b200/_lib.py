@@ -14,7 +14,6 @@ LIB_PATH = os.path.join(_HERE, "libcoper_sm100.so")
 PREC = {"fp32": 0, "bf16": 1, "tf32x3": 2, "fp16x3": 3}
 # flags of coper_cpg_fc_bwd (include/coper.h)
 CPG_BWD_REUSE_FWD, CPG_BWD_INPUT_GRADS_ONLY, CPG_BWD_WEIGHT_GRADS_ONLY, CPG_BWD_DCB_ACCUMULATE = 1, 2, 4, 8
-CPG_FWD_F_PREPARED = 1
 
 vp, i32, i64, u64, f32, sz = C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_float, C.c_size_t
 
@@ -25,7 +24,6 @@ SIGNATURES = {
     "coper_last_cuda_error": (i32, []),
     "coper_launch_count": (C.c_longlong, []),
     "coper_device_is_sm100": (i32, []),
-    "coper_set_sm_budget": (i32, [i32]),
     "coper_set_pdl": (i32, [i32]),
     "coper_gather_rows": (i32, [vp, i64, i64, i32, vp, i32, vp, vp]),
     "coper_gather_rows2": (i32, [vp, i64, i64, i32, vp, i32, vp, vp, i64, i64, i32, vp, i32, vp, vp, vp, f32, f32, f32, vp]),
@@ -40,8 +38,6 @@ SIGNATURES = {
     "coper_bn_stats_finalize": (i32, [vp, i64, i32, vp, vp, vp, vp, vp, vp, f32, f32, i32, i32, vp, vp, vp, vp, vp]),
     "coper_bn_act_fwd": (i32, [vp, i64, i32, vp, vp, i32, f32, vp, u64, vp, vp]),
     "coper_bn_act_fwd_moving": (i32, [vp, i64, i32, vp, vp, vp, vp, f32, i32, vp, vp]),
-    "coper_bn_act_fwd_prepared": (i32, [vp, i64, i32, vp, vp, i32, f32, vp, u64, vp, i64, i32, i32, vp, vp]),
-    "coper_bn_act_fwd_moving_prepared": (i32, [vp, i64, i32, vp, vp, vp, vp, f32, i32, vp, i64, i32, i32, vp, vp]),
     "coper_bn_act_bwd_stats": (i32, [vp, vp, i64, i32, vp, vp, vp, vp, i32, f32, vp, u64, vp, vp]),
     "coper_bn_act_bwd_stats_finalize": (i32, [vp, vp, i64, i32, vp, vp, vp, vp, i32, f32, vp, u64, vp, vp, i32, vp, vp, vp, vp,
                                               vp]),
@@ -51,7 +47,6 @@ SIGNATURES = {
     "coper_dropout_apply": (i32, [vp, i64, f32, vp, u64, vp]),
     "coper_cpg_fc_fwd_workspace_bytes": (sz, [i32, i32, i32, i32, i32]),
     "coper_cpg_fc_fwd": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, f32, vp, u64, vp, vp, sz, i32, vp]),
-    "coper_cpg_fc_fwd_ex": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, f32, vp, u64, vp, vp, sz, i32, i32, vp]),
     "coper_cpg_fc_bwd_workspace_bytes": (sz, [i32, i32, i32, i32, i32]),
     "coper_cpg_fc_bwd": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, sz, i32, i32,
                                vp]),

@@ -8,7 +8,6 @@ namespace coper {
 
 extern thread_local int g_last_cuda_error;
 extern long long g_launch_count;  // kernels launched by this library (every launch is followed by check_launch)
-extern thread_local int g_sm_budget;   // coper_set_sm_budget: grid cap of the persistent tcgen05 kernels (0 = all SMs)
 
 inline int check_launch() {
   ++g_launch_count;
@@ -42,7 +41,7 @@ static inline cudaStream_t as_stream(coper_stream_t s) { return reinterpret_cast
 // (griddepcontrol.wait), before touching any memory.  Correctness never depends on the attribute: without it (or after
 // a non-kernel stream operation, an event wait, a kernel of another library) both instructions are no-ops and the
 // launch is an ordinary one.  The tcgen05 kernels place the wait after their prologue (barrier init, TMEM allocation,
-// descriptor prefetch - nothing that reads a predecessor's output).  COPER_PDL=0 in the environment turns it off.
+// descriptor prefetch - nothing that reads a predecessor's output).  coper_set_pdl(0) turns it off.
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_enter() {

@@ -24,8 +24,7 @@ using namespace simt;
 size_t umma_cpg_fwd_workspace_bytes(int B, int dc, int F, int d, int prec);
 size_t umma_cpg_bwd_workspace_bytes(int B, int dc, int F, int d, int prec);
 int umma_cpg_fwd_partials(const float* c, const float* f, const float* P, const void* P_prepared, int B, int dc, int F,
-                          int d, void* ws, size_t ws_bytes, int prec, bool f_prepared, cudaStream_t st, float** slabs,
-                          int* n_slabs);
+                          int d, void* ws, size_t ws_bytes, int prec, cudaStream_t st, float** slabs, int* n_slabs);
 int umma_cpg_bwd(const float* c, const float* f, const float* P, const void* P_prepared, const float* dy, int B, int dc,
                  int F, int d, float* dP, float* df, float* dc_out, void* ws, size_t ws_bytes, int prec,
                  int flags, cudaStream_t st);
@@ -356,14 +355,6 @@ int coper_cpg_fc_fwd(const float* c, const float* f, const float* P, const void*
                      const float* Pb, int B, int dc, int F, int d, int dcb, float keep_out, const uint64_t* seed_dev,
                      uint64_t salt_out, float* y, void* workspace, size_t workspace_bytes, int prec,
                      coper_stream_t stream) {
-  return coper_cpg_fc_fwd_ex(c, f, P, P_prepared, cb, Pb, B, dc, F, d, dcb, keep_out, seed_dev, salt_out, y, workspace,
-                             workspace_bytes, prec, 0, stream);
-}
-
-int coper_cpg_fc_fwd_ex(const float* c, const float* f, const float* P, const void* P_prepared, const float* cb,
-                        const float* Pb, int B, int dc, int F, int d, int dcb, float keep_out, const uint64_t* seed_dev,
-                        uint64_t salt_out, float* y, void* workspace, size_t workspace_bytes, int prec, int flags,
-                        coper_stream_t stream) {
   COPER_CHECK_ARG(c && f && P && cb && Pb && y && workspace && B > 0 && dc > 0 && F > 0 && d > 0 && dcb > 0);
   COPER_CHECK_ARG(keep_out > 0.f);
   cudaStream_t st = as_stream(stream);
@@ -371,8 +362,7 @@ int coper_cpg_fc_fwd_ex(const float* c, const float* f, const float* P, const vo
   int n_slabs = 0;
   int rc;
   if (cpg_on_tensor_pipe(F, d, prec)) {
-    if ((rc = umma_cpg_fwd_partials(c, f, P, P_prepared, B, dc, F, d, workspace, workspace_bytes, prec,
-                                    (flags & COPER_CPG_FWD_F_PREPARED) != 0, st, &part, &n_slabs)))
+    if ((rc = umma_cpg_fwd_partials(c, f, P, P_prepared, B, dc, F, d, workspace, workspace_bytes, prec, st, &part, &n_slabs)))
       return rc;
   } else if (prec >= COPER_PREC_FP32 && prec <= COPER_PREC_FP16X3) {
     CpgLayout L = cpg_fwd_layout(B, dc, F, d);

@@ -3,22 +3,14 @@
 // 128-bit vectorised where the shape allows, grids sized in multiples of the SM count.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace coper {
 thread_local int g_last_cuda_error = 0;
 long long g_launch_count = 0;
-thread_local int g_sm_budget = 0;
-// programmatic dependent launch: on unless COPER_PDL=0 in the environment or switched off by coper_set_pdl
-static int g_pdl = -1;
-bool pdl_enabled() {
-  if (g_pdl < 0) {
-    const char* e = getenv("COPER_PDL");
-    g_pdl = (e && e[0] == '0') ? 0 : 1;
-  }
-  return g_pdl != 0;
-}
+// programmatic dependent launch: on unless switched off by coper_set_pdl
+static int g_pdl = 1;
+bool pdl_enabled() { return g_pdl != 0; }
 constexpr int kSMs = 148;
 
 // ------------------------------------------------------------------ gather (models.py:176,178)
@@ -996,13 +988,7 @@ const char* coper_status_string(int s) {
 int coper_last_cuda_error(void) { return g_last_cuda_error; }
 long long coper_launch_count(void) { return g_launch_count; }
 int coper_set_pdl(int on) {
-  const char* e = getenv("COPER_PDL");
-  g_pdl = (e && e[0] == '0') ? 0 : (on ? 1 : 0);      // the environment switch wins (measurements)
-  return COPER_OK;
-}
-int coper_set_sm_budget(int n_sms) {
-  COPER_CHECK_ARG(n_sms >= 0);
-  g_sm_budget = n_sms;
+  g_pdl = on ? 1 : 0;
   return COPER_OK;
 }
 int coper_device_is_sm100(void) {

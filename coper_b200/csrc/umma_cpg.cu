@@ -292,8 +292,7 @@ size_t umma_cpg_bwd_workspace_bytes(int B, int dc, int F, int d, int prec) {
 
 // Computes the split-K slabs of (c (x) f) . P^ into the workspace; *slabs / *n_slabs describe them.
 int umma_cpg_fwd_partials(const float* c, const float* f, const float* P, const void* P_prepared, int B, int dc, int F,
-                          int d, void* ws, size_t ws_bytes, int prec, bool f_prepared, cudaStream_t st, float** slabs,
-                          int* n_slabs) {
+                          int d, void* ws, size_t ws_bytes, int prec, cudaStream_t st, float** slabs, int* n_slabs) {
   if (F % 32 != 0 || d > 256) return COPER_ERR_UNSUPPORTED;
   CpgFwdPlan L = cpg_fwd_plan(B, dc, F, d, prec);
   if (!ws || ws_bytes < L.total) return COPER_ERR_WORKSPACE;
@@ -303,8 +302,7 @@ int umma_cpg_fwd_partials(const float* c, const float* f, const float* P, const 
   const void* Pp = P_prepared ? P_prepared : w + L.off_P;
   float* out = reinterpret_cast<float*>(w + L.off_slabs);
   int rc;
-  if (L.off_f != 0) return COPER_ERR_INVALID_ARG;            // COPER_CPG_FWD_F_PREPARED documents the operand at offset 0
-  if (!f_prepared && (rc = tc_prepare(f, B, F, F, prec, fp, st))) return rc;
+  if ((rc = tc_prepare(f, B, F, F, prec, fp, st))) return rc;
   if (!P_prepared && (rc = tc_prepare(P, (int64_t)dc * F, d, d, prec, w + L.off_P, st))) return rc;
   CpgFwdEpi epi;
   epi.c = c; epi.dc = dc; epi.out = out; epi.ld = d; epi.split_stride = (long long)B * d;

@@ -33,14 +33,6 @@ void umma_fused_plan(int B, int64_t Ns, int* QB, int* R);
 int umma_bce_dq_fused(const TcOperand& E, const TcOperand& Q, const float* bias, const uint32_t* bitsT, int B, int64_t Ns,
                       int d, float pos, float neg, float inv_count, void* GT, int64_t ldGT, float* dq_part,
                       float* dbias_part, double* loss_part, int* grid_out, cudaStream_t st);
-// COPER_FUSED_SCORER=0 selects the three-kernel schedule (A/B measurements); read once
-static bool fused_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("COPER_FUSED_SCORER");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
 
 constexpr int kEntEpiWarps = 16;
 constexpr int kBceEpiWarps = 16;   // the BCE epilogue is MUFU / latency bound: 4 warps per scheduler
@@ -600,7 +592,7 @@ static BceTcLayout bce_tc_layout(int B, int64_t Ns, int d, int prec) {
 size_t umma_bce_workspace_bytes(int B, int64_t Ns, int d, int prec) { return bce_tc_layout(B, Ns, d, prec).total; }
 // dbias slabs the scorer pass of these arguments writes: QB from the fused kernel, else one per query-block chunk row
 static int bce_dbias_slabs_used(const BceTcLayout& L, int B, int64_t Ns, int d, int prec) {
-  if (fused_enabled() && umma_fused_ok(B, Ns, d, prec)) {
+  if (umma_fused_ok(B, Ns, d, prec)) {
     int QB, R;
     umma_fused_plan(B, Ns, &QB, &R);
     return QB;
@@ -700,7 +692,7 @@ int umma_score1n_bce_fwd_bwd(const float* q, const float* E, const void* E_prepa
   if ((rc = tc_prepare(q, B, d, d, prec, qp, st))) return rc;
   if (!E_prepared && (rc = tc_prepare(E, Ns, d, d, prec, w + L.off_E, st))) return rc;
   TcOperand Qo = tc_operand(qp, B, d, prec), Eo = tc_operand(Ep, Ns, d, prec);
-  if (fused_enabled() && umma_fused_ok(B, Ns, d, prec)) {
+  if (umma_fused_ok(B, Ns, d, prec)) {
     // ---- single pass over E: scores -> loss, dbias, G (TMA store, entity-major) AND dq (G consumed from shared memory)
     int QB, R, grid = 0;
     umma_fused_plan(B, Ns, &QB, &R);

@@ -553,7 +553,6 @@ int launch_gemm(const TcOperand& A, const TcOperand& B, const GemmProblem& p, co
   long long supers = (long long)p.m_tiles * p.n_tiles * p.splits * (p.groups_inner ? 1 : p.groups);
   int grid = (int)(supers < sms ? supers : sms);
   if (grid_override > 0 && grid_override < grid) grid = grid_override;
-  if (g_sm_budget > 0 && g_sm_budget < grid) grid = g_sm_budget;      // coper_set_sm_budget (a second stream's share)
   if (grid < 1) return COPER_ERR_INVALID_ARG;
   launch_pdl(umma_gemm_kernel<Cfg, Epi>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, st, tA, tAlo, tB, tBlo, pp, epi);
   return check_launch();

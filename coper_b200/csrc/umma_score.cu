@@ -213,130 +213,6 @@ __global__ void __launch_bounds__(256) prepare_fp16x3_fused_kernel(const float* 
   }
 }
 
-// The activation that PRODUCES a per-batch operand (batch norm + relu + dropout of the conv feature map -> f; of the FC
-// output -> q) and its fp16x3 split in ONE launch: pass 1 writes the fp32 activation (the backward pass needs it) and
-// reduces max |.|, the grid barrier of prepare_fp16x3_fused_kernel, pass 2 re-reads what the same thread wrote and emits
-// the planes.  Same activation expressions as bn_act_fwd_kernel / bn_act_fwd_moving_kernel (elementwise.cu), same
-// exponent rule and rounding as prepare_fp16x3_fused_kernel -> same bits as the two launches it replaces.
-struct BnActSrc {
-  const float* x;
-  int C;                       // channels: channel of flat element e is e % C
-  const float* a;              // affine pair of coper_bn_finalize ... (training form)
-  const float* b;
-  const float* gamma;          // ... or, with a == NULL, the moving-statistics form of coper_bn_act_fwd_moving
-  const float* beta;
-  const float* moving_mean;
-  const float* moving_var;
-  float eps;
-  int relu;
-  float keep, inv_keep;
-  uint32_t thr;
-  const uint64_t* seed_dev;
-  uint64_t salt;
-  float* out;
-};
-__device__ __forceinline__ void bn_act_affine(const BnActSrc& A, int ch, float& ac, float& bc) {
-  if (A.a) {
-    ac = __ldg(A.a + ch);
-    bc = __ldg(A.b + ch);
-  } else {
-    const float inv = 1.0f / sqrtf(__ldg(A.moving_var + ch) + A.eps);
-    ac = __ldg(A.gamma + ch) * inv;
-    bc = __ldg(A.beta + ch) - __ldg(A.moving_mean + ch) * ac;
-  }
-}
-__global__ void __launch_bounds__(256) bn_act_prepare_fp16x3_kernel(BnActSrc A, int64_t rows, int cols,
-                                                                    __half* __restrict__ dst, int64_t ldp,
-                                                                    uint32_t* __restrict__ trailer) {
-  pdl_enter();
-  __shared__ float wmax[8];
-  const uint64_t seed = (A.seed_dev ? *A.seed_dev : 0ull) + A.salt;
-  const int gpr = (int)(ldp / 8);
-  const int64_t units = rows * gpr;
-  // 8 adjacent columns of a row are 8 adjacent channels, read / written as float4 pairs
-  const bool vec = ((cols & 7) == 0) && ((A.C & 7) == 0) &&
-                   (((reinterpret_cast<uintptr_t>(A.x) | reinterpret_cast<uintptr_t>(A.out)) & 15) == 0);
-  float m = 0.f;
-  for (int64_t u = (int64_t)blockIdx.x * 256 + threadIdx.x; u < units; u += (int64_t)gridDim.x * 256) {
-    const int64_t r = u / gpr;
-    const int c0 = (int)(u - r * gpr) * 8;
-    if (c0 >= cols) continue;
-    const int64_t e0 = r * cols + c0;
-    float v[8];
-    if (vec) {
-      const float4 x0 = __ldg(reinterpret_cast<const float4*>(A.x + e0)), x1 = __ldg(reinterpret_cast<const float4*>(A.x + e0) + 1);
-      const float xs[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
-      const int ch0 = (int)(e0 % A.C);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        float ac, bc;
-        bn_act_affine(A, ch0 + k, ac, bc);
-        float t = fmaf(ac, xs[k], bc);
-        if (A.relu) t = fmaxf(t, 0.f);
-        if (A.keep < 1.0f) t *= drop_factor(A.keep, A.inv_keep, A.thr, seed, (uint64_t)(e0 + k));
-        v[k] = t;
-        m = fmaxf(m, fabsf(t));
-      }
-      *reinterpret_cast<float4*>(A.out + e0) = make_float4(v[0], v[1], v[2], v[3]);
-      *(reinterpret_cast<float4*>(A.out + e0) + 1) = make_float4(v[4], v[5], v[6], v[7]);
-    } else {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        if (c0 + k >= cols) break;
-        float ac, bc;
-        bn_act_affine(A, (int)((e0 + k) % A.C), ac, bc);
-        float t = fmaf(ac, A.x[e0 + k], bc);
-        if (A.relu) t = fmaxf(t, 0.f);
-        if (A.keep < 1.0f) t *= drop_factor(A.keep, A.inv_keep, A.thr, seed, (uint64_t)(e0 + k));
-        A.out[e0 + k] = t;
-        m = fmaxf(m, fabsf(t));
-      }
-    }
-  }
-  m = warp_max(m);
-  if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = m;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int w = 1; w < 8; ++w) m = fmaxf(m, wmax[w]);
-    if (m > 0.f) atomicMax(trailer + 1, __float_as_uint(m));
-    __threadfence();
-    atomicAdd(trailer + 3, 1u);
-    const long long t0 = clock64();
-    while (*reinterpret_cast<volatile uint32_t*>(trailer + 3) < gridDim.x) {
-      if (clock64() - t0 > 4000000000ll) __trap();
-    }
-    __threadfence();
-  }
-  __syncthreads();
-  const uint32_t mbits = *reinterpret_cast<volatile uint32_t*>(trailer + 1);
-  const int e = fp16x3_exponent(mbits);
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    reinterpret_cast<int*>(trailer)[0] = e;
-    trailer[2] = mbits;
-  }
-  const float sc = exp2f((float)e);
-  __half* lo_plane = dst + rows * ldp;
-  for (int64_t u = (int64_t)blockIdx.x * 256 + threadIdx.x; u < units; u += (int64_t)gridDim.x * 256) {
-    const int64_t r = u / gpr;
-    const int c0 = (int)(u - r * gpr) * 8;
-    const int64_t e0 = r * cols + c0;
-    float x[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) x[k] = (c0 + k < cols) ? A.out[e0 + k] : 0.f;     // this thread's own stores of pass 1
-    __half2 h[4], l[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const float a = x[2 * k] * sc, b = x[2 * k + 1] * sc;
-      h[k] = __floats2half2_rn(a, b);
-      const float2 hf = __half22float2(h[k]);
-      l[k] = __floats2half2_rn(a - hf.x, b - hf.y);
-    }
-    *reinterpret_cast<uint4*>(dst + u * 8) = *reinterpret_cast<uint4*>(h);
-    *reinterpret_cast<uint4*>(lo_plane + u * 8) = *reinterpret_cast<uint4*>(l);
-  }
-}
-
 // entity-major scorer kernels: umma_entity.cu
 int umma_score1n_fwd_prepared(const void* q_prep, const void* E_prep, const float* bias, int B, int64_t Ns, int d,
                               float* scores, int64_t ld, int prec, cudaStream_t st);
@@ -420,51 +296,6 @@ int coper_prepare_operand(const float* src, int64_t rows, int cols, int64_t ld_s
   COPER_CHECK_ARG(src && dst && rows > 0 && cols > 0 && ld_src >= cols);
   COPER_CHECK_ARG((reinterpret_cast<uintptr_t>(dst) & 15) == 0);
   return prepare(src, rows, cols, ld_src, prec, dst, as_stream(stream));
-}
-static int bn_act_prepared(const BnActSrc& A, int64_t R, int64_t op_rows, int op_cols, int prec, void* prepared,
-                           cudaStream_t st) {
-  if (prec == COPER_PREC_FP16X3 && op_rows * op_cols <= ((int64_t)4 << 20)) {
-    const int64_t ldp = prepared_ld(op_cols, prec);
-    uint32_t* trailer = static_cast<uint32_t*>(tc_fp16x3_trailer(prepared, op_rows, op_cols));
-    int rc = check_cuda(cudaMemsetAsync(trailer, 0, 16, st));
-    if (rc) return rc;
-    const int64_t want = (op_rows * (ldp / 8) + 256 * 4 - 1) / (256 * 4);
-    int g = (int)(want < (int64_t)sm_count() * 2 ? want : (int64_t)sm_count() * 2);
-    if (g < 1) g = 1;
-    launch_pdl(bn_act_prepare_fp16x3_kernel, g, 256, 0, st, A, op_rows, op_cols, static_cast<__half*>(prepared), ldp, trailer);
-    return check_launch();
-  }
-  // other precisions / operands too large for the co-resident grid: the two launches
-  int rc;
-  if (A.a)
-    rc = coper_bn_act_fwd(A.x, R, A.C, A.a, A.b, A.relu, A.keep, A.seed_dev, A.salt, A.out, (coper_stream_t)st);
-  else
-    rc = coper_bn_act_fwd_moving(A.x, R, A.C, A.gamma, A.beta, A.moving_mean, A.moving_var, A.eps, A.relu, A.out,
-                                 (coper_stream_t)st);
-  if (rc) return rc;
-  return prepare(A.out, op_rows, op_cols, op_cols, prec, prepared, st);
-}
-int coper_bn_act_fwd_prepared(const float* x, int64_t R, int C, const float* a, const float* b, int relu, float keep_post,
-                              const uint64_t* seed_dev, uint64_t salt_post, float* out, int64_t op_rows, int op_cols,
-                              int prec, void* prepared, coper_stream_t stream) {
-  COPER_CHECK_ARG(x && a && b && out && prepared && R > 0 && C > 0 && keep_post > 0.f);
-  COPER_CHECK_ARG(op_rows > 0 && op_cols > 0 && op_rows * op_cols == R * C);
-  COPER_CHECK_ARG((reinterpret_cast<uintptr_t>(prepared) & 15) == 0);
-  if (prec != COPER_PREC_BF16 && prec != COPER_PREC_TF32X3 && prec != COPER_PREC_FP16X3) return COPER_ERR_UNSUPPORTED;
-  BnActSrc A{x, C, a, b, nullptr, nullptr, nullptr, nullptr, 0.f, relu, keep_post, 1.0f / keep_post,
-             keep_threshold(keep_post), seed_dev, salt_post, out};
-  return bn_act_prepared(A, R, op_rows, op_cols, prec, prepared, as_stream(stream));
-}
-int coper_bn_act_fwd_moving_prepared(const float* x, int64_t R, int C, const float* gamma, const float* beta,
-                                     const float* moving_mean, const float* moving_var, float eps, int relu, float* out,
-                                     int64_t op_rows, int op_cols, int prec, void* prepared, coper_stream_t stream) {
-  COPER_CHECK_ARG(x && gamma && beta && moving_mean && moving_var && out && prepared && R > 0 && C > 0);
-  COPER_CHECK_ARG(op_rows > 0 && op_cols > 0 && op_rows * op_cols == R * C);
-  COPER_CHECK_ARG((reinterpret_cast<uintptr_t>(prepared) & 15) == 0);
-  if (prec != COPER_PREC_BF16 && prec != COPER_PREC_TF32X3 && prec != COPER_PREC_FP16X3) return COPER_ERR_UNSUPPORTED;
-  BnActSrc A{x, C, nullptr, nullptr, gamma, beta, moving_mean, moving_var, eps, relu, 1.0f, 1.0f, 0xFFFFFFFFu, nullptr, 0,
-             out};
-  return bn_act_prepared(A, R, op_rows, op_cols, prec, prepared, as_stream(stream));
 }
 int coper_score1n_fwd_prepared(const void* q_prep, const void* E_prep, const float* bias, int B, int64_t Ns, int d,
                                float* scores, int64_t ld_scores, int prec, coper_stream_t stream) {

@@ -30,15 +30,14 @@ one fused kernel).
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional
 
 import numpy as np
 import torch
 
 from . import _lib, sharding
-from ._lib import (CPG_BWD_DCB_ACCUMULATE, CPG_BWD_INPUT_GRADS_ONLY, CPG_BWD_REUSE_FWD, CPG_BWD_WEIGHT_GRADS_ONLY,
-                   CPG_FWD_F_PREPARED, PREC, call, call_plain, ptr)
+from ._lib import (CPG_BWD_DCB_ACCUMULATE, CPG_BWD_INPUT_GRADS_ONLY, CPG_BWD_REUSE_FWD, CPG_BWD_WEIGHT_GRADS_ONLY, PREC,
+                   call, call_plain, ptr)
 from .sharding import EntityShard
 
 BN_EPS = 1e-3           # tf.layers.batch_normalization default epsilon (models.py:386-388)
@@ -97,7 +96,7 @@ class ConvE:
                  shard: Optional[EntityShard] = None, reference_bug_compat: bool = True,
                  conv_in_height: int = 10, process_group=None, use_graphs: bool = True,
                  init_fast: bool = False, graphs_multi_gpu: bool = False, data_parallel: bool = False,
-                 overlap_grad_allreduce: bool = True, overlap_entity_grad: bool = True):
+                 overlap_grad_allreduce: bool = True):
         md = model_descriptors
         _lib.load()
         if not torch.cuda.is_available():
@@ -185,20 +184,11 @@ class ConvE:
         # the entity-gradient GEMM dE = G^T.q (HBM-bound) depends on nothing the rest of the backward pass produces and
         # nothing there depends on it until the head-entity scatter: it is enqueued on a second stream and runs under
         # the latency-bound FC / CPG / conv backward chain (fork / join are captured into the step's CUDA graph)
-        self.overlap_entity_grad = bool(overlap_entity_grad)
         self._side = torch.cuda.Stream(device=self.dev)
         self._side_pending = False
-        self._split_cpg_bwd = os.environ.get("COPER_SPLIT_CPG_BWD", "1") != "0"      # (A/B switch for measurements)
         # programmatic dependent launch pays on the launch-bound steps of the named datasets and costs on the HBM-bound
         # step of a 10 M-row table (DESIGN 4.6): per model, by the size of the entity table
         self._pdl = int(self.shard.rows) * int(self.ent_emb_size) <= (64 << 20)
-        # (A/B switches for measurements, DESIGN 4.6) activation + operand form in one launch: measured SLOWER than the two
-        # launches at the dataset shapes (the co-resident grid of its barrier caps the parallelism over the 9 MB feature
-        # map) - off unless asked for; Conv1BN backward inside the conv backward: on
-        self._fuse_act_prepare = os.environ.get("COPER_FUSE_ACT_PREPARE", "0") == "1"
-        self._fold_conv_bn = os.environ.get("COPER_FOLD_CONV_BN", "1") != "0"
-        # SMs the side stream's persistent GEMMs may take (coper_set_sm_budget; 0 = all)
-        self._side_sms = int(os.environ.get("COPER_SIDE_SMS", "0"))
         # CUDA graphs: the device side of a train / eval step is a fixed kernel sequence over pointer-stable buffers
         # (step counter, dropout seed and clip scale live in device memory), so it is captured once per batch size
         # and replayed with one launch.  The sharded path captures its NCCL collectives into the same graph
@@ -700,34 +690,20 @@ class ConvE:
         return b
 
     # ------------------------------------------------------------------------------------------
-    def _bn_forward(self, bn: _BatchNorm, x, R, C, b, use_batch, is_train, bessel, relu, keep_post, salt, out,
-                    prepared=None):
-        """prepared = (device pointer, rows, cols): also emit the tensor-pipe operand form of `out` viewed [rows, cols]
-        (the activation and coper_prepare_operand in one launch)."""
+    def _bn_forward(self, bn: _BatchNorm, x, R, C, b, use_batch, is_train, bessel, relu, keep_post, salt, out):
         lib = _lib.load()
         nch = 0
         stat, Rt = b.stat, R
-
-        def act():
-            if prepared is None:
-                call("coper_bn_act_fwd", ptr(x), R, C, ptr(bn.a), ptr(bn.b), int(relu), keep_post, ptr(self.seed_dev),
-                     salt, ptr(out))
-            else:
-                call("coper_bn_act_fwd_prepared", ptr(x), R, C, ptr(bn.a), ptr(bn.b), int(relu), keep_post,
-                     ptr(self.seed_dev), salt, ptr(out), prepared[1], prepared[2], self.prec, prepared[0])
-
         if use_batch and not self.dp:        # statistics + finalize: one launch (the last block to arrive finalises)
             call("coper_bn_stats_finalize", ptr(x), R, C, ptr(b.stat), ptr(self.sync_word), ptr(bn.gamma), ptr(bn.beta),
                  ptr(bn.moving_mean), ptr(bn.moving_var), self.batch_norm_momentum, BN_EPS, int(is_train), int(bessel),
                  ptr(bn.a), ptr(bn.b), ptr(bn.mean), ptr(bn.invstd))
-            return act()
+            call("coper_bn_act_fwd", ptr(x), R, C, ptr(bn.a), ptr(bn.b), int(relu), keep_post, ptr(self.seed_dev), salt,
+                 ptr(out))
+            return
         if not use_batch and not is_train and keep_post >= 1.0:      # inference: moving statistics, one launch
-            if prepared is None:
-                call("coper_bn_act_fwd_moving", ptr(x), R, C, ptr(bn.gamma), ptr(bn.beta), ptr(bn.moving_mean),
-                     ptr(bn.moving_var), BN_EPS, int(relu), ptr(out))
-            else:
-                call("coper_bn_act_fwd_moving_prepared", ptr(x), R, C, ptr(bn.gamma), ptr(bn.beta), ptr(bn.moving_mean),
-                     ptr(bn.moving_var), BN_EPS, int(relu), ptr(out), prepared[1], prepared[2], self.prec, prepared[0])
+            call("coper_bn_act_fwd_moving", ptr(x), R, C, ptr(bn.gamma), ptr(bn.beta), ptr(bn.moving_mean),
+                 ptr(bn.moving_var), BN_EPS, int(relu), ptr(out))
             return
         if use_batch:
             nch = lib.coper_colstats_chunks(R)
@@ -737,7 +713,8 @@ class ConvE:
         call("coper_bn_finalize", ptr(stat), nch, Rt, C, ptr(bn.gamma), ptr(bn.beta), ptr(bn.moving_mean),
              ptr(bn.moving_var), self.batch_norm_momentum, BN_EPS, int(use_batch), int(use_batch and is_train),
              int(bessel), ptr(bn.a), ptr(bn.b), ptr(bn.mean), ptr(bn.invstd))
-        act()
+        call("coper_bn_act_fwd", ptr(x), R, C, ptr(bn.a), ptr(bn.b), int(relu), keep_post, ptr(self.seed_dev), salt,
+             ptr(out))
 
     def _bn_backward(self, bn: _BatchNorm, dout, x, R, C, b, use_batch, relu, keep_post, salt_post, keep_pre,
                      salt_pre, dx, apply=True):
@@ -759,10 +736,6 @@ class ConvE:
         if apply:
             call("coper_bn_act_bwd_apply", ptr(dout), ptr(x), R, C, ptr(bn.a), ptr(bn.b), ptr(bn.mean), ptr(bn.invstd),
                  ptr(bn.c1), ptr(bn.c2), int(relu), keep_post, ptr(self.seed_dev), salt_post, keep_pre, salt_pre, ptr(dx))
-
-    def _side_budget(self, on: bool):
-        if self._side_sms > 0:
-            call_plain("coper_set_sm_budget", self._side_sms if on else 0)
 
     def _gather_stats(self, b, n):
         if getattr(b, "stat_all", None) is None:
@@ -840,9 +813,9 @@ class ConvE:
              ptr(self.step_state) if advance else None, ptr(self.seed_dev) if advance else None,
              self.learning_rate, self.beta1, self.beta2)
         sharding.exchange_rows(b.x0, self.world, self.group)
-        self._front_end(b, is_train, gather_rel=False, prepare_q=True)
+        self._front_end(b, is_train, gather_rel=False)
 
-    def _front_end(self, b, is_train: bool, gather_rel: bool = True, prepare_q: bool = False):
+    def _front_end(self, b, is_train: bool, gather_rel: bool = True):
         """b.x0, b.rel -> b.q for the rows of buffer set b (conv block, fused CPG-FC, FC block)."""
         B, d, dr, F, C = b.B, self.ent_emb_size, self.rel_emb_size, self.F, self.C
         x_img = b.x0
@@ -869,12 +842,8 @@ class ConvE:
                  self.conv_filter_height, self.conv_filter_width, C, 1, ptr(b.z))
         use_batch = self.batch_norm_train_stats and is_train
         keep1 = 1.0 - (self.hidden_dropout if is_train else 0.0)
-        # fp16x3: the activation that produces f also writes f's operand form where coper_cpg_fc_fwd expects it (the
-        # start of its workspace) - one launch instead of two
-        f_prep = (self._fuse_act_prepare and self.prec == PREC["fp16x3"] and not self.concat_rel and F % 32 == 0
-                  and d <= 256)
         self._bn_forward(self.conv1_bn, b.z, B * self.OH * self.OW, C, b, use_batch, is_train, True, True, keep1,
-                         SALT_FEATURE_MAP, b.fconv, prepared=(ptr(b.ws_cpg), B, F) if f_prep else None)
+                         SALT_FEATURE_MAP, b.fconv)
         if self.concat_rel:                  # tf.concat([fc_input, rel_emb], axis=1)  (models.py:406-407)
             b.f[:, :self.F_conv].copy_(b.fconv)
             b.f[:, self.F_conv:].copy_(b.r)
@@ -885,15 +854,9 @@ class ConvE:
             cw = cb = b.cconst
         Pw, Pb = self.fc_weights.projections[-1], self.fc_bias.projections[-1]
         keep2 = 1.0 - (self.output_dropout if is_train else 0.0)
-        call("coper_cpg_fc_fwd_ex", ptr(cw), ptr(b.f), ptr(Pw), ptr(self.P_prep), ptr(cb), ptr(Pb), B, Pw.shape[0], F, d,
-             Pb.shape[0], keep2, ptr(self.seed_dev), SALT_OUTPUT, ptr(b.y), ptr(b.ws_cpg), b.ws_cpg_bytes, self.prec,
-             CPG_FWD_F_PREPARED if f_prep else 0)
-        # evaluation on the tensor-pipe scorer: q's operand form comes out of the same launch as q
-        q_prep = (self._fuse_act_prepare and prepare_q and not is_train and self.prec == PREC["fp16x3"]
-                  and b.q_prep is not None)
-        self._bn_forward(self.fc_bn, b.y, B, d, b, use_batch, is_train, False, True, 1.0, 0, b.q,
-                         prepared=(ptr(b.q_prep), B, d) if q_prep else None)
-        b.q_prepared = bool(q_prep)
+        call("coper_cpg_fc_fwd", ptr(cw), ptr(b.f), ptr(Pw), ptr(self.P_prep), ptr(cb), ptr(Pb), B, Pw.shape[0], F, d,
+             Pb.shape[0], keep2, ptr(self.seed_dev), SALT_OUTPUT, ptr(b.y), ptr(b.ws_cpg), b.ws_cpg_bytes, self.prec)
+        self._bn_forward(self.fc_bn, b.y, B, d, b, use_batch, is_train, False, True, 1.0, 0, b.q)
         b.cw, b.cb = cw, cb
 
     def _forward_q_dp(self, bg, bl, is_train: bool):
@@ -936,27 +899,22 @@ class ConvE:
         if self.use_negative_sampling:
             self._sampled_scorer(b)
         elif self._norm_fused_now:
-            split = self.overlap_entity_grad
             call("coper_score1n_bce_fwd_bwd_norm", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
                  ptr(bg.bitsT), bg.B, Ns, d, float(pos), float(neg), inv_count, ptr(bg.loss_sum),
-                 ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), None if split else ptr(g["ent_emb"]), ptr(g["pred_bias"]),
-                 ptr(self.dE_sumsq), ptr(bg.ws), bg.ws_bytes, self.prec)
-            if split:
-                main = torch.cuda.current_stream()
-                self._side.wait_stream(main)
-                with torch.cuda.stream(self._side):
-                    if self.rel_emb is not None:     # cleared here, off the main chain, for the scatter after the join
-                        g["rel_emb"].zero_()
-                        self.grad_sq["rel_emb"].zero_()
-                        rel_cleared = True
-                    self._side_budget(True)
-                    call("coper_score1n_bce_dE", ptr(self._grad_buf(bg)), bg.B, Ns, d, inv_count, ptr(g["ent_emb"]),
-                         ptr(self.dE_sumsq), ptr(g["pred_bias"]), ptr(bg.ws), bg.ws_bytes, self.prec)
-                    self._side_budget(False)
-                    if self.world == 1:              # the mean loss the caller reads (models.py:451)
-                        torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
-                        loss_done = True
-                self._side_pending = True
+                 ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), None, ptr(g["pred_bias"]), ptr(self.dE_sumsq), ptr(bg.ws),
+                 bg.ws_bytes, self.prec)
+            self._side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(self._side):
+                if self.rel_emb is not None:     # cleared here, off the main chain, for the scatter after the join
+                    g["rel_emb"].zero_()
+                    self.grad_sq["rel_emb"].zero_()
+                    rel_cleared = True
+                call("coper_score1n_bce_dE", ptr(self._grad_buf(bg)), bg.B, Ns, d, inv_count, ptr(g["ent_emb"]),
+                     ptr(self.dE_sumsq), ptr(g["pred_bias"]), ptr(bg.ws), bg.ws_bytes, self.prec)
+                if self.world == 1:              # the mean loss the caller reads (models.py:451)
+                    torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
+                    loss_done = True
+            self._side_pending = True
         else:
             call("coper_score1n_bce_fwd_bwd", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
                  ptr(bg.bits if self.prec == 0 else bg.bitsT), bg.B, Ns, d, float(pos), float(neg), inv_count,
@@ -976,9 +934,9 @@ class ConvE:
         self._bn_backward(self.fc_bn, b.dq, b.y, B, d, b, use_batch, True, 1.0, 0, keep2, SALT_OUTPUT, b.dy)
         Pw, Pb = self.fc_weights.projections[-1], self.fc_bias.projections[-1]
         nw, nb = len(self.fc_weights.projections) - 1, len(self.fc_bias.projections) - 1
-        # the generator's weight gradients (dP^, dPb) feed nothing but the clip / optimizer: with the side stream on,
-        # they are computed there while the chain through df / dc continues (DESIGN 4.5)
-        split_w = self.overlap_entity_grad and not dp and self.variant != "param_lookup" and self._split_cpg_bwd
+        # the generator's weight gradients (dP^, dPb) feed nothing but the clip / optimizer: they are computed on the
+        # side stream while the chain through df / dc continues (DESIGN 4.5)
+        split_w = not dp and self.variant != "param_lookup"
         reuse = CPG_BWD_REUSE_FWD if self.prec != 0 else 0
         # g_linear (no hidden generator layers: both contexts ARE the relation embedding): d rel_emb = dc + dcb is formed
         # by the call itself - dc lands in b.dr, the bias generator's dcb is added to it
@@ -993,9 +951,7 @@ class ConvE:
         if split_w:
             self._side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(self._side):
-                self._side_budget(True)
                 call("coper_cpg_fc_bwd", *cpg_bwd_args, reuse | CPG_BWD_WEIGHT_GRADS_ONLY)
-                self._side_budget(False)
             self._side_pending = True
         if self.variant == "param_lookup":
             # the tables are read through embedding_lookup (models.py:91): IndexedSlices gradients, one [F*d] / [d]
@@ -1020,7 +976,7 @@ class ConvE:
             if self.variant == "cpg":
                 b.dr.add_(b.df[:, self.F_conv:])
         # shared filters: the Conv1BN backward is folded into the conv backward (dz never goes to HBM)
-        fold = self.conv_w_gen is None and self._fold_conv_bn
+        fold = self.conv_w_gen is None
         self._bn_backward(self.conv1_bn, b.dfconv, b.z, R1, C, b, use_batch, True, keep1, SALT_FEATURE_MAP, 1.0, 0, b.dz,
                           apply=not fold)
         plain = self.variant == "plain"
@@ -1039,15 +995,10 @@ class ConvE:
                 self._ctx_backward(gen_, net, b, dctx_, b.dr, True)
         else:
             bn1 = self.conv1_bn
-            if fold:
-                call("coper_conv_bwd_bn", ptr(b.dfconv), ptr(b.z), ptr(b.xc if plain else b.x0), B, self.H, self.W,
-                     ptr(self.conv1_weights), self.conv_filter_height, self.conv_filter_width, C, 0, ptr(bn1.a),
-                     ptr(bn1.b), ptr(bn1.mean), ptr(bn1.invstd), ptr(bn1.c1), ptr(bn1.c2), 1, keep1, ptr(self.seed_dev),
-                     SALT_FEATURE_MAP, ptr(b.dxc if plain else b.dx0), ptr(b.dwc_part), ptr(b.dbc_part), ptr(b.dz))
-            else:
-                call("coper_conv_bwd", ptr(b.dz), ptr(b.xc if plain else b.x0), B, self.H, self.W,
-                     ptr(self.conv1_weights), self.conv_filter_height, self.conv_filter_width, C, 0,
-                     ptr(b.dxc if plain else b.dx0), ptr(b.dwc_part), ptr(b.dbc_part))
+            call("coper_conv_bwd_bn", ptr(b.dfconv), ptr(b.z), ptr(b.xc if plain else b.x0), B, self.H, self.W,
+                 ptr(self.conv1_weights), self.conv_filter_height, self.conv_filter_width, C, 0, ptr(bn1.a), ptr(bn1.b),
+                 ptr(bn1.mean), ptr(bn1.invstd), ptr(bn1.c1), ptr(bn1.c2), 1, keep1, ptr(self.seed_dev),
+                 SALT_FEATURE_MAP, ptr(b.dxc if plain else b.dx0), ptr(b.dwc_part), ptr(b.dbc_part), ptr(b.dz))
             if plain:                            # tf.concat backward: the two halves of the stacked image
                 b.dx0.copy_(b.dxc[:, :d])
                 b.dr.copy_(b.dxc[:, d:])
@@ -1285,8 +1236,7 @@ class ConvE:
     def _score(self, b):
         d = self.ent_emb_size
         if self.E_prep is not None:
-            if not getattr(b, "q_prepared", False):
-                call("coper_prepare_operand", ptr(b.q), b.B, d, d, self.prec, ptr(b.q_prep))
+            call("coper_prepare_operand", ptr(b.q), b.B, d, d, self.prec, ptr(b.q_prep))
             call("coper_score1n_fwd_prepared", ptr(b.q_prep), ptr(self.E_prep), ptr(self.pred_bias), b.B,
                  self.shard.rows, d, ptr(self._scores_buf(b)), b.ld, self.prec)
         else:
@@ -1320,8 +1270,7 @@ class ConvE:
         b.rank_counts.zero_()
         if self.E_prep is not None:
             # tensor-pipe engines: rank counts straight from the scorer's accumulators, logits never written
-            if not getattr(b, "q_prepared", False):
-                call("coper_prepare_operand", ptr(b.q), b.B, d, d, self.prec, ptr(b.q_prep))
+            call("coper_prepare_operand", ptr(b.q), b.B, d, d, self.prec, ptr(b.q_prep))
             call("coper_score1n_gold_prepared", ptr(b.q_prep), ptr(self.E_prep), ptr(self.pred_bias), b.B, s.rows, d,
                  ptr(b.e2), s.lo, ptr(b.gold), ptr(b.ws), b.ws_bytes, self.prec)
             sharding.reduce_gold(b.gold, self.world, self.group)

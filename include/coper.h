@@ -56,14 +56,8 @@ long long coper_launch_count(void);
 /* Programmatic dependent launch between consecutive kernels of a stream (every kernel of the library is launched with
  * the programmatic-stream-serialization attribute and begins with griddepcontrol.launch_dependents / .wait): on by
  * default; worth ~8 % on the launch-bound evaluation step of the named datasets, and measured to COST ~10 % on the
- * HBM-bound 10 M-entity step (DESIGN 4.6) - a caller with tables of that size switches it off.  COPER_PDL=0 in the
- * environment forces it off. */
+ * HBM-bound 10 M-entity step (DESIGN 4.6) - a caller with tables of that size switches it off. */
 int coper_set_pdl(int on);
-/* Persistent tcgen05 kernels launched by the calling thread after this call use at most n_sms CTAs (one per SM); 0 = all
- * SMs (default).  For a caller that runs an independent GEMM of the step on a second stream (coper_score1n_bce_dE, the
- * weight-gradient half of coper_cpg_fc_bwd): a persistent kernel on every SM leaves no room for the other stream's
- * kernels, a share does. */
-int coper_set_sm_budget(int n_sms);
 /* 1 if the running device is compute capability 10.x (tcgen05 paths usable), 0 otherwise, <0 on error */
 int coper_device_is_sm100(void);
 
@@ -145,16 +139,6 @@ int coper_bn_act_bwd_stats(const float* dout, const float* x, int64_t R, int C, 
                            const uint64_t* seed_dev, uint64_t salt_post, float* partials, coper_stream_t stream);
 int coper_bn_act_bwd_finalize(const float* partials, int nchunk, int64_t R, int C, int use_batch_stats,
                               float* dgamma, float* dbeta, float* c1, float* c2, coper_stream_t stream);
-/* coper_bn_act_fwd / coper_bn_act_fwd_moving that ALSO emit the tensor-pipe operand form of their output, viewed as
- * [op_rows, op_cols] (op_rows * op_cols == R * C; `prepared` sized by coper_prepared_bytes): the activation that produces
- * f (conv block) or q (FC block) and coper_prepare_operand in one launch (fp16x3; other precisions run the two kernels).
- * Same bits as the two calls. */
-int coper_bn_act_fwd_prepared(const float* x, int64_t R, int C, const float* a, const float* b, int relu, float keep_post,
-                              const uint64_t* seed_dev, uint64_t salt_post, float* out, int64_t op_rows, int op_cols,
-                              int prec, void* prepared, coper_stream_t stream);
-int coper_bn_act_fwd_moving_prepared(const float* x, int64_t R, int C, const float* gamma, const float* beta,
-                                     const float* moving_mean, const float* moving_var, float eps, int relu, float* out,
-                                     int64_t op_rows, int op_cols, int prec, void* prepared, coper_stream_t stream);
 int coper_bn_act_bwd_stats_finalize(const float* dout, const float* x, int64_t R, int C, const float* a, const float* b,
                                     const float* mean, const float* invstd, int relu, float keep_post,
                                     const uint64_t* seed_dev, uint64_t salt_post, float* partials,
@@ -185,15 +169,6 @@ int coper_cpg_fc_fwd(const float* c, const float* f, const float* P, const void*
                      const float* Pb, int B, int dc, int F, int d, int dcb, float keep_out, const uint64_t* seed_dev,
                      uint64_t salt_out, float* y, void* workspace, size_t workspace_bytes, int prec,
                      coper_stream_t stream);
-/* coper_cpg_fc_fwd with flags.  COPER_CPG_FWD_F_PREPARED (tensor-pipe precisions): the operand form of f already lies
- * at the START of `workspace` (coper_prepared_bytes(B, F, prec) bytes - where the call would put it itself), written
- * e.g. by coper_bn_act_fwd_prepared; the call does not convert f again.  Ignored where the contraction does not run on
- * the tensor pipe (see the F % 32 / d <= 256 rule above). */
-#define COPER_CPG_FWD_F_PREPARED 1
-int coper_cpg_fc_fwd_ex(const float* c, const float* f, const float* P, const void* P_prepared, const float* cb,
-                        const float* Pb, int B, int dc, int F, int d, int dcb, float keep_out, const uint64_t* seed_dev,
-                        uint64_t salt_out, float* y, void* workspace, size_t workspace_bytes, int prec, int flags,
-                        coper_stream_t stream);
 /* backward (models.py:198 autodiff of the above): given dy [B,d] (already through the dropout mask)
  *   dP [dc,F*d], dPb [dcb,d], df [B,F], dc_out [B,dc], dcb_out [B,dcb].
  * flags (bit mask):

@@ -312,64 +312,6 @@ def test_bn_act_fwd_moving_equals_two_calls(L, R, C, relu):
     assert np.allclose(out.cpu().numpy(), want, rtol=1e-5, atol=1e-5)
 
 
-# ------------------------------------------------------------------------------------------ activation + operand form
-@pytest.mark.parametrize("prec", ["fp16x3", "bf16", "tf32x3"])
-@pytest.mark.parametrize("R,C,rows,cols,keep", [(512 * 18 * 8, 32, 512, 4608, 0.7), (512, 200, 512, 200, 1.0),
-                                                (96, 40, 96, 40, 0.8), (64 * 9, 4, 64, 36, 1.0), (33, 7, 33, 7, 0.9)])
-def test_bn_act_fwd_prepared_equals_two_calls(L, prec, R, C, rows, cols, keep):
-    rng = np.random.default_rng(9)
-    p = L.PREC[prec]
-    x = dev((rng.normal(size=(R, C)) * 2).astype(np.float32))
-    a, b = dev(rng.normal(size=C).astype(np.float32)), dev(rng.normal(size=C).astype(np.float32))
-    seed = dev(np.array([11], np.int64), torch.int64)
-    nbytes = L.load().coper_prepared_bytes(rows, cols, p)
-    ref, out = torch.zeros(R, C, device="cuda"), torch.zeros(R, C, device="cuda")
-    pref = torch.zeros(nbytes, dtype=torch.uint8, device="cuda")
-    pout = torch.full((nbytes,), 0x5A, dtype=torch.uint8, device="cuda")
-    L.call("coper_bn_act_fwd", L.ptr(x), R, C, L.ptr(a), L.ptr(b), 1, keep, L.ptr(seed), 77, L.ptr(ref))
-    L.call("coper_prepare_operand", L.ptr(ref), rows, cols, cols, p, L.ptr(pref))
-    L.call("coper_bn_act_fwd_prepared", L.ptr(x), R, C, L.ptr(a), L.ptr(b), 1, keep, L.ptr(seed), 77, L.ptr(out), rows,
-           cols, p, L.ptr(pout))
-    assert same_bits(out, ref)
-    ldp = (cols + 3) // 4 * 4 if prec == "tf32x3" else (cols + 7) // 8 * 8
-    planes = rows * ldp * (2 if prec == "bf16" else 4 if prec == "fp16x3" else 8)      # bytes the planes occupy
-    assert torch.equal(pout[:planes], pref[:planes])
-    if prec == "fp16x3":                                         # trailer: exponent, max |x|, running max
-        t0 = nbytes - 256
-        assert torch.equal(pout[t0:t0 + 12].view(torch.int32), pref[t0:t0 + 12].view(torch.int32))
-    # moving-statistics form
-    gamma, beta = dev(rng.normal(size=C).astype(np.float32)), dev(rng.normal(size=C).astype(np.float32))
-    mm, mv = dev(rng.normal(size=C).astype(np.float32)), dev(rng.uniform(0.5, 2, size=C).astype(np.float32))
-    pout.fill_(0x5A)
-    L.call("coper_bn_act_fwd_moving", L.ptr(x), R, C, L.ptr(gamma), L.ptr(beta), L.ptr(mm), L.ptr(mv), 1e-3, 1, L.ptr(ref))
-    L.call("coper_prepare_operand", L.ptr(ref), rows, cols, cols, p, L.ptr(pref))
-    L.call("coper_bn_act_fwd_moving_prepared", L.ptr(x), R, C, L.ptr(gamma), L.ptr(beta), L.ptr(mm), L.ptr(mv), 1e-3, 1,
-           L.ptr(out), rows, cols, p, L.ptr(pout))
-    assert same_bits(out, ref)
-    assert torch.equal(pout[:planes], pref[:planes])
-
-
-@pytest.mark.parametrize("prec", ["fp16x3", "bf16", "tf32x3", "fp32"])
-def test_cpg_fc_fwd_with_prepared_f_equals_plain_call(L, prec):
-    rng = np.random.default_rng(10)
-    B, dc, F, d, dcb = 96, 8, 64, 40, 8
-    p = L.PREC[prec]
-    c, f = dev(rng.normal(size=(B, dc)).astype(np.float32)), dev(rng.normal(size=(B, F)).astype(np.float32))
-    P, Pb = dev(rng.normal(size=(dc, F * d)).astype(np.float32)), dev(rng.normal(size=(dcb, d)).astype(np.float32))
-    cb = dev(rng.normal(size=(B, dcb)).astype(np.float32))
-    seed = dev(np.array([3], np.int64), torch.int64)
-    lib = L.load()
-    nbytes = max(lib.coper_cpg_fc_fwd_workspace_bytes(B, dc, F, d, p), 256)
-    ws0, ws1 = (torch.zeros(nbytes, dtype=torch.uint8, device="cuda") for _ in range(2))
-    y0, y1 = torch.zeros(B, d, device="cuda"), torch.zeros(B, d, device="cuda")
-    args = (L.ptr(c), L.ptr(f), L.ptr(P), None, L.ptr(cb), L.ptr(Pb), B, dc, F, d, dcb, 0.8, L.ptr(seed), 5)
-    L.call("coper_cpg_fc_fwd", *args, L.ptr(y0), L.ptr(ws0), nbytes, p)
-    if prec != "fp32":
-        L.call("coper_prepare_operand", L.ptr(f), B, F, F, p, L.ptr(ws1))     # the operand form of f at the start of ws
-    L.call("coper_cpg_fc_fwd_ex", *args, L.ptr(y1), L.ptr(ws1), nbytes, p, L.CPG_FWD_F_PREPARED)
-    assert same_bits(y0, y1)
-
-
 # ------------------------------------------------------------------------------------------ conv backward with Conv1BN folded in
 @pytest.mark.parametrize("B,H,W,KH,C,keep", [(37, 20, 10, 3, 32, 0.7), (8, 16, 16, 3, 32, 1.0), (5, 10, 10, 3, 8, 0.8),
                                              (4, 12, 8, 2, 32, 0.9)])
