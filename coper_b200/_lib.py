@@ -76,6 +76,11 @@ SIGNATURES = {
     "coper_score1n_rank_workspace_bytes": (sz, [i32, i32, i32]),
     "coper_score1n_gold_prepared": (i32, [vp, vp, vp, i32, i64, i32, vp, i64, vp, vp, sz, i32, vp]),
     "coper_score1n_rank_prepared": (i32, [vp, vp, vp, i32, i64, i32, vp, vp, vp, vp, i32, vp]),
+    "coper_score1n_topk_workspace_bytes": (sz, [i32, i64, i32, i32, i32]),
+    "coper_score1n_topk_prepared": (i32, [vp, vp, vp, i32, i64, i32, vp, i64, i32, vp, vp, vp, sz, i32, vp]),
+    "coper_topk_scores_workspace_bytes": (sz, [i32, i64, i32]),
+    "coper_topk_scores": (i32, [vp, i64, i32, i64, vp, i64, i32, vp, vp, vp, sz, vp]),
+    "coper_topk_merge": (i32, [vp, vp, i32, i32, i32, vp, vp, vp]),
     "coper_csr_to_bits_t": (i32, [vp, vp, i32, i64, i64, vp, vp]),
     "coper_dense_to_bits_t": (i32, [vp, i32, i64, i64, vp, vp]),
     "coper_bits_t_set": (i32, [vp, i32, i64, i64, vp, vp]),
@@ -97,6 +102,7 @@ SIGNATURES = {
     "coper_amsgrad_step": (i32, [vp, vp, vp, vp, vp, i64, vp, f32, f32, f32, vp, i32, vp]),
 }
 SUMSQ_BLOCKS = 256
+TOPK_MAX = 128  # COPER_TOPK_MAX
 MT_CHUNK = 16384
 
 _lib = None

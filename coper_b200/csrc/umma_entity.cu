@@ -367,6 +367,111 @@ struct DiagEpiT : EpiBase {
   }
 };
 
+// ------------------------------------------------------------------------------------------ top-k
+// One list per (CTA, lane quadrant, query) in global memory: a binary min-heap of k keys (topk.cu: score-then-id
+// order as one uint64, 0 = empty slot), written only by the warp that owns the quadrant and the query column - no locks.
+// Per query column the warp keeps a threshold tau (the score of the heap's minimum, -inf while the heap has an empty
+// slot) in shared memory, laid out like RankEpiT's gold logits.  Dense loop per logit: s = acc + bias, x = s - tau,
+// funnel-shift the sign bit (sign clear <=> s >= tau; -inf / +inf thresholds make every / no logit a candidate).
+// Chunks with a candidate that survives the filter word take the insert path: per column with candidates, its owner
+// lane j pulls the candidate rows' scores by shuffle and pushes them (O(log k) per push), then raises tau.
+__device__ __noinline__ void topk_heap_push(uint64_t* h, int k, uint64_t key) {
+  if (key <= h[0]) return;
+  int i = 0;
+  for (;;) {
+    const int l = 2 * i + 1;
+    if (l >= k) break;
+    uint64_t hc = h[l];
+    int c = l;
+    if (l + 1 < k) {
+      const uint64_t hr = h[l + 1];
+      if (hr < hc) { hc = hr; c = l + 1; }
+    }
+    if (hc >= key) break;
+    h[i] = hc;
+    i = c;
+  }
+  h[i] = key;
+}
+// threshold of a heap root: its score, -inf for an empty slot, and -0 for a zero score (so that s - tau keeps its sign
+// bit clear for s = +0 and s = -0 alike)
+__device__ __forceinline__ float topk_key_score(uint64_t key) {
+  if (key == 0ull) return -INFINITY;
+  const uint32_t u = (uint32_t)(key >> 32);
+  if (u == 0x80000000u) return -0.f;
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7FFFFFFFu) : ~u);
+}
+template <int NCH>
+struct TopkEpiT : EpiBase {
+  RowState<NCH> rs;
+  uint64_t* lists;          // [grid * 4][N][k]
+  int k, cur_col0;
+  uint32_t id_hi;           // 0x7FFFFFFF - ent_lo: the key's id field of entity row n is id_hi - n (topk.cu)
+  __device__ __forceinline__ float* tau_smem() {
+    __shared__ float tau_s[kEntEpiWarps][NCH * 32];
+    return tau_s[(threadIdx.x >> 5) - 4];
+  }
+  __device__ __forceinline__ uint64_t* heap(const GemmProblem& p, int col) const {
+    return lists + ((int64_t)(blockIdx.x * 4 + ((threadIdx.x >> 5) & 3)) * p.N + col) * k;
+  }
+  __device__ __forceinline__ void tile_begin(const GemmProblem& p, const TileCoord&, int row, int col0) {
+    if (col0 != cur_col0) {                          // new query block: thresholds of its lists
+      cur_col0 = col0;
+      float* ts = tau_smem();
+      const int lane = threadIdx.x & 31;
+      __syncwarp();
+#pragma unroll
+      for (int i = 0; i < NCH; ++i) {
+        const int c = col0 + i * 32 + lane;
+        ts[i * 32 + lane] = c < p.N ? topk_key_score(heap(p, c)[0]) : INFINITY;   // (masked in chunk as well)
+      }
+      __syncwarp();
+    }
+    rs.begin(p, row, col0);
+  }
+  __device__ __forceinline__ void tile_prefetch(const GemmProblem& p, const TileCoord&, int row, int col0) { rs.prefetch(p, row, col0); }
+  __device__ __forceinline__ void chunk(const GemmProblem& p, const TileCoord&, int row, int col, const uint32_t (&r)[32],
+                                        int ci) {
+    float* ts = tau_smem() + ci * 32;
+    uint32_t msk = 0;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const float x = (__uint_as_float(r[j]) + rs.bias_cur) - ts[j];
+      msk = __funnelshift_l(__float_as_uint(x), msk, 1);
+    }
+    uint32_t cand = ~__brev(msk) & ~rs.w_cur[ci];     // bit j <-> column j; filter bit set = excluded
+    if (row >= p.M) cand = 0u;                        // padded entity rows
+    // columns past the last query: their TMEM words may never have been written by the MMA (it writes n_eff columns),
+    // so the +inf threshold alone cannot exclude them (a stale NaN passes the sign test)
+    if (p.N - col < 32) cand &= (1u << (p.N - col)) - 1u;
+    if (!__any_sync(0xffffffffu, cand != 0u)) return;
+    const int lane = threadIdx.x & 31;
+    const uint32_t cols = __reduce_or_sync(0xffffffffu, cand);
+    const uint32_t key_lo0 = id_hi - (uint32_t)(row - lane);
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      if ((cols >> j) & 1u) {                         // warp-uniform
+        uint32_t rows = __ballot_sync(0xffffffffu, (cand >> j) & 1u);
+        const float sj = __uint_as_float(r[j]) + rs.bias_cur;
+        uint64_t* h = heap(p, col + j);
+        while (rows) {
+          const int src = __ffs(rows) - 1;
+          rows &= rows - 1;
+          const float v = __shfl_sync(0xffffffffu, sj, src);
+          if (lane == j) {
+            uint32_t u = __float_as_uint(v == 0.f ? 0.f : v);
+            u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+            const uint32_t lo = ((key_lo0 - (uint32_t)src) << 1) | (uint32_t)(__float_as_uint(v) == 0x80000000u);
+            topk_heap_push(h, k, ((uint64_t)u << 32) | (uint64_t)lo);
+          }
+        }
+        if (lane == j) ts[j] = topk_key_score(h[0]);
+      }
+    }
+    __syncwarp();
+  }
+};
+
 // rows e2[b] - ent_lo of a prepared operand [Ns, ldp] -> [B, ldp] (zero rows when not owned); 16-byte vectors
 __global__ void gather_prepared_kernel(const uint4* __restrict__ src, int64_t Ns, int vec_per_row, int planes,
                                        const int64_t* __restrict__ e2, int64_t ent_lo, int B, uint4* __restrict__ dst,
@@ -541,6 +646,42 @@ int umma_score1n_rank(const void* q_prep, const void* E_prep, const float* bias,
   if (Ns > 0x7fffffff - 512) return COPER_ERR_UNSUPPORTED;
   TcOperand Q = tc_operand(q_prep, B, d, prec), E = tc_operand(E_prep, Ns, d, prec);
   ENT_DISPATCH(rank_impl, E, Q, bias, B, Ns, d, gold, filtT, n_greater, n_equal, st);
+}
+
+// ------------------------------------------------------------------------------------------ fused top-k
+int topk_merge_keys(const uint64_t* lists, int B, int k, int per, int first_div, int step, int n_groups, float* out_s,
+                    int64_t* out_id, cudaStream_t st);                                                   // topk.cu
+// heaps of every (CTA slot, lane quadrant, query); the grid is at most sm_count() CTAs
+size_t umma_topk_workspace_bytes(int B, int k) { return align_up((size_t)sm_count() * 4 * B * k * sizeof(uint64_t), 256); }
+
+template <class Cfg>
+static int topk_impl(const TcOperand& E, const TcOperand& Q, const float* bias, int B, int64_t Ns, int d,
+                     const uint32_t* filtT, int64_t ent_lo, int k, float* out_s, int64_t* out_id, void* ws,
+                     cudaStream_t st) {
+  GemmProblem p = ent_problem(B, Ns, d, Cfg::BLOCK_N);
+  constexpr int kEntNCH = ent_nch<Cfg>();
+  const int grid = ent_grid(p);
+  uint64_t* lists = static_cast<uint64_t*>(ws);
+  int rc = check_cuda(cudaMemsetAsync(lists, 0, (size_t)grid * 4 * B * k * sizeof(uint64_t), st));   // empty heaps
+  if (rc) return rc;
+  TopkEpiT<kEntNCH> epi;
+  epi.rs.init(bias, filtT, (B + 31) / 32);
+  epi.lists = lists; epi.k = k; epi.cur_col0 = -1;
+  epi.id_hi = 0x7FFFFFFFu - (uint32_t)ent_lo;
+  if ((rc = launch_gemm<Cfg, TopkEpiT<kEntNCH>>(E, Q, p, epi, st, grid))) return rc;
+  // with a grid that is a multiple of n_tiles, CTA c only ever saw query block c % n_tiles
+  if (p.n_tiles <= grid) return topk_merge_keys(lists, B, k, 4, Cfg::BLOCK_N, p.n_tiles, grid / p.n_tiles, out_s, out_id, st);
+  return topk_merge_keys(lists, B, k, 4, 0, 1, grid, out_s, out_id, st);
+}
+int umma_score1n_topk(const void* q_prep, const void* E_prep, const float* bias, int B, int64_t Ns, int d,
+                      const uint32_t* filtT, int64_t ent_lo, int k, float* out_s, int64_t* out_id, void* ws,
+                      size_t ws_bytes, int prec, cudaStream_t st) {
+  if (prec != COPER_PREC_BF16 && prec != COPER_PREC_TF32X3 && prec != COPER_PREC_FP16X3) return COPER_ERR_UNSUPPORTED;
+  if (Ns > 0x7fffffff - 512 || ent_lo + Ns >= 0x7FFFFFFFll) return COPER_ERR_UNSUPPORTED;
+  if (!ws || ws_bytes < umma_topk_workspace_bytes(B, k) || (reinterpret_cast<uintptr_t>(ws) & 255))
+    return COPER_ERR_WORKSPACE;
+  TcOperand Q = tc_operand(q_prep, B, d, prec), E = tc_operand(E_prep, Ns, d, prec);
+  ENT_DISPATCH(topk_impl, E, Q, bias, B, Ns, d, filtT, ent_lo, k, out_s, out_id, ws, st);
 }
 
 // ------------------------------------------------------------------------------------------ training scorer
@@ -768,6 +909,21 @@ int coper_score1n_rank_prepared(const void* q_prep, const void* E_prep, const fl
   COPER_CHECK_ARG(B > 0 && Ns > 0 && d > 0);
   return umma_score1n_rank(q_prep, E_prep, bias, B, Ns, d, gold, filter_bits_t, n_greater, n_equal, prec,
                            as_stream(stream));
+}
+
+size_t coper_score1n_topk_workspace_bytes(int B, int64_t Ns, int d, int k, int prec) {
+  if (prec != COPER_PREC_BF16 && prec != COPER_PREC_TF32X3 && prec != COPER_PREC_FP16X3) return 0;
+  if (B <= 0 || Ns <= 0 || d <= 0 || k < 1 || k > COPER_TOPK_MAX) return 0;
+  return umma_topk_workspace_bytes(B, k);
+}
+int coper_score1n_topk_prepared(const void* q_prep, const void* E_prep, const float* bias, int B, int64_t Ns, int d,
+                                const uint32_t* filter_bits_t, int64_t ent_lo, int k, float* out_scores,
+                                int64_t* out_ids, void* workspace, size_t workspace_bytes, int prec,
+                                coper_stream_t stream) {
+  COPER_CHECK_ARG(q_prep && E_prep && bias && out_scores && out_ids && B > 0 && Ns > 0 && d > 0 && ent_lo >= 0);
+  COPER_CHECK_ARG(k >= 1 && k <= COPER_TOPK_MAX);
+  return umma_score1n_topk(q_prep, E_prep, bias, B, Ns, d, filter_bits_t, ent_lo, k, out_scores, out_ids, workspace,
+                           workspace_bytes, prec, as_stream(stream));
 }
 
 }  // extern "C"

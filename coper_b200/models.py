@@ -1233,6 +1233,69 @@ class ConvE:
         self._score(b)
         return b.S[:, :self.shard.rows]
 
+    def predict_topk(self, batch: Dict, k: int = 10, filtered: bool = True):
+        """The k most likely tail entities of each query (e1, rel, ?): (scores fp32 [B, k], ids int64 [B, k]).
+        Scores are the logits ``predict_all`` computes; entities are sorted by score descending, then by id ascending.
+        ``filtered=True`` excludes the known true tails ``batch['e2_multi*']`` (the standard filtered prediction;
+        ``e2`` is not needed and not excluded).  A query with fewer than k eligible entities is padded with
+        (-inf, -1).  Under entity sharding every rank returns the same global result.  Both tensors are buffers of the
+        (batch size, k) slot, overwritten by the next call with the same batch size and k (clone them to keep them).
+        Speed (DESIGN §6d): well ahead of ``predict_all`` + ``torch.topk`` at 1 M+ entities and small k; at WN18RR's
+        40 k entities with k >= 10, and at k = 100 below 10 M entities, that route is faster."""
+        k = int(k)
+        if not 1 <= k <= _lib.TOPK_MAX:
+            raise ValueError("k must be in [1, %d], got %d" % (_lib.TOPK_MAX, k))
+        keys = ("e1", "rel")
+        if filtered:
+            if "e2_multi_rowptr" not in batch and batch.get("e2_multi") is None:
+                raise ValueError("filtered top-k needs the known true tails: e2_multi, or e2_multi_rowptr / e2_multi_col")
+            keys += ("e2_multi_rowptr", "e2_multi_col", "e2_multi")
+        b = self.stage_batch({key: batch[key] for key in keys if key in batch})
+        t = self._topk_buffers(b, k)
+        self._run_graphed(("topk", b.B, k, bool(filtered)), lambda: self._topk_device(b, t, filtered))
+        return t.scores, t.ids
+
+    def _topk_buffers(self, b, k):
+        if not hasattr(b, "topk"):
+            b.topk = {}
+        if k in b.topk:
+            return b.topk[k]
+        lib, dev, B, P = _lib.load(), self.dev, b.B, self.world
+        t = type("TopkBuf", (), {})()
+        t.scores = torch.empty(B, k, dtype=torch.float32, device=dev)
+        t.ids = torch.empty(B, k, dtype=torch.int64, device=dev)
+        if self.E_prep is not None:
+            t.ws_bytes = lib.coper_score1n_topk_workspace_bytes(B, self.shard.rows, self.ent_emb_size, k, self.prec)
+        else:
+            t.ws_bytes = lib.coper_topk_scores_workspace_bytes(B, self.shard.rows, k)
+        t.ws = torch.empty(t.ws_bytes, dtype=torch.uint8, device=dev)
+        if P > 1:        # this rank's list, and every rank's list after the exchange
+            t.local_scores, t.local_ids = torch.empty_like(t.scores), torch.empty_like(t.ids)
+            t.all_scores = torch.empty(P, B, k, dtype=torch.float32, device=dev)
+            t.all_ids = torch.empty(P, B, k, dtype=torch.int64, device=dev)
+        b.topk[k] = t
+        return t
+
+    def _topk_device(self, b, t, filtered):
+        if self.dp and b.B % self.world == 0:
+            self._forward_q_dp(b, self._local_buffers(b), False)
+        else:
+            self._forward_q(b, False)
+        s, d, k = self.shard, self.ent_emb_size, t.scores.shape[1]
+        out_s, out_i = (t.local_scores, t.local_ids) if self.world > 1 else (t.scores, t.ids)
+        if self.E_prep is not None:
+            # tensor-pipe engines: top-k straight from the scorer's accumulators, logits never written
+            call("coper_prepare_operand", ptr(b.q), b.B, d, d, self.prec, ptr(b.q_prep))
+            call("coper_score1n_topk_prepared", ptr(b.q_prep), ptr(self.E_prep), ptr(self.pred_bias), b.B, s.rows, d,
+                 ptr(b.bitsT) if filtered else None, s.lo, k, ptr(out_s), ptr(out_i), ptr(t.ws), t.ws_bytes, self.prec)
+        else:
+            self._score(b)
+            call("coper_topk_scores", ptr(b.S), b.ld, b.B, s.rows, ptr(b.bits) if filtered else None, s.lo, k,
+                 ptr(out_s), ptr(out_i), ptr(t.ws), t.ws_bytes)
+        if self.world > 1:
+            all_s, all_i = sharding.gather_topk(out_s, out_i, self.world, self.group, out=(t.all_scores, t.all_ids))
+            call("coper_topk_merge", ptr(all_s), ptr(all_i), all_s.shape[0], b.B, k, ptr(t.scores), ptr(t.ids))
+
     def _score(self, b):
         d = self.ent_emb_size
         if self.E_prep is not None:

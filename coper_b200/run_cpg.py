@@ -82,8 +82,17 @@ def main(argv=None):
     ap.add_argument("--needs-test-set-cleaning", action="store_true")
     ap.add_argument("--no-save-best-embeddings", action="store_true")
     ap.add_argument("--model-load-path", default=None)
+    ap.add_argument("--predict-topk", type=int, default=None, metavar="K",
+                    help="with --model-load-path: write the K most likely tails of every test query (filtered by the "
+                         "known true tails) to <evaluation dir>/predictions_test.tsv")
     ap.add_argument("--seed", type=int, default=0)
     args = ap.parse_args(argv)
+    if args.predict_topk is not None:
+        if args.model_load_path is None:
+            ap.error("--predict-topk needs --model-load-path")
+        from ._lib import TOPK_MAX
+        if not 1 <= args.predict_topk <= TOPK_MAX:
+            ap.error("--predict-topk K needs 1 <= K <= %d" % TOPK_MAX)
     logging.basicConfig(level=logging.INFO, format="%(asctime)s %(name)s %(levelname)s %(message)s")
 
     from . import configs, data, synthetic
@@ -202,6 +211,10 @@ def main(argv=None):
     if args.model_load_path is not None:
         model.load_checkpoint(args.model_load_path)
         _evaluate(model, make_eval("test"), "test", eval_path, 0)
+        if args.predict_topk is not None:
+            names = None if args.synthetic else _id_names(data_dir)
+            _write_predictions(model, make_eval("test"), args.predict_topk, names,
+                               os.path.join(eval_path, "predictions_test.tsv"), rank == 0)
         return _finish(world)
     loss = None
     for step in range(cfg.training.max_steps):
@@ -238,6 +251,44 @@ def main(argv=None):
     if loss is not None:
         logger.info("final logged loss %.6f; best dev step %s", loss, best_iter)
     return _finish(world)
+
+
+def _id_names(data_dir):
+    """(entity names, relation names) indexed by id from entities.txt / relations.txt, or None without them.  Ids are
+    line numbers, blank lines included, as the loader assigns them (data.py)."""
+    out = []
+    for f in ("entities.txt", "relations.txt"):
+        path = os.path.join(data_dir, f)
+        if not os.path.exists(path):
+            return None
+        with open(path) as fh:
+            out.append([line.strip() for line in fh])
+    return tuple(out)
+
+
+def _write_predictions(model, batches, k, names, path, write):
+    """One line per query: e1, relation, then k (entity, score) pairs, best first, tab-separated.  Every rank runs
+    predict_topk (a collective when sharded); ``write`` selects the rank that writes the file."""
+    ent = (lambda i: names[0][i]) if names else str
+    rel = (lambda i: names[1][i]) if names else str
+    fh = open(path, "w") if write else None
+    n = 0
+    for batch in batches:
+        scores, ids = model.predict_topk(batch, k=k, filtered=True)
+        scores, ids = scores.cpu().numpy(), ids.cpu().numpy()
+        if fh is None:
+            continue
+        e1, r = np.asarray(batch["e1"]).reshape(-1), np.asarray(batch["rel"]).reshape(-1)
+        for b in range(len(e1)):
+            cols = [ent(int(e1[b])), rel(int(r[b]))]
+            for s, i in zip(scores[b], ids[b]):
+                if i >= 0:
+                    cols += [ent(int(i)), "%.6g" % s]
+            fh.write("\t".join(cols) + "\n")
+            n += 1
+    if fh is not None:
+        fh.close()
+        logger.info("wrote the top-%d predictions of %d test queries to %s", k, n, path)
 
 
 def _finish(world):

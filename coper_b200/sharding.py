@@ -11,6 +11,7 @@ collective on a tiny tensor; dE / dbias / optimizer state of the table never lea
   reduce_scorer_partials all-reduce(sum) of the partial loss (fp64) and the partial dq = G_shard . E_shard
   reduce_sharded_sumsq   all-reduce(sum) of the squared-norm partials of the sharded gradients (global-norm clip)
   reduce_gold_and_counts all-reduce(sum) of the owner-provided gold logits, then of the integer rank counts
+  gather_topk            all-gather of the per-shard top-k lists [B, k] (ConvE.predict_topk merges them on device)
 
 "Data-parallel front end" (weak scaling: the global batch grows with the number of GPUs): every rank receives the
 global batch [Bg] but runs the front end only on ITS Bg/P rows; the scorer still sees all Bg queries against the
@@ -147,6 +148,24 @@ def reduce_counts(n_greater: torch.Tensor, n_equal: torch.Tensor, world: int, gr
         _all_reduce(n_greater, group)
         _all_reduce(n_equal, group)
     return n_greater, n_equal
+
+
+def gather_topk(scores: torch.Tensor, ids: torch.Tensor, world: int, group=None, out=None):
+    """Per-rank top-k lists [B, k] (scores fp32, global ids int64) -> every rank's lists [P, B, k] in rank order on
+    every rank; coper_topk_merge then selects the global top k.  ``out``: optional (scores, ids) [P, B, k] buffers.
+    Without an active group the result is this rank's list alone, [1, B, k]."""
+    if not _active(world, group):
+        if out is None:
+            return scores.unsqueeze(0), ids.unsqueeze(0)
+        out[0][0].copy_(scores)
+        out[1][0].copy_(ids)
+        return out[0][:1], out[1][:1]
+    P = dist.get_world_size(group)
+    if out is None:
+        out = (scores.new_empty((P,) + tuple(scores.shape)), ids.new_empty((P,) + tuple(ids.shape)))
+    _all_gather(out[0].view((-1,) + tuple(scores.shape[1:])), scores.contiguous(), group)   # [P * B, k] form
+    _all_gather(out[1].view((-1,) + tuple(ids.shape[1:])), ids.contiguous(), group)
+    return out
 
 
 # ---- data-parallel front end -------------------------------------------------------------------------------------

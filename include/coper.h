@@ -340,6 +340,34 @@ int coper_score1n_rank_prepared(const void* q_prep, const void* E_prep, const fl
                                 int32_t* n_equal, int prec, coper_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Top-k link prediction: for each query b the k best entities n of this shard [ent_lo, ent_lo + Ns) under
+ *   score s[b, n] = q[b].E[n] + bias[n]   (the fp32 logits the engine's own scorer writes, bit for bit),
+ *   eligible: every entity, or (filter bits != NULL) every entity whose filter bit is clear,
+ *   order: score descending, then global entity id ascending (a total order: the result does not depend on tile
+ *          schedule, grid size, shard count or list order; -0 and +0 compare equal).  Scores are assumed finite.
+ * Output: out_scores fp32 [B, k], out_ids int64 [B, k] (global ids ent_lo + n), sorted by that order; a query with
+ * fewer than k eligible entities is padded with (-inf, -1).  1 <= k <= COPER_TOPK_MAX, ent_lo + Ns < 2^31 - 1.
+ *   coper_score1n_topk_prepared: tensor-pipe engines, fused with the scorer (the logits never leave TMEM); same
+ *       operands and configuration choice as coper_score1n_fwd_prepared.  filter_bits_t: the entity-major matrix
+ *       (coper_csr_to_bits_t), NULL = unfiltered.  workspace: coper_score1n_topk_workspace_bytes (256-byte aligned).
+ *   coper_topk_scores: logits already in HBM, scores [B, ld] (fp32 engine: coper_score1n_fwd); filter_bits: the
+ *       query-major rows of coper_csr_to_bits, NULL = unfiltered.  workspace: coper_topk_scores_workspace_bytes.
+ *   coper_topk_merge: [n_lists, B, k] lists padded with (-inf, -1) -> [B, k] (e.g. the per-shard results of a
+ *       sharded model).  Deterministic and independent of the order of the lists. */
+#define COPER_TOPK_MAX 128
+size_t coper_score1n_topk_workspace_bytes(int B, int64_t Ns, int d, int k, int prec);
+int coper_score1n_topk_prepared(const void* q_prep, const void* E_prep, const float* bias, int B, int64_t Ns, int d,
+                                const uint32_t* filter_bits_t, int64_t ent_lo, int k, float* out_scores,
+                                int64_t* out_ids, void* workspace, size_t workspace_bytes, int prec,
+                                coper_stream_t stream);
+size_t coper_topk_scores_workspace_bytes(int B, int64_t Ns, int k);
+int coper_topk_scores(const float* scores, int64_t ld, int B, int64_t Ns, const uint32_t* filter_bits, int64_t ent_lo,
+                      int k, float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                      coper_stream_t stream);
+int coper_topk_merge(const float* in_scores, const int64_t* in_ids, int n_lists, int B, int k, float* out_scores,
+                     int64_t* out_ids, coper_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * a10 scatter / K8(3) — gradient of the embedding gathers (IndexedSlices -> dense, models.py:198):
  *   dst[idx[i] - row_lo, :] += src[i, :] for row_lo <= idx[i] < row_hi; one writer per destination row
  *   (sort by key, warp per segment, fixed summation order) -> deterministic. */
