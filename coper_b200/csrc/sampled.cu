@@ -18,11 +18,15 @@ namespace coper {
 constexpr int kSampWarps = 8;
 constexpr int kSampMaxK = 8;     // d <= 256: up to 8 strided elements per lane
 
+// kShard (coper_score_sampled_bce_fwd_bwd_sharded): E / bias hold the rows [row_lo, row_hi) of the table and only the
+// positions whose id falls there are scored; the others read nothing and add nothing.  The arithmetic of a scored
+// position is the same in both instantiations, so its score and g are bit-identical to the unsharded call's.
+template <bool kShard>
 __global__ void __launch_bounds__(kSampWarps * 32) sampled_score_bce_kernel(
     const float* __restrict__ q, const float* __restrict__ E, const float* __restrict__ bias,
     const int32_t* __restrict__ lookup, const float* __restrict__ labels, int L, int64_t N, int d, float one_minus_eps,
     float inv_num_ent, float inv_count, double* __restrict__ loss_part, float* __restrict__ scores,
-    float* __restrict__ g_out, float* __restrict__ dq) {
+    float* __restrict__ g_out, float* __restrict__ dq, int64_t row_lo, int64_t row_hi) {
   pdl_enter();
   __shared__ float red[kSampWarps][256];
   __shared__ double lred[kSampWarps];
@@ -37,7 +41,11 @@ __global__ void __launch_bounds__(kSampWarps * 32) sampled_score_bce_kernel(
   double lsum = 0.0;
   for (int l = warp; l < L; l += kSampWarps) {
     const int64_t p = (int64_t)b * L + l;
-    const int64_t ent = lookup[p];
+    int64_t ent = lookup[p];
+    if constexpr (kShard) {
+      if (ent < row_lo || ent >= row_hi) continue;       // warp-uniform (one position per warp): another shard's row
+      ent -= row_lo;
+    }
     const float* row = E + ent * d;
     float er[kSampMaxK];
     float dot = 0.f;
@@ -94,16 +102,32 @@ __global__ void iota32_kernel(int32_t* p, int n) {
   if (i < n) p[i] = i;
 }
 
+// sharded scatter: sort key = local row of an owned position, n_rows (sorts after every owned row) for the others
+__global__ void sampled_shard_keys_kernel(const int32_t* __restrict__ lookup, int M, int64_t row_lo, int64_t row_hi,
+                                          int32_t* __restrict__ keys, int32_t* __restrict__ pos) {
+  pdl_enter();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= M) return;
+  const int64_t id = lookup[i];
+  keys[i] = (int32_t)((id >= row_lo && id < row_hi) ? id - row_lo : row_hi - row_lo);
+  pos[i] = i;
+}
+
 // one warp per sorted position; segment heads walk their segment: slice value = g[pos] * q[pos / L, :]
+// (kShard: keys >= n_rows are the non-owned positions at the end of the sorted order and are skipped)
+template <bool kShard>
 __global__ void sampled_scatter_kernel(const int32_t* __restrict__ keys, const int32_t* __restrict__ pos, int M, int L,
                                        const float* __restrict__ g, const float* __restrict__ q, int d,
                                        float* __restrict__ dE_sum, float* __restrict__ dE_sq,
-                                       float* __restrict__ db_sum, float* __restrict__ db_sq) {
+                                       float* __restrict__ db_sum, float* __restrict__ db_sq, int n_rows) {
   pdl_enter();
   const int seg = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (seg >= M) return;
   const int32_t key = keys[seg];
+  if constexpr (kShard) {
+    if (key >= n_rows) return;
+  }
   if (seg > 0 && keys[seg - 1] == key) return;   // not a segment head
   int end = seg + 1;
   while (end < M && keys[end] == key) ++end;
@@ -242,9 +266,10 @@ __global__ void __launch_bounds__(kSampleThreads) sample_labels_kernel(
 }
 
 struct SampLayout {
-  size_t off_loss, off_keys_out, off_pos_in, off_pos_out, off_cub, cub_bytes, total;
+  size_t off_loss, off_keys_in, off_keys_out, off_pos_in, off_pos_out, off_cub, cub_bytes, total;
 };
-static SampLayout samp_layout(int B, int L) {
+// sharded: + the [B*L] local-row sort keys (the unsharded call sorts the lookup ids themselves)
+static SampLayout samp_layout(int B, int L, bool sharded = false) {
   SampLayout S;
   const int M = B * L;
   size_t o = 0;
@@ -257,8 +282,54 @@ static SampLayout samp_layout(int B, int L) {
                                   (int32_t*)nullptr, M);
   S.cub_bytes = cb;
   S.off_cub = o; o = align_up(o + cb, 256);
+  S.off_keys_in = o;
+  if (sharded) o = align_up(o + (size_t)M * sizeof(int32_t), 256);
   S.total = o;
   return S;
+}
+
+template <bool kShard>
+static int score_sampled(const float* q, const float* E, const float* bias, const int32_t* lookup, const float* labels,
+                         int B, int L, int64_t N, int d, float one_minus_eps, float inv_num_ent, float inv_count,
+                         double* loss_sum, float* scores, float* g, float* dq, float* dE_sum, float* dE_sq,
+                         float* dbias_sum, float* dbias_sq, int64_t row_lo, int64_t row_hi, void* workspace,
+                         size_t workspace_bytes, cudaStream_t st) {
+  SampLayout S = samp_layout(B, L, kShard);
+  if (workspace_bytes < S.total) return COPER_ERR_WORKSPACE;
+  char* ws = static_cast<char*>(workspace);
+  double* loss_part = reinterpret_cast<double*>(ws + S.off_loss);
+  int32_t* keys_out = reinterpret_cast<int32_t*>(ws + S.off_keys_out);
+  int32_t* pos_in = reinterpret_cast<int32_t*>(ws + S.off_pos_in);
+  int32_t* pos_out = reinterpret_cast<int32_t*>(ws + S.off_pos_out);
+  launch_pdl(sampled_score_bce_kernel<kShard>, B, kSampWarps * 32, 0, st, q, E, bias, lookup, labels, L, N, d,
+             one_minus_eps, inv_num_ent, inv_count, loss_part, scores, g, dq, row_lo, row_hi);
+  int rc = check_launch();
+  if (rc) return rc;
+  launch_pdl(sum_loss_kernel, 1, 256, 0, st, loss_part, B, loss_sum);
+  if ((rc = check_launch())) return rc;
+  const int M = B * L;
+  // sort keys: the global ids (< N), or the local rows with the sentinel row_hi - row_lo (<= rows)
+  const int32_t* keys_in = lookup;
+  int64_t key_bound = N;
+  if constexpr (kShard) {
+    int32_t* keys = reinterpret_cast<int32_t*>(ws + S.off_keys_in);
+    launch_pdl(sampled_shard_keys_kernel, ceil_div(M, 256), 256, 0, st, lookup, M, row_lo, row_hi, keys, pos_in);
+    keys_in = keys;
+    key_bound = row_hi - row_lo + 1;
+  } else {
+    launch_pdl(iota32_kernel, ceil_div(M, 256), 256, 0, st, pos_in, M);
+  }
+  if ((rc = check_launch())) return rc;
+  int end_bit = 1;
+  while (end_bit < 31 && (int64_t(1) << end_bit) < key_bound) ++end_bit;
+  size_t cb = S.cub_bytes;
+  // (radix sort is stable: the slices of a row are summed in position order, in both forms of the call)
+  rc = check_cuda(cub::DeviceRadixSort::SortPairs(ws + S.off_cub, cb, keys_in, keys_out, pos_in, pos_out, M, 0, end_bit,
+                                                  st));
+  if (rc) return rc;
+  launch_pdl(sampled_scatter_kernel<kShard>, ceil_div(M, 8), 256, 0, st, keys_out, pos_out, M, L, g, q, d, dE_sum, dE_sq,
+             dbias_sum, dbias_sq, (int)(row_hi - row_lo));
+  return check_launch();
 }
 }  // namespace coper
 
@@ -285,31 +356,29 @@ int coper_score_sampled_bce_fwd_bwd(const float* q, const float* E, const float*
   COPER_CHECK_ARG(q && E && bias && lookup && labels && loss_sum && g && dq && dE_sum && dE_sq && dbias_sum && dbias_sq);
   COPER_CHECK_ARG(B > 0 && L > 0 && N > 0 && d > 0 && workspace);
   if (d > 32 * kSampMaxK) return COPER_ERR_UNSUPPORTED;
-  SampLayout S = samp_layout(B, L);
-  if (workspace_bytes < S.total) return COPER_ERR_WORKSPACE;
-  cudaStream_t st = as_stream(stream);
-  char* ws = static_cast<char*>(workspace);
-  double* loss_part = reinterpret_cast<double*>(ws + S.off_loss);
-  int32_t* keys_out = reinterpret_cast<int32_t*>(ws + S.off_keys_out);
-  int32_t* pos_in = reinterpret_cast<int32_t*>(ws + S.off_pos_in);
-  int32_t* pos_out = reinterpret_cast<int32_t*>(ws + S.off_pos_out);
-  launch_pdl(sampled_score_bce_kernel, B, kSampWarps * 32, 0, st, q, E, bias, lookup, labels, L, N, d, one_minus_eps,
-             inv_num_ent, inv_count, loss_part, scores, g, dq);
-  int rc = check_launch();
-  if (rc) return rc;
-  launch_pdl(sum_loss_kernel, 1, 256, 0, st, loss_part, B, loss_sum);
-  if ((rc = check_launch())) return rc;
-  const int M = B * L;
-  launch_pdl(iota32_kernel, ceil_div(M, 256), 256, 0, st, pos_in, M);
-  if ((rc = check_launch())) return rc;
-  int end_bit = 1;
-  while (end_bit < 31 && (int64_t(1) << end_bit) < N) ++end_bit;
-  size_t cb = S.cub_bytes;
-  rc = check_cuda(cub::DeviceRadixSort::SortPairs(ws + S.off_cub, cb, lookup, keys_out, pos_in, pos_out, M, 0, end_bit, st));
-  if (rc) return rc;
-  launch_pdl(sampled_scatter_kernel, ceil_div(M, 8), 256, 0, st, keys_out, pos_out, M, L, g, q, d, dE_sum, dE_sq,
-             dbias_sum, dbias_sq);
-  return check_launch();
+  return score_sampled<false>(q, E, bias, lookup, labels, B, L, N, d, one_minus_eps, inv_num_ent, inv_count, loss_sum,
+                              scores, g, dq, dE_sum, dE_sq, dbias_sum, dbias_sq, 0, N, workspace, workspace_bytes,
+                              as_stream(stream));
+}
+
+size_t coper_score_sampled_sharded_workspace_bytes(int B, int L) {
+  return (B <= 0 || L <= 0) ? 256 : samp_layout(B, L, true).total;
+}
+
+int coper_score_sampled_bce_fwd_bwd_sharded(const float* q, const float* E, const float* bias, const int32_t* lookup,
+                                            const float* labels, int B, int L, int64_t N, int d, float one_minus_eps,
+                                            float inv_num_ent, float inv_count, double* loss_sum, float* scores,
+                                            float* g, float* dq, float* dE_sum, float* dE_sq, float* dbias_sum,
+                                            float* dbias_sq, int64_t row_lo, int64_t row_hi, void* workspace,
+                                            size_t workspace_bytes, coper_stream_t stream) {
+  COPER_CHECK_ARG(q && E && bias && lookup && labels && loss_sum && g && dq && dE_sum && dE_sq && dbias_sum && dbias_sq);
+  COPER_CHECK_ARG(B > 0 && L > 0 && N > 0 && N < (int64_t(1) << 31) && (int64_t)B * L < (int64_t(1) << 31) && d > 0 &&
+                  workspace);
+  COPER_CHECK_ARG(row_lo >= 0 && row_hi > row_lo && row_hi <= N);
+  if (d > 32 * kSampMaxK) return COPER_ERR_UNSUPPORTED;
+  return score_sampled<true>(q, E, bias, lookup, labels, B, L, N, d, one_minus_eps, inv_num_ent, inv_count, loss_sum,
+                             scores, g, dq, dE_sum, dE_sq, dbias_sum, dbias_sq, row_lo, row_hi, workspace,
+                             workspace_bytes, as_stream(stream));
 }
 
 }  // extern "C"

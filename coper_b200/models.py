@@ -18,8 +18,8 @@ Supported configurations = the three model types the reference ships configs for
 g_linear ``[]`` or g_MLP ``[n, ...]``), ``plain`` (``context_rel_out: null``: shared FC weights, relation image stacked
 under the entity image) and ``param_lookup`` (``do_parameter_lookup``: per-relation tables), plus CPG-generated conv
 filters (``context_rel_conv: [...]`` together with ``context_rel_out``); training with full 1-N labels
-(``num_labels: null``, entity-sharded across GPUs) or with sampled labels (``use_negative_sampling``,
-``models.py:438-443``: ``batch['lookup_values']`` [B, L] or labels drawn on the device; single GPU).  Evaluation is
+(``num_labels: null``) or with sampled labels (``use_negative_sampling``, ``models.py:438-443``:
+``batch['lookup_values']`` [B, L] or labels drawn on the device), both entity-sharded across GPUs.  Evaluation is
 always 1-N.  ``concat_rel`` and generated conv filters combined with shared FC weights / parameter tables raise
 NotImplementedError (no shipped configuration uses them, SURVEY §8f row 4).
 
@@ -166,8 +166,6 @@ class ConvE:
         if self.shard.rows <= 0:
             raise ValueError("%r owns no entity rows: %d entities cannot be sharded %d ways in blocks of %d rows - use "
                              "fewer ranks for this table" % (self.shard, self.num_ent, self.world, self.shard.per))
-        if self.use_negative_sampling and self.world > 1:
-            raise NotImplementedError("sampled-label training is single-GPU (the 1-N path is the entity-sharded one)")
         # data-parallel front end (SURVEY §8e): every rank receives the GLOBAL batch [Bg], runs lookups' conv / CPG /
         # FC on its own Bg/P rows (batch-norm statistics synchronised), all-gathers q and scores all Bg queries
         # against its entity rows; replicated-parameter gradients are all-reduced in one flat bucket.
@@ -897,7 +895,7 @@ class ConvE:
         self._norm_fused_now = self._norm_fused and bg.B <= 4096       # (the scatter correction is the small-M kernel's)
         rel_cleared = loss_done = False
         if self.use_negative_sampling:
-            self._sampled_scorer(b)
+            self._sampled_scorer(bg)
         elif self._norm_fused_now:
             call("coper_score1n_bce_fwd_bwd_norm", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
                  ptr(bg.bitsT), bg.B, Ns, d, float(pos), float(neg), inv_count, ptr(bg.loss_sum),
@@ -1038,9 +1036,9 @@ class ConvE:
             call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), s.lo, s.hi, ptr(bg.ws),
                  bg.ws_bytes)
             if gsq_e is not None:
-                torch.mul(b.dx0, b.dx0, out=b.dx0_sq)
-                call("coper_segscatter_add", ptr(b.e1), B, ptr(b.dx0_sq), d, ptr(gsq_e), s.lo, s.hi, ptr(b.ws),
-                     b.ws_bytes)
+                torch.mul(bg.dx0, bg.dx0, out=bg.dx0_sq)
+                call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0_sq), d, ptr(gsq_e), s.lo, s.hi, ptr(bg.ws),
+                     bg.ws_bytes)
         if self.rel_emb is None:
             if dp:
                 raise NotImplementedError
@@ -1075,26 +1073,34 @@ class ConvE:
             sb.labels, sb.scores, sb.g = (torch.zeros(b.B, L, **f) for _ in range(3))
             sb.h_lookup = torch.zeros(b.B, L, dtype=torch.int32).pin_memory()
             sb.h_labels = torch.zeros(b.B, L, dtype=torch.float32).pin_memory()
-            nbytes = _lib.load().coper_score_sampled_workspace_bytes(b.B, L)
+            lib = _lib.load()
+            nbytes = lib.coper_score_sampled_sharded_workspace_bytes(b.B, L) if self.world > 1 else \
+                lib.coper_score_sampled_workspace_bytes(b.B, L)
             sb.ws = torch.empty(nbytes, dtype=torch.uint8, device=self.dev)
             b.samp[L] = sb
         return b.samp[L]
 
     def _sampled_scorer(self, b):
-        """models.py:438-443 + 448-453 on the staged [B, L] lookup ids / labels (b.cur_samp)."""
-        sb, g, gsq = b.cur_samp, self.grads, self.grad_sq
+        """models.py:438-443 + 448-453 on the staged [B, L] lookup ids / labels (b.cur_samp).  Entity-sharded: every
+        rank scores all B x L positions whose id it owns; loss_sum and dq are its partials (summed by the caller)."""
+        sb, g, gsq, s = b.cur_samp, self.grads, self.grad_sq, self.shard
         for t in (g["ent_emb"], gsq["ent_emb"], g["pred_bias"], gsq["pred_bias"]):
             t.zero_()
         if b.cur_sampling is not None:       # labels drawn on the device from the staged CSR positives (data.py:228-277)
             L, prop_negatives = b.cur_sampling
+            # every rank draws the same [B, L], the single-GPU draw of this seed and step: the data-parallel seed word
+            # carries rank << 32 (per-rank dropout masks), which the salt takes off again (the kernel keys on seed + salt)
+            salt = (SALT_SAMPLE - ((s.rank << 32) if self.dp else 0)) % (1 << 64)
             call("coper_sample_labels", ptr(b.rowptr), ptr(b.col), b.B, self.num_ent, L,
-                 int(1.0 / (1.0 + prop_negatives) * L), ptr(self.seed_dev), SALT_SAMPLE, ptr(sb.lookup),
-                 ptr(sb.labels))
-        call("coper_score_sampled_bce_fwd_bwd", ptr(b.q), ptr(self.ent_emb), ptr(self.pred_bias), ptr(sb.lookup),
-             ptr(sb.labels), b.B, sb.L, self.num_ent, self.ent_emb_size, 1.0 - self.label_smoothing_epsilon,
-             1.0 / self.num_ent, 1.0 / (float(b.B) * float(sb.L)), ptr(b.loss_sum), ptr(sb.scores), ptr(sb.g),
-             ptr(b.dq), ptr(g["ent_emb"]), ptr(gsq["ent_emb"]), ptr(g["pred_bias"]), ptr(gsq["pred_bias"]),
-             ptr(sb.ws), sb.ws.numel())
+                 int(1.0 / (1.0 + prop_negatives) * L), ptr(self.seed_dev), salt, ptr(sb.lookup), ptr(sb.labels))
+        args = (ptr(b.q), ptr(self.ent_emb), ptr(self.pred_bias), ptr(sb.lookup), ptr(sb.labels), b.B, sb.L,
+                self.num_ent, self.ent_emb_size, 1.0 - self.label_smoothing_epsilon, 1.0 / self.num_ent,
+                1.0 / (float(b.B) * float(sb.L)), ptr(b.loss_sum), ptr(sb.scores), ptr(sb.g), ptr(b.dq),
+                ptr(g["ent_emb"]), ptr(gsq["ent_emb"]), ptr(g["pred_bias"]), ptr(gsq["pred_bias"]))
+        if self.world > 1:
+            call("coper_score_sampled_bce_fwd_bwd_sharded", *args, s.lo, s.hi, ptr(sb.ws), sb.ws.numel())
+        else:
+            call("coper_score_sampled_bce_fwd_bwd", *args, ptr(sb.ws), sb.ws.numel())
 
     def _clip_and_apply(self):
         """tf.clip_by_global_norm(5.0) (models.py:199) + AMSGrad apply (amsgrad.py:130-159): one multi-tensor

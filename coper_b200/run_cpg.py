@@ -2,7 +2,7 @@
 
     python -m coper_b200.run_cpg --dataset WN18RR --model-type cpg --data-dir temp/WN18RR/data/WN18RR
     python -m coper_b200.run_cpg --synthetic wn18rr --max-steps 200          # no dataset files needed
-    torchrun --nproc-per-node 8 -m coper_b200.run_cpg --dataset YAGO3-10 --full-1n   # entity-sharded over 8 GPUs
+    torchrun --nproc-per-node 8 -m coper_b200.run_cpg --dataset WN18RR             # entity-sharded over 8 GPUs
 
 Where the reference edits flags in source (``run_cpg.py:38-46``: ``use_cpg``, ``use_parameter_lookup``,
 ``save_best_embeddings``, ``model_load_path``, the loader instance) they are command-line options here; everything else
@@ -16,7 +16,9 @@ replaced by the log lines (SURVEY §5.5).
 Under ``torchrun`` (one process per GPU) the entity table is sharded by entity id and the batch (the config's
 ``batch_size``, unchanged) is split over the ranks (``ConvE(..., shard=..., data_parallel=True)``): every rank reads the
 same batches from its own, identically seeded loader; rank 0 logs and writes the config / embedding pickle, every rank
-saves the checkpoint of its own rows.  Full 1-N labels only (``--full-1n`` for the sampled-label configs).
+saves the checkpoint of its own rows.  Sampled-label configurations (``num_labels``) train sharded the same way: every
+rank stages the same global [B, num_labels] ids / labels (or draws them on its GPU with ``--device-sampling``, identically
+on every rank) and scores the ones its entity rows own; ``--full-1n`` switches to full 1-N labels, as on one GPU.
 """
 from __future__ import annotations
 
@@ -194,8 +196,6 @@ def main(argv=None):
             yaml.dump(_plain(cfg), outfile, default_flow_style=False)
 
     md = configs.model_descriptors(cfg, num_ent, num_rel, use_cpg, use_parameter_lookup)
-    if world > 1 and md["use_negative_sampling"]:
-        raise SystemExit("sampled-label configurations train on one GPU; pass --full-1n for the entity-sharded 1-N path")
     split_batch = world > 1 and cfg.training.batch_size % world == 0 and not use_parameter_lookup
     model = ConvE(md, seed=args.seed, prec=args.prec, conv_in_height=conv_h, init_fast=num_ent > 1_000_000,
                   shard=EntityShard(num_ent, rank, world), data_parallel=split_batch,

@@ -292,6 +292,24 @@ int coper_score_sampled_bce_fwd_bwd(const float* q, const float* E, const float*
                                     float* dq, float* dE_sum, float* dE_sq, float* dbias_sum, float* dbias_sq,
                                     void* workspace, size_t workspace_bytes, coper_stream_t stream);
 
+/* The same step on ONE entity shard (the entity-sharded multi-GPU schedules): lookup holds GLOBAL ids [B, L]; E / bias
+ * are this rank's rows [row_hi - row_lo, d] / [row_hi - row_lo] of the [N, d] / [N] table.  Only positions whose id lies
+ * in [row_lo, row_hi) are scored: their scores / g entries are written with exactly the values the unsharded call
+ * writes for the same q; the entries of all other positions are LEFT UNTOUCHED.  loss_sum and dq [B, d] are this rank's
+ * PARTIALS (a query none of whose lookups the rank owns gets dq = 0): summed over the shards of a partition of [0, N)
+ * they are the unsharded values up to fp32 summation order.  dE_sum, dE_sq [row_hi - row_lo, d] and dbias_sum, dbias_sq
+ * [row_hi - row_lo] are shard-local and accumulated as above; each row equals, bit for bit, the matching row of the
+ * unsharded result (its slices are summed in the same position order).  Workspace:
+ * coper_score_sampled_sharded_workspace_bytes (the [B*L] local sort keys on top of the unsharded layout).  Needs
+ * 0 <= row_lo < row_hi <= N < 2^31, B*L < 2^31, d <= 256. */
+size_t coper_score_sampled_sharded_workspace_bytes(int B, int L);
+int coper_score_sampled_bce_fwd_bwd_sharded(const float* q, const float* E, const float* bias, const int32_t* lookup,
+                                            const float* labels, int B, int L, int64_t N, int d, float one_minus_eps,
+                                            float inv_num_ent, float inv_count, double* loss_sum, float* scores,
+                                            float* g, float* dq, float* dE_sum, float* dE_sq, float* dbias_sum,
+                                            float* dbias_sq, int64_t row_lo, int64_t row_hi, void* workspace,
+                                            size_t workspace_bytes, coper_stream_t stream);
+
 /* labels / filters: CSR positives (rowptr int32 [B+1], col int32 [nnz], global entity ids) -> bit rows for
  * the shard [ent_lo, ent_hi); replaces the dense fp32 multi-hot of data.py:182-186,318-322. */
 int coper_csr_to_bits(const int32_t* rowptr, const int32_t* col, int B, int64_t ent_lo, int64_t ent_hi,
