@@ -72,6 +72,8 @@ SIGNATURES = {
     "coper_score_sampled_sharded_workspace_bytes": (sz, [i32, i32]),
     "coper_score_sampled_bce_fwd_bwd_sharded": (i32, [vp, vp, vp, vp, vp, i32, i32, i64, i32, f32, f32, f32, vp, vp, vp,
                                                       vp, vp, vp, vp, vp, i64, i64, vp, sz, vp]),
+    "coper_score_candidates": (i32, [vp, vp, vp, vp, i32, i32, i32, i64, i64, vp, vp]),
+    "coper_candidate_rank": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i64, i64, vp, vp, i32, vp, vp, vp]),
     "coper_csr_to_bits": (i32, [vp, vp, i32, i64, i64, vp, vp]),
     "coper_dense_to_bits": (i32, [vp, i32, i64, vp, vp]),
     "coper_gold_scores": (i32, [vp, i64, i32, i64, vp, i64, vp, vp]),

@@ -39,8 +39,15 @@ def ranking_and_hits(model, results_dir, data_iterator_handle, name, session=Non
     ties = 0
     count = 0
     pending = []
+    n_cand = set()
     for batch in data_iterator_handle:
-        rank_dev, n_equal_dev = model.filtered_ranks(batch)
+        if "candidates" in batch:
+            # rank among the batch's C given candidates (OGB-style negatives), filtered iff it carries the true tails
+            filtered = "e2_multi_rowptr" in batch or batch.get("e2_multi") is not None
+            rank_dev, n_equal_dev = model.candidate_ranks(batch, batch["candidates"], filtered=filtered)
+            n_cand.add(int(batch["candidates"].shape[1]))
+        else:
+            rank_dev, n_equal_dev = model.filtered_ranks(batch)
         # keep the device busy: read the previous batch's ranks while this one runs
         pending.append((rank_dev.clone(), n_equal_dev.clone()))
         if len(pending) > 1:
@@ -55,6 +62,9 @@ def ranking_and_hits(model, results_dir, data_iterator_handle, name, session=Non
     if ties:
         logger.warning("%d unfiltered scores tie with a gold score; the reference's argsort order is "
                        "unspecified for those (reported rank = 1 + #strictly greater)", ties)
+    if n_cand:
+        logger.info("Ranks are against C = %s given candidates per query, not against all entities.",
+                    "/".join(str(c) for c in sorted(n_cand)))
     logger.info("Evaluated %d samples." % count)
 
     hits = {}

@@ -9,6 +9,8 @@ this object offers the equivalent eager calls:
     loss = model.train_step(batch)          # == session.run((model.loss, model.train_op), {is_train: True})
     scores = model.predict_all(batch)       # == session.run(model.predictions_all)
     ranks, n_equal = model.filtered_ranks(batch)   # metrics.py:44-51 done on device
+    scores = model.score_candidates(batch, candidates)         # [B, C] logits of given tails (-1 = padding)
+    ranks, n_equal = model.candidate_ranks(batch, candidates)  # rank of e2 among C given candidates
 
 PyTorch is used only for device memory, streams, CUDA graphs and torch.distributed; every
 arithmetic step of the hot path is a call into the C ABI (``include/coper.h``).  There is no
@@ -19,9 +21,10 @@ g_linear ``[]`` or g_MLP ``[n, ...]``), ``plain`` (``context_rel_out: null``: sh
 under the entity image) and ``param_lookup`` (``do_parameter_lookup``: per-relation tables), plus CPG-generated conv
 filters (``context_rel_conv: [...]`` together with ``context_rel_out``); training with full 1-N labels
 (``num_labels: null``) or with sampled labels (``use_negative_sampling``, ``models.py:438-443``:
-``batch['lookup_values']`` [B, L] or labels drawn on the device), both entity-sharded across GPUs.  Evaluation is
-always 1-N.  ``concat_rel`` and generated conv filters combined with shared FC weights / parameter tables raise
-NotImplementedError (no shipped configuration uses them, SURVEY §8f row 4).
+``batch['lookup_values']`` [B, L] or labels drawn on the device), both entity-sharded across GPUs.  Evaluation ranks
+against all N entities, or against C given candidates per query (``candidate_ranks``).  ``concat_rel`` and generated
+conv filters combined with shared FC weights / parameter tables raise NotImplementedError (no shipped configuration
+uses them, SURVEY §8f row 4).
 
 Engines (``prec``): ``fp32`` (CUDA-core FFMA, the on-device parity reference), ``tf32x3`` / ``fp16x3`` (fp32-class
 3-term compensated tcgen05 engines), ``bf16`` (tcgen05, the 10 M-entity throughput path; its scorer + BCE + dq run as
@@ -1354,3 +1357,120 @@ class ConvE:
         sharding.reduce_counts(b.n_greater, b.n_equal, self.world, self.group)
         torch.add(b.n_greater, 1, out=b.rank)        # inside the captured step: the caller reads b.rank
         return b.rank, b.n_equal
+
+    # ------------------------------------------------------------------------------------------ given candidates
+    def score_candidates(self, batch: Dict, candidates):
+        """Logits of given tails: ``candidates`` int [B, C] of global entity ids (host or device), -1 = padding.
+        Returns fp32 [B, C] with s[b, j] = q[b].E[candidates[b, j]] + bias[candidates[b, j]] and -inf at padding;
+        ``batch`` needs ``e1`` and ``rel`` only.  Host candidates outside [-1, num_ent) raise ValueError; on the device
+        an id >= num_ent scores 0.  The scores are exact fp32 dot products with the master entity table for every
+        ``prec`` - the logits the sampled-label training step computes, bit for bit - so they match ``predict_all``
+        only to the engine's score tolerance (bf16: 1e-2).  Under entity sharding every rank returns the single-GPU
+        result (a logit of -0 comes back as +0).  The tensor is a buffer of the (B, C) slot, overwritten by the next
+        call with the same B and C (clone it to keep it)."""
+        b, c = self._stage_candidates({k: batch[k] for k in ("e1", "rel")}, candidates, with_e2=False)
+        self._run_graphed(("cand_score", b.B, c.C), lambda: self._cand_score_device(b, c))
+        return c.scores
+
+    def candidate_ranks(self, batch: Dict, candidates, filtered: bool = True):
+        """Rank of the gold tail ``batch['e2']`` among given candidates (int [B, C] global ids, -1 = padding), as
+        ``filtered_ranks`` ranks it among all entities: rank = 1 + #{j : candidates[b, j] != e2[b], not a known true
+        tail, s[b, j] > s[b, e2[b]]}; n_equal counts the ties the same way.  A candidate listed twice counts twice.
+        ``filtered=True`` excludes the known true tails ``batch['e2_multi*']`` (ValueError without them);
+        ``filtered=False`` excludes only the gold entity itself.  Scores as in ``score_candidates``.  Returns int32
+        device tensors (rank, n_equal) [B], buffers of the (B, C) slot, overwritten by the next call with the same B
+        and C (clone them to keep them)."""
+        if not (isinstance(batch["e2"], torch.Tensor) and batch["e2"].is_cuda):
+            e2 = np.asarray(batch["e2"])
+            if int(e2.min()) < 0 or int(e2.max()) >= self.num_ent:
+                raise ValueError("e2 out of range (train rows carry e2 = -1 in the reference; SURVEY Q17)")
+        keys = ("e1", "rel", "e2")
+        if filtered:
+            if "e2_multi_rowptr" not in batch and batch.get("e2_multi") is None:
+                raise ValueError("filtered candidate ranks need the known true tails: e2_multi, or e2_multi_rowptr / "
+                                 "e2_multi_col")
+            keys += ("e2_multi_rowptr", "e2_multi_col", "e2_multi")
+        b, c = self._stage_candidates({k: batch[k] for k in keys if k in batch}, candidates, with_e2=True)
+        self._run_graphed(("cand_rank", b.B, c.C, bool(filtered)), lambda: self._cand_rank_device(b, c, filtered))
+        return c.rank, c.n_equal
+
+    def _cand_buffers(self, b, C):
+        """(B, C) slot: int32 [B, C] candidates followed by the [B] gold ids in one device block, staged through one
+        pinned host block (one copy per call), the [B, C] scores and the rank outputs."""
+        if not hasattr(b, "cand"):
+            b.cand = {}
+        if C not in b.cand:
+            B, dev = b.B, self.dev
+            t = type("CandBuf", (), {})()
+            t.C = C
+            t.d_ids = torch.zeros(B * C + B, dtype=torch.int32, device=dev)
+            t.cand, t.e2 = t.d_ids[:B * C].view(B, C), t.d_ids[B * C:]
+            t.h_ids = torch.zeros(B * C + B, dtype=torch.int32).pin_memory()
+            t.h_np = t.h_ids.numpy()
+            t.scores = torch.zeros(B, C, dtype=torch.float32, device=dev)
+            t.gold = torch.zeros(B, dtype=torch.float32, device=dev)
+            t.counts = torch.zeros(2, B, dtype=torch.int32, device=dev)
+            t.n_greater, t.n_equal = t.counts[0], t.counts[1]
+            t.rank = torch.zeros(B, dtype=torch.int32, device=dev)
+            b.cand[C] = t
+        return b.cand[C]
+
+    def _stage_candidates(self, batch, candidates, with_e2):
+        on_device = isinstance(candidates, torch.Tensor) and candidates.is_cuda
+        if not on_device:
+            candidates = np.asarray(candidates)
+        if len(candidates.shape) != 2 or candidates.shape[1] < 1 or candidates.shape[0] != len(batch["e1"]):
+            raise ValueError("candidates must be [B, C] with C >= 1 and B = len(e1), got %s" % (tuple(candidates.shape),))
+        if not on_device and (int(candidates.min()) < -1 or int(candidates.max()) >= self.num_ent):
+            raise ValueError("candidate ids must lie in [0, %d) or be -1 (padding)" % self.num_ent)
+        b = self.stage_batch(batch)             # e1, rel and the filter bits; e2 travels in the candidate block
+        B, C = b.B, int(candidates.shape[1])
+        c = self._cand_buffers(b, C)
+        # each region of the block comes from where its ids live; two host regions travel in one copy
+        e2 = batch["e2"] if with_e2 else None
+        e2_on_device = isinstance(e2, torch.Tensor) and e2.is_cuda
+        if on_device:
+            c.cand.copy_(candidates)
+        else:
+            c.h_np[:B * C] = candidates.reshape(-1)
+        if e2 is not None and e2_on_device:
+            c.e2.copy_(e2)
+        elif e2 is not None:
+            c.h_np[B * C:] = np.asarray(e2).reshape(-1)
+        host_e2 = e2 is not None and not e2_on_device
+        if not on_device and host_e2:
+            c.d_ids.copy_(c.h_ids, non_blocking=True)
+        elif not on_device:
+            c.cand.copy_(c.h_ids[:B * C].view(B, C), non_blocking=True)
+        elif host_e2:
+            c.e2.copy_(c.h_ids[B * C:], non_blocking=True)
+        b.h2d_event.record()               # the next stage_batch waits for this copy before reusing pinned memory
+        return b, c
+
+    def _eval_q(self, b):
+        if self.dp and b.B % self.world == 0:
+            self._forward_q_dp(b, self._local_buffers(b), False)
+        else:
+            self._forward_q(b, False)
+
+    def _cand_score_device(self, b, c):
+        s = self.shard
+        self._eval_q(b)
+        call("coper_score_candidates", ptr(b.q), ptr(self.ent_emb), ptr(self.pred_bias), ptr(c.cand), b.B, c.C,
+             self.ent_emb_size, s.lo, s.hi, ptr(c.scores))
+        sharding.exchange_rows(c.scores, self.world, self.group)     # non-owned positions hold exact zeros
+        c.scores.masked_fill_(c.cand < 0, float("-inf"))
+
+    def _cand_rank_device(self, b, c, filtered):
+        s, d = self.shard, self.ent_emb_size
+        self._eval_q(b)
+        c.counts.zero_()
+        # the gold logit by the same kernel and arithmetic as the candidates it is compared with
+        call("coper_score_candidates", ptr(b.q), ptr(self.ent_emb), ptr(self.pred_bias), ptr(c.e2), b.B, 1, d, s.lo,
+             s.hi, ptr(c.gold))
+        sharding.reduce_gold(c.gold, self.world, self.group)
+        bits = (b.bits if self.prec == 0 else b.bitsT) if filtered else None
+        call("coper_candidate_rank", ptr(b.q), ptr(self.ent_emb), ptr(self.pred_bias), ptr(c.cand), ptr(c.e2), b.B,
+             c.C, d, s.lo, s.hi, ptr(c.gold), ptr(bits), int(self.prec != 0), ptr(c.n_greater), ptr(c.n_equal))
+        sharding.reduce_counts(c.n_greater, c.n_equal, self.world, self.group)
+        torch.add(c.n_greater, 1, out=c.rank)

@@ -87,8 +87,14 @@ def main(argv=None):
     ap.add_argument("--predict-topk", type=int, default=None, metavar="K",
                     help="with --model-load-path: write the K most likely tails of every test query (filtered by the "
                          "known true tails) to <evaluation dir>/predictions_test.tsv")
+    ap.add_argument("--score-triples", default=None, metavar="FILE",
+                    help="with --model-load-path: score the tab-separated (head, relation, tail) lines of FILE and write "
+                         "them with their logit and sigmoid(logit) to <evaluation dir>/scores_<FILE name without its "
+                         "extension>.tsv")
     ap.add_argument("--seed", type=int, default=0)
     args = ap.parse_args(argv)
+    if args.score_triples is not None and args.model_load_path is None:
+        ap.error("--score-triples needs --model-load-path")
     if args.predict_topk is not None:
         if args.model_load_path is None:
             ap.error("--predict-topk needs --model-load-path")
@@ -195,6 +201,9 @@ def main(argv=None):
         with open(os.path.join(config_save_dir, "config.yml"), "w") as outfile:
             yaml.dump(_plain(cfg), outfile, default_flow_style=False)
 
+    triples = None
+    if args.score_triples is not None:      # read (and reject) the file before the model is built
+        triples = _read_triples(args.score_triples, None if args.synthetic else _id_names(data_dir), num_ent, num_rel)
     md = configs.model_descriptors(cfg, num_ent, num_rel, use_cpg, use_parameter_lookup)
     split_batch = world > 1 and cfg.training.batch_size % world == 0 and not use_parameter_lookup
     model = ConvE(md, seed=args.seed, prec=args.prec, conv_in_height=conv_h, init_fast=num_ent > 1_000_000,
@@ -215,6 +224,10 @@ def main(argv=None):
             names = None if args.synthetic else _id_names(data_dir)
             _write_predictions(model, make_eval("test"), args.predict_topk, names,
                                os.path.join(eval_path, "predictions_test.tsv"), rank == 0)
+        if triples is not None:
+            base = os.path.splitext(os.path.basename(args.score_triples))[0]
+            _write_triple_scores(model, triples, cfg.training.batch_size,
+                                 os.path.join(eval_path, "scores_%s.tsv" % base), rank == 0)
         return _finish(world)
     loss = None
     for step in range(cfg.training.max_steps):
@@ -289,6 +302,60 @@ def _write_predictions(model, batches, k, names, path, write):
     if fh is not None:
         fh.close()
         logger.info("wrote the top-%d predictions of %d test queries to %s", k, n, path)
+
+
+def _read_triples(path, names, num_ent, num_rel):
+    """Tab-separated (head, relation, tail) lines -> (e1, rel, e2) int64 arrays and the input columns.  Names map
+    through ``names`` (entities.txt / relations.txt); without them the columns are integer ids.  A name that is not
+    known, an id out of range or a line without three columns exits with the file and line number."""
+    index = [{n: i for i, n in enumerate(t)} for t in names] if names else None
+    ids, cols = [], []
+    with open(path) as fh:
+        for lineno, line in enumerate(fh, 1):
+            line = line.rstrip("\r\n")
+            if not line.strip():
+                continue
+            f = line.split("\t")
+            if len(f) != 3:
+                sys.exit("%s:%d: expected 3 tab-separated columns (head, relation, tail), got %d" % (path, lineno, len(f)))
+            row = []
+            for col, what, kind, n in ((f[0], "entity", 0, num_ent), (f[1], "relation", 1, num_rel),
+                                       (f[2], "entity", 0, num_ent)):
+                if index is not None:
+                    i = index[kind].get(col.strip(), -1)
+                    if i < 0:
+                        sys.exit("%s:%d: unknown %s name %r" % (path, lineno, what, col))
+                else:
+                    try:
+                        i = int(col)
+                    except ValueError:
+                        sys.exit("%s:%d: %r is not an integer %s id (the dataset has no name files)" %
+                                 (path, lineno, col, what))
+                    if not 0 <= i < n:
+                        sys.exit("%s:%d: %s id %d out of range [0, %d)" % (path, lineno, what, i, n))
+                row.append(i)
+            ids.append(row)
+            cols.append(f)
+    ids = np.asarray(ids, dtype=np.int64).reshape(-1, 3)
+    return ids[:, 0], ids[:, 1], ids[:, 2], cols
+
+
+def _write_triple_scores(model, triples, batch_size, path, write):
+    """One line per input line: its three columns, the logit (%.6g) and sigmoid(logit).  Every rank scores (a
+    collective when sharded); ``write`` selects the rank that writes the file."""
+    e1, rel, e2, cols = triples
+    fh = open(path, "w") if write else None
+    for i in range(0, len(e1), batch_size):
+        sl = slice(i, i + batch_size)
+        s = model.score_candidates({"e1": e1[sl], "rel": rel[sl]}, e2[sl].reshape(-1, 1)).cpu().numpy()[:, 0]
+        if fh is None:
+            continue
+        sig = 0.5 * (1.0 + np.tanh(0.5 * s.astype(np.float64)))
+        for j in range(len(s)):
+            fh.write("\t".join(cols[i + j] + ["%.6g" % s[j], "%.6g" % sig[j]]) + "\n")
+    if fh is not None:
+        fh.close()
+        logger.info("wrote the scores of %d triples to %s", len(e1), path)
 
 
 def _finish(world):

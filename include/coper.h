@@ -310,6 +310,29 @@ int coper_score_sampled_bce_fwd_bwd_sharded(const float* q, const float* E, cons
                                             float* dbias_sq, int64_t row_lo, int64_t row_hi, void* workspace,
                                             size_t workspace_bytes, coper_stream_t stream);
 
+/* a8, forward only — scores of GIVEN candidate entities (models.py:438-443, predictions_lookup for arbitrary ids) and
+ * the filtered rank of the gold tail among them; the [B, N] logits are never formed.  cand int32 [B, C] holds GLOBAL
+ * entity ids; E / bias are this rank's rows [row_hi - row_lo, d] / [row_hi - row_lo] of the table.
+ *   coper_score_candidates: scores fp32 [B, C]; a position whose id lies in [row_lo, row_hi) gets
+ *       s = q[b].E[id] + bias[id], bit-identical to the score coper_score_sampled_bce_fwd_bwd writes for the same q,
+ *       table and id (the same lane-strided fp32 fmaf chain, warp reduction and bias add); every other position
+ *       (padding -1, ids outside the table, ids another shard owns) gets exactly 0 and reads nothing - summed over the
+ *       shards of a partition of [0, N) the scores are the unsharded ones.  The gold logit of coper_candidate_rank is
+ *       this call with C = 1 and cand = e2 (summed over the shards).
+ *   coper_candidate_rank: counts ACCUMULATED into n_greater / n_equal int32 [B] (zero them first):
+ *       n_greater[b] += #{j : cand[b,j] owned, cand[b,j] != e2[b], !filtered(b, cand[b,j]), s(b,j) >  gold[b]}
+ *       n_equal[b]   += the same with ==.   rank = 1 + sum over shards of n_greater; duplicates count once per
+ *       occurrence.  filter_bits: the shard's query-major rows of coper_csr_to_bits (entity_major = 0) or the
+ *       entity-major matrix of coper_csr_to_bits_t (entity_major = 1); NULL = unfiltered.  e2 int32 [B].
+ * Exact fp32 from the master table for every engine (gather-bound, no tensor-pipe variant); deterministic.  Needs
+ * 1 <= B, 1 <= C, B*C < 2^31, 0 <= row_lo < row_hi < 2^31 (COPER_ERR_INVALID_ARG), d <= 256 (COPER_ERR_UNSUPPORTED). */
+int coper_score_candidates(const float* q, const float* E, const float* bias, const int32_t* cand, int B, int C, int d,
+                           int64_t row_lo, int64_t row_hi, float* scores, coper_stream_t stream);
+int coper_candidate_rank(const float* q, const float* E, const float* bias, const int32_t* cand, const int32_t* e2,
+                         int B, int C, int d, int64_t row_lo, int64_t row_hi, const float* gold,
+                         const uint32_t* filter_bits, int entity_major, int32_t* n_greater, int32_t* n_equal,
+                         coper_stream_t stream);
+
 /* labels / filters: CSR positives (rowptr int32 [B+1], col int32 [nnz], global entity ids) -> bit rows for
  * the shard [ent_lo, ent_hi); replaces the dense fp32 multi-hot of data.py:182-186,318-322. */
 int coper_csr_to_bits(const int32_t* rowptr, const int32_t* col, int B, int64_t ent_lo, int64_t ent_hi,
