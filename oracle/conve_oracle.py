@@ -491,7 +491,7 @@ def backward(out, cfg: OracleConfig):
     kr = (cw[:, :, None] * f[:, None, :]).reshape(B, dc * F)
     dPw = (kr.T @ dy).reshape(dc, F * d)
     dPb = cb.T @ dy
-    T = np.einsum("bj,kij->bki", dy, P3)                        # T[b,k,i] = sum_j P[k,i,j] dy[b,j]
+    T = np.einsum("bj,kij->bki", dy, P3, optimize=True)         # T[b,k,i] = sum_j P[k,i,j] dy[b,j] (as a GEMM)
     df = np.einsum("bk,bki->bi", cw, T)
     dcw = np.einsum("bi,bki->bk", f, T)
     dcb = dy @ Pb.T
