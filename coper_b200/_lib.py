@@ -8,6 +8,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcoper_sm100.so")
 
@@ -91,7 +93,6 @@ SIGNATURES = {
     "coper_bits_t_set": (i32, [vp, i32, i64, i64, vp, vp]),
     "coper_segscatter_workspace_bytes": (sz, [i32]),
     "coper_segscatter_add_sq": (i32, [vp, i32, vp, i32, vp, vp, i64, i64, vp]),
-    "coper_segscatter_add_norm": (i32, [vp, i32, vp, i32, vp, vp, i64, i64, vp, vp]),
     "coper_segscatter_add_pair": (i32, [vp, i32, vp, i32, vp, vp, i64, i64, vp, vp, i32, vp, i32, vp, vp, i64, i64, vp]),
     "coper_segscatter_add": (i32, [vp, i32, vp, i32, vp, i64, i64, vp, sz, vp]),
     "coper_reduce_partials": (i32, [vp, i32, i64, f32, i32, vp, vp]),
@@ -109,6 +110,9 @@ SIGNATURES = {
 SUMSQ_BLOCKS = 256
 TOPK_MAX = 128  # COPER_TOPK_MAX
 MT_CHUNK = 16384
+# mirrors coper_param_desc (include/coper.h): one record per tensor of the multi-tensor clip / AMSGrad launches
+PARAM_DESC = np.dtype([("theta", "<u8"), ("grad", "<u8"), ("m", "<u8"), ("v", "<u8"), ("vhat", "<u8"), ("prepared", "<u8"),
+                       ("grad_sq", "<u8"), ("n", "<i8"), ("prepared_prec", "<i4"), ("mode", "<i4")])
 
 _lib = None
 launch_count = 0  # number of C-ABI compute calls issued by this process (bench.py reports it)

@@ -227,26 +227,16 @@ int coper_segscatter_add_sq(const int64_t* idx, int M, const float* src, int wid
   return check_launch();
 }
 
-int coper_segscatter_add_norm(const int64_t* idx, int M, const float* src, int width, float* dst, float* dst_sq,
-                              int64_t row_lo, int64_t row_hi, double* norm_delta, coper_stream_t stream) {
-  COPER_CHECK_ARG(idx && src && dst && norm_delta && M >= 0 && width > 0 && row_hi >= row_lo);
-  if (M > kSegSmallM) return COPER_ERR_UNSUPPORTED;
-  if (M == 0) return COPER_OK;
-  SegSmallJob A{idx, M, src, width, dst, dst_sq, row_lo, row_hi, norm_delta};
-  launch_pdl(segscatter_small_kernel, ceil_div(M, 8), 256, 0, as_stream(stream), A, ceil_div(M, 8), SegSmallJob{}, 0);
-  return check_launch();
-}
-
 int coper_segscatter_add_pair(const int64_t* idx_a, int M_a, const float* src_a, int width_a, float* dst_a,
                               float* dst_sq_a, int64_t lo_a, int64_t hi_a, double* norm_delta_a, const int64_t* idx_b,
                               int M_b, const float* src_b, int width_b, float* dst_b, float* dst_sq_b, int64_t lo_b,
                               int64_t hi_b, coper_stream_t stream) {
   COPER_CHECK_ARG(idx_a && src_a && dst_a && M_a > 0 && width_a > 0 && hi_a >= lo_a);
-  COPER_CHECK_ARG(idx_b && src_b && dst_b && M_b > 0 && width_b > 0 && hi_b >= lo_b);
+  COPER_CHECK_ARG(M_b == 0 || (idx_b && src_b && dst_b && M_b > 0 && width_b > 0 && hi_b >= lo_b));
   if (M_a > kSegSmallM || M_b > kSegSmallM) return COPER_ERR_UNSUPPORTED;
   SegSmallJob A{idx_a, M_a, src_a, width_a, dst_a, dst_sq_a, lo_a, hi_a, norm_delta_a};
   SegSmallJob Bj{idx_b, M_b, src_b, width_b, dst_b, dst_sq_b, lo_b, hi_b, nullptr};
-  const int row_owner = hi_b - lo_b <= kSegRowOwnerRows && hi_b > lo_b;
+  const int row_owner = M_b > 0 && hi_b - lo_b <= kSegRowOwnerRows && hi_b > lo_b;
   const int ba = ceil_div(M_a, 8), bb = row_owner ? (int)(hi_b - lo_b) : ceil_div(M_b, 8);
   launch_pdl(segscatter_small_kernel, ba + bb, 256, 0, as_stream(stream), A, ba, Bj, row_owner);
   return check_launch();

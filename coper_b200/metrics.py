@@ -15,6 +15,8 @@ import os
 
 import numpy as np
 
+from .models import has_known_tails
+
 __all__ = ["ranking_and_hits"]
 
 logger = logging.getLogger(__name__)
@@ -43,8 +45,7 @@ def ranking_and_hits(model, results_dir, data_iterator_handle, name, session=Non
     for batch in data_iterator_handle:
         if "candidates" in batch:
             # rank among the batch's C given candidates (OGB-style negatives), filtered iff it carries the true tails
-            filtered = "e2_multi_rowptr" in batch or batch.get("e2_multi") is not None
-            rank_dev, n_equal_dev = model.candidate_ranks(batch, batch["candidates"], filtered=filtered)
+            rank_dev, n_equal_dev = model.candidate_ranks(batch, batch["candidates"], filtered=has_known_tails(batch))
             n_cand.add(int(batch["candidates"].shape[1]))
         else:
             rank_dev, n_equal_dev = model.filtered_ranks(batch)

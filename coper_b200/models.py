@@ -94,6 +94,175 @@ class ContextualParameterGenerator:
         self.hidden = list(context_size[1:])
 
 
+def has_known_tails(batch: Dict) -> bool:
+    """Does the batch carry the known true tails of its queries (``e2_multi``, or ``e2_multi_rowptr`` / ``e2_multi_col``)?"""
+    return "e2_multi_rowptr" in batch or batch.get("e2_multi") is not None
+
+
+class _BatchSlot:
+    """Static device buffers of one batch size (pointer-stable -> CUDA-graph friendly).  Fields that a variant does not
+    use are None; lazily filled ones start as None / {} / 0."""
+
+    def __init__(self, m: "ConvE", B: int):
+        dev, f32 = m.dev, torch.float32
+        d, dr, F, C = m.ent_emb_size, m.rel_emb_size, m.F, m.C
+        Ns = m.shard.rows
+        z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
+        lib = _lib.load()
+        self.B, self.ld, self.words = B, -(-Ns // 32) * 32, -(-Ns // 32)
+        # query ids + CSR row pointers live in ONE device block so that a host batch needs one H2D copy for them:
+        # [e1 | rel | e2] int64 [3, B] followed by rowptr int32 [B + 1]
+        head_words = 6 * B + (B + 2)
+        self.d_head = z(head_words, dt=torch.int32)
+        self.h_head = torch.zeros(head_words, dtype=torch.int32).pin_memory()
+        idx64 = self.d_head[:6 * B].view(torch.int64).view(3, B)
+        self.e1, self.rel, self.e2 = idx64[0], idx64[1], idx64[2]
+        self.h_head_np = self.h_head.numpy()
+        self.h_idx_np = self.h_head_np[:6 * B].view(np.int64).reshape(3, B)
+        self.h_rowptr_np = self.h_head_np[6 * B:6 * B + B + 1]
+        self.x0, self.r = z(B, d), z(B, dr)
+        Fc = m.F_conv
+        self.z, self.f = z(B, Fc), z(B, F)
+        # concat_rel: the conv block works on contiguous [B, F_conv] buffers; f / df hold [conv features | rel_emb]
+        self.fconv, self.dfconv = (z(B, Fc), z(B, Fc)) if m.concat_rel else (self.f, None)
+        self.y, self.q = z(B, d), z(B, d)
+        self.q_prep = None
+        if m.E_prep is not None:
+            self.q_prep = torch.zeros(lib.coper_prepared_bytes(B, d, m.prec), dtype=torch.uint8, device=dev)
+        self.dq, self.dy, self.df, self.dz, self.dx0, self.dr = z(B, d), z(B, d), z(B, F), z(B, Fc), z(B, d), z(B, dr)
+        if not m.concat_rel:
+            self.dfconv = self.df
+        R1 = B * m.OH * m.OW
+        nch = max(lib.coper_colstats_chunks(R1), lib.coper_colstats_chunks(B))
+        maxC = max([C, d] + [n for gcp in m.generators for n in gcp.hidden])
+        self.stat = z(nch * maxC * 2)
+        self.stat1 = z(maxC * 2)
+        self.stat_all = None          # data-parallel front end: every rank's statistics partials (first use)
+        # allocated on first use (each exactly once, so captured graphs keep valid pointers):
+        #   S  logits fp32 [B, ld] (predict_all / the two-pass ranking of the fp32 engine)
+        #   G  dL/dS in the scorer's operand form (train); never read by the host
+        self.S = self.G = None
+        # label / filter bits: query-major rows for the fp32 engine, the entity-major matrix for the tensor pipe
+        self.bits = z(B, self.words, dt=torch.int32) if m.prec == 0 else None
+        self.bitsT = z(max(Ns, 1), -(-B // 32), dt=torch.int32) if m.prec != 0 else None
+        self.loss_sum = z(1, dt=torch.float64)
+        self.gold = z(B)
+        self.rank_counts = z(2, B, dt=torch.int32)       # one buffer: cleared by one fill per evaluation batch
+        self.n_greater, self.n_equal = self.rank_counts[0], self.rank_counts[1]
+        self.rank = z(B, dt=torch.int32)
+        self.loss_mean = z(1, dt=torch.float64)
+        self.dwc_part, self.dbc_part = z(B, m.conv_filter_height * m.conv_filter_width * C), z(B, C)
+        dcw = m.fc_weights.projections[-1].shape[0]
+        dcb = m.fc_bias.projections[-1].shape[0]
+        # the CPG workspace is kept apart: the backward reuses the operands the forward prepared in it
+        ws_cpg = max(lib.coper_cpg_fc_fwd_workspace_bytes(B, dcw, F, d, m.prec),
+                     lib.coper_cpg_fc_bwd_workspace_bytes(B, dcw, F, d, m.prec))
+        self.ws_cpg = torch.empty(ws_cpg, dtype=torch.uint8, device=dev)
+        self.ws_cpg_bytes = ws_cpg
+        ws = max(lib.coper_score1n_bce_workspace_bytes(B, Ns, d, m.prec),
+                 lib.coper_score1n_workspace_bytes(B, Ns, d, m.prec),
+                 lib.coper_segscatter_workspace_bytes(B), lib.coper_score1n_rank_workspace_bytes(B, d, m.prec))
+        self.ws = torch.empty(ws, dtype=torch.uint8, device=dev)
+        self.ws_bytes = ws
+        # context nets: activations per hidden layer for the two generators
+        self.ctx = {}
+        for cpg in m.generators:
+            self.ctx[cpg.name] = {"pre": [z(B, n) for n in cpg.hidden], "act": [z(B, n) for n in cpg.hidden],
+                                  "dact": [z(B, n) for n in cpg.hidden], "dpre": [z(B, n) for n in cpg.hidden]}
+        self.dcw, self.dcb = z(B, dcw), z(B, dcb)
+        # contexts the forward pass used for the FC weights / bias and the conv filter / bias generators
+        self.cw = self.cb = self.ccw = self.ccb = None
+        # per-query filters [B, KH*KW*C], biases [B, C], context gradients (generated conv filters)
+        self.wq = self.bq = self.dccw = self.dccb = None
+        if m.conv_w_gen is not None:
+            KK = m.conv_filter_height * m.conv_filter_width * C
+            self.wq, self.bq = z(B, KK), z(B, C)
+            self.dccw = z(B, m.conv_w_gen.projections[-1].shape[0])
+            self.dccb = z(B, m.conv_b_gen.projections[-1].shape[0])
+        self.xc = self.dxc = self.cconst = None
+        self.f_sq = self.dy_sq = self.df_scratch = None
+        if m.variant == "plain":          # the stacked [entity image; relation image] and its gradient
+            self.xc, self.dxc = z(B, d + dr), z(B, d + dr)
+            self.cconst = torch.ones(B, 1, dtype=f32, device=dev)
+        if m.variant == "param_lookup":   # one-hot(rel) context; squared operands of the slice-wise bookkeeping
+            self.cconst = z(B, m.num_rel)
+            self.f_sq, self.dy_sq, self.df_scratch = z(B, F), z(B, d), z(B, F)
+        self.dx0_sq = z(B, d) if m.use_negative_sampling else None
+        self.dr_sq = z(B, dr)
+        # sub-slots, each built once per key: sampled labels (by L), top-k (by k), given candidates (by C)
+        self.samp: Dict[int, _SampledSlot] = {}
+        self.topk: Dict[int, _TopkSlot] = {}
+        self.cand: Dict[int, _CandSlot] = {}
+        # the sampled-label step: its [B, L] sub-slot and (num_labels, prop_negatives) when drawn on the device
+        self.cur_samp, self.cur_sampling = None, None
+        # pinned staging for host batches; csr_gen counts reallocations of col (graphs that captured the old pointer
+        # must not be replayed)
+        self.csr_cap, self.csr_gen = 0, 0
+        self.rowptr = self.d_head[6 * B:6 * B + B + 1]
+        self.col = self.h_col = self.h_col_np = None
+        self.h2d_event = None
+
+
+class _SampledSlot:
+    """[B, L] lookup ids / labels of the sampled-label step, their pinned staging, scores, dL/dS and workspace."""
+
+    def __init__(self, m: "ConvE", B: int, L: int):
+        f = dict(dtype=torch.float32, device=m.dev)
+        self.L = L
+        self.lookup = torch.zeros(B, L, dtype=torch.int32, device=m.dev)
+        self.labels, self.scores, self.g = (torch.zeros(B, L, **f) for _ in range(3))
+        self.h_lookup = torch.zeros(B, L, dtype=torch.int32).pin_memory()
+        self.h_labels = torch.zeros(B, L, dtype=torch.float32).pin_memory()
+        lib = _lib.load()
+        nbytes = lib.coper_score_sampled_sharded_workspace_bytes(B, L) if m.world > 1 else \
+            lib.coper_score_sampled_workspace_bytes(B, L)
+        self.ws = torch.empty(nbytes, dtype=torch.uint8, device=m.dev)
+
+
+class _TopkSlot:
+    """(B, k) outputs of predict_topk, the scorer's workspace and, under entity sharding, the per-rank lists."""
+
+    def __init__(self, m: "ConvE", B: int, k: int):
+        lib, dev, P = _lib.load(), m.dev, m.world
+        self.scores = torch.empty(B, k, dtype=torch.float32, device=dev)
+        self.ids = torch.empty(B, k, dtype=torch.int64, device=dev)
+        if m.E_prep is not None:
+            self.ws_bytes = lib.coper_score1n_topk_workspace_bytes(B, m.shard.rows, m.ent_emb_size, k, m.prec)
+        else:
+            self.ws_bytes = lib.coper_topk_scores_workspace_bytes(B, m.shard.rows, k)
+        self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
+        self.local_scores = self.local_ids = self.all_scores = self.all_ids = None
+        if P > 1:        # this rank's list, and every rank's list after the exchange
+            self.local_scores, self.local_ids = torch.empty_like(self.scores), torch.empty_like(self.ids)
+            self.all_scores = torch.empty(P, B, k, dtype=torch.float32, device=dev)
+            self.all_ids = torch.empty(P, B, k, dtype=torch.int64, device=dev)
+
+
+class _CandSlot:
+    """(B, C) slot: int32 [B, C] candidates followed by the [B] gold ids in one device block, staged through one
+    pinned host block (one copy per call), the [B, C] scores and the rank outputs."""
+
+    def __init__(self, m: "ConvE", B: int, C: int):
+        dev = m.dev
+        self.C = C
+        self.d_ids = torch.zeros(B * C + B, dtype=torch.int32, device=dev)
+        self.cand, self.e2 = self.d_ids[:B * C].view(B, C), self.d_ids[B * C:]
+        self.h_ids = torch.zeros(B * C + B, dtype=torch.int32).pin_memory()
+        self.h_np = self.h_ids.numpy()
+        self.scores = torch.zeros(B, C, dtype=torch.float32, device=dev)
+        self.gold = torch.zeros(B, dtype=torch.float32, device=dev)
+        self.counts = torch.zeros(2, B, dtype=torch.int32, device=dev)
+        self.n_greater, self.n_equal = self.counts[0], self.counts[1]
+        self.rank = torch.zeros(B, dtype=torch.int32, device=dev)
+
+
+def _slot(table: Dict, key, cls, *args):
+    """table[key], built as cls(*args) on first use (exactly once: captured graphs keep valid pointers)."""
+    if key not in table:
+        table[key] = cls(*args)
+    return table[key]
+
+
 class ConvE:
     def __init__(self, model_descriptors: Dict, device: Optional[str] = None, seed: int = 0, prec: str = "fp32",
                  shard: Optional[EntityShard] = None, reference_bug_compat: bool = True,
@@ -304,7 +473,7 @@ class ConvE:
             tr.append((nm + "/beta", bn.beta, False))
         self.trainables = tr
         self.grads = {n: torch.zeros_like(p) for n, p, _ in tr}
-        if getattr(self, "dp", False):
+        if self.dp:
             # gradients that every rank only holds a partial sum of (its own rows of the batch) live in ONE flat
             # buffer; BN gamma / beta gradients come out of the synchronised statistics and the entity-table
             # gradients are row-sharded: neither is in the bucket.  The generator's last projection (dc*F*d floats,
@@ -338,7 +507,7 @@ class ConvE:
             # sampled labels (models.py:438-443): ent_emb / pred_bias are read only through gathers as well
             self.sparse_vars |= {"ent_emb", "pred_bias"}
         self.grad_sq = {n: torch.zeros_like(p) for n, p, _ in tr if n in self.sparse_vars}
-        if getattr(self, "dp", False):
+        if self.dp:
             self.grad_sq["rel_emb"] = self._flat_gsq_rel
         if not self.bug_compat:
             self.m = {n: torch.zeros_like(p) for n, p, _ in tr}
@@ -360,9 +529,7 @@ class ConvE:
             self.P_prep = torch.zeros(lib.coper_prepared_bytes(Pw.shape[0] * self.F, d, self.prec), dtype=torch.uint8,
                                       device=self.dev)
         # multi-tensor work list (include/coper.h: coper_param_desc, COPER_MT_CHUNK)
-        desc = np.zeros(len(tr), dtype=np.dtype([("theta", "<u8"), ("grad", "<u8"), ("m", "<u8"), ("v", "<u8"),
-                                                 ("vhat", "<u8"), ("prepared", "<u8"), ("grad_sq", "<u8"),
-                                                 ("n", "<i8"), ("prepared_prec", "<i4"), ("mode", "<i4")]))
+        desc = np.zeros(len(tr), dtype=_lib.PARAM_DESC)
         chunks, offsets = [], [0]
         last_w = self._last_w_name
         for i, (n, p, _) in enumerate(tr):
@@ -499,101 +666,8 @@ class ConvE:
 
     # ------------------------------------------------------------------------------------------
     def _buffers(self, B: int, key=None):
-        """Static per-batch-size device buffers (pointer-stable -> CUDA-graph friendly)."""
-        key = B if key is None else key
-        if key in self._bufs:
-            return self._bufs[key]
-        dev, f32 = self.dev, torch.float32
-        d, dr, F, C = self.ent_emb_size, self.rel_emb_size, self.F, self.C
-        Ns = self.shard.rows
-        ld = -(-Ns // 32) * 32
-        words = -(-Ns // 32)
-        z = lambda *s, dt=f32: torch.zeros(*s, dtype=dt, device=dev)
-        lib = _lib.load()
-        b = type("Buf", (), {})()
-        b.B, b.ld, b.words = B, ld, words
-        # query ids + CSR row pointers live in ONE device block so that a host batch needs one H2D copy for them:
-        # [e1 | rel | e2] int64 [3, B] followed by rowptr int32 [B + 1]
-        head_words = 6 * B + (B + 2)
-        b.d_head = z(head_words, dt=torch.int32)
-        b.h_head = torch.zeros(head_words, dtype=torch.int32).pin_memory()
-        idx64 = b.d_head[:6 * B].view(torch.int64).view(3, B)
-        b.e1, b.rel, b.e2 = idx64[0], idx64[1], idx64[2]
-        b.h_head_np = b.h_head.numpy()
-        b.h_idx_np = b.h_head_np[:6 * B].view(np.int64).reshape(3, B)
-        b.h_rowptr_np = b.h_head_np[6 * B:6 * B + B + 1]
-        b.x0, b.r = z(B, d), z(B, dr)
-        Fc = self.F_conv
-        b.z, b.f = z(B, Fc), z(B, F)
-        # concat_rel: the conv block works on contiguous [B, F_conv] buffers; b.f / b.df hold [conv features | rel_emb]
-        b.fconv, b.dfconv = (z(B, Fc), z(B, Fc)) if self.concat_rel else (b.f, None)
-        b.y, b.q = z(B, d), z(B, d)
-        b.q_prep = None
-        if self.E_prep is not None:
-            b.q_prep = torch.zeros(lib.coper_prepared_bytes(B, d, self.prec), dtype=torch.uint8, device=dev)
-        b.dq, b.dy, b.df, b.dz, b.dx0, b.dr = z(B, d), z(B, d), z(B, F), z(B, Fc), z(B, d), z(B, dr)
-        if not self.concat_rel:
-            b.dfconv = b.df
-        R1 = B * self.OH * self.OW
-        nch = max(lib.coper_colstats_chunks(R1), lib.coper_colstats_chunks(B))
-        maxC = max([C, d] + [n for gcp in self.generators for n in gcp.hidden])
-        b.stat = z(nch * maxC * 2)
-        b.stat1 = z(maxC * 2)
-        # allocated on first use (each exactly once, so captured graphs keep valid pointers):
-        #   b.S  logits fp32 [B, ld] (predict_all / the two-pass ranking of the fp32 engine)
-        #   b.G  dL/dS in the scorer's operand form (train); never read by the host
-        b.S = b.G = None
-        # label / filter bits: query-major rows for the fp32 engine, the entity-major matrix for the tensor pipe
-        b.bits = z(B, words, dt=torch.int32) if self.prec == 0 else None
-        b.bitsT = z(max(Ns, 1), -(-B // 32), dt=torch.int32) if self.prec != 0 else None
-        b.loss_sum = z(1, dt=torch.float64)
-        b.gold = z(B)
-        b.rank_counts = z(2, B, dt=torch.int32)       # one buffer: cleared by one fill per evaluation batch
-        b.n_greater, b.n_equal = b.rank_counts[0], b.rank_counts[1]
-        b.rank = z(B, dt=torch.int32)
-        b.loss_mean = z(1, dt=torch.float64)
-        b.dwc_part, b.dbc_part = z(B, self.conv_filter_height * self.conv_filter_width * C), z(B, C)
-        dcw = self.fc_weights.projections[-1].shape[0]
-        dcb = self.fc_bias.projections[-1].shape[0]
-        # the CPG workspace is kept apart: the backward reuses the operands the forward prepared in it
-        ws_cpg = max(lib.coper_cpg_fc_fwd_workspace_bytes(B, dcw, F, d, self.prec),
-                     lib.coper_cpg_fc_bwd_workspace_bytes(B, dcw, F, d, self.prec))
-        b.ws_cpg = torch.empty(ws_cpg, dtype=torch.uint8, device=dev)
-        b.ws_cpg_bytes = ws_cpg
-        ws = max(lib.coper_score1n_bce_workspace_bytes(B, Ns, d, self.prec),
-                 lib.coper_score1n_workspace_bytes(B, Ns, d, self.prec),
-                 lib.coper_segscatter_workspace_bytes(B), lib.coper_score1n_rank_workspace_bytes(B, d, self.prec))
-        b.ws = torch.empty(ws, dtype=torch.uint8, device=dev)
-        b.ws_bytes = ws
-        # context nets: activations per hidden layer for the two generators
-        b.ctx = {}
-        for cpg in self.generators:
-            b.ctx[cpg.name] = {"pre": [z(B, n) for n in cpg.hidden], "act": [z(B, n) for n in cpg.hidden],
-                               "dact": [z(B, n) for n in cpg.hidden], "dpre": [z(B, n) for n in cpg.hidden]}
-        b.dcw, b.dcb = z(B, dcw), z(B, dcb)
-        if self.conv_w_gen is not None:      # per-query filters [B, KH*KW*C], biases [B, C], context gradients
-            KK = self.conv_filter_height * self.conv_filter_width * C
-            b.wq, b.bq = z(B, KK), z(B, C)
-            b.dccw = z(B, self.conv_w_gen.projections[-1].shape[0])
-            b.dccb = z(B, self.conv_b_gen.projections[-1].shape[0])
-        if self.variant == "plain":          # the stacked [entity image; relation image] and its gradient
-            b.xc, b.dxc = z(B, d + dr), z(B, d + dr)
-            b.cconst = torch.ones(B, 1, dtype=f32, device=dev)
-        if self.variant == "param_lookup":   # one-hot(rel) context; squared operands of the slice-wise bookkeeping
-            b.cconst = z(B, self.num_rel)
-            b.f_sq, b.dy_sq, b.df_scratch = z(B, F), z(B, d), z(B, F)
-        b.dr2 = z(B, dr)
-        b.dx0_sq = z(B, d) if self.use_negative_sampling else None
-        b.samp = {}                                  # per-L buffers of the sampled-label path
-        b.dr_sq = z(B, dr)
-        # pinned staging for host batches
-        b.csr_cap = 0
-        b.rowptr = b.d_head[6 * B:6 * B + B + 1]
-        b.col = None
-        b.h_col = None
-        b.h2d_event = None
-        self._bufs[key] = b
-        return b
+        """The batch slot of batch size B (key: the slot's name in ``_bufs``, default B)."""
+        return _slot(self._bufs, B if key is None else key, _BatchSlot, self, B)
 
     def _local_buffers(self, bg):
         """Data-parallel front end: buffer set of this rank's Bg/P rows; its query ids alias the global batch."""
@@ -620,7 +694,7 @@ class ConvE:
         if b.csr_cap < nnz:
             cap = max(1024, int(nnz * 1.5))
             b.col = torch.zeros(cap, dtype=torch.int32, device=self.dev)
-            b.csr_gen = getattr(b, "csr_gen", 0) + 1     # graphs that captured the old pointer must not be replayed
+            b.csr_gen += 1
             b.h_col = torch.zeros(cap, dtype=torch.int32).pin_memory()
             b.h_col_np = b.h_col.numpy()
             b.csr_cap = cap
@@ -672,9 +746,7 @@ class ConvE:
                 call("coper_csr_to_bits_t", ptr(b.rowptr), ptr(b.col), B, s.lo, s.hi, ptr(b.bitsT))
         elif not on_device:
             b.d_head[:6 * B].copy_(b.h_head[:6 * B], non_blocking=True)
-        if has_csr:
-            pass
-        elif "e2_multi" in batch and batch["e2_multi"] is not None:
+        if not has_csr and batch.get("e2_multi") is not None:
             dense = batch["e2_multi"]
             if not (isinstance(dense, torch.Tensor) and dense.is_cuda):
                 dense = torch.as_tensor(np.asarray(dense), dtype=torch.float32).to(self.dev, non_blocking=True)
@@ -739,7 +811,7 @@ class ConvE:
                  ptr(bn.c1), ptr(bn.c2), int(relu), keep_post, ptr(self.seed_dev), salt_post, keep_pre, salt_pre, ptr(dx))
 
     def _gather_stats(self, b, n):
-        if getattr(b, "stat_all", None) is None:
+        if b.stat_all is None:
             b.stat_all = torch.zeros(self.world * b.stat.numel(), dtype=torch.float32, device=self.dev)
         return sharding.gather_stat_partials(b.stat_all[:self.world * n], b.stat[:n], self.world, self.group)
 
@@ -869,16 +941,20 @@ class ConvE:
         self._front_end(bl, is_train)
         sharding.gather_batch(bg.q, bl.q, self.world, self.group)
 
-    def _train_device(self, b):
-        """fwd + bwd + clip + AMSGrad on staged buffers; everything is enqueued, nothing syncs."""
-        if self.dp:
-            return self._train_device_dp(b)
-        self._train_device_impl(b, b)
+    def _eval_q(self, b):
+        """Evaluation forward pass: q of every query of b (moving statistics, no dropout).  A batch that does not split
+        evenly over the ranks runs the data-parallel front end replicated, with identical results."""
+        if self.dp and b.B % self.world == 0:
+            self._forward_q_dp(b, self._local_buffers(b), False)
+        else:
+            self._forward_q(b, False)
 
-    def _train_device_dp(self, bg):
-        self._train_device_impl(bg, self._local_buffers(bg))
+    def _train_device(self, b, apply: bool = True):
+        """fwd + bwd (+ clip + AMSGrad when apply) on staged buffers; everything is enqueued, nothing syncs.
+        apply=False leaves the gradients for a later _clip_and_apply()."""
+        self._train_device_impl(b, self._local_buffers(b) if self.dp else b, apply)
 
-    def _train_device_impl(self, bg, b):
+    def _train_device_impl(self, bg, b, apply):
         """bg: buffers of the batch the scorer sees; b: buffers of the rows this rank's front end owns
         (b is bg unless the front end is data-parallel)."""
         dp = b is not bg
@@ -1019,22 +1095,17 @@ class ConvE:
         if self._side_pending:      # join: the scatter below adds into dE, the clip reads every gradient
             torch.cuda.current_stream().wait_stream(self._side)
             self._side_pending = False
-        pair = bg.B <= 4096 and small and self.rel_emb is not None
-        if pair:      # head-entity and relation scatters: one launch
-            if not rel_cleared:
-                g["rel_emb"].zero_()
-                self.grad_sq["rel_emb"].zero_()
+        rel = self.rel_emb is not None
+        if rel and not rel_cleared:
+            g["rel_emb"].zero_()
+            self.grad_sq["rel_emb"].zero_()
+        if bg.B <= 4096:      # head-entity scatter, with the relation scatter as its second job: one launch
+            rel_job = (ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), ptr(self.grad_sq["rel_emb"]), 0, self.num_rel) \
+                if rel else (None, 0, None, 0, None, None, 0, 0)
             call("coper_segscatter_add_pair", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), ptr(gsq_e), s.lo, s.hi,
-                 ptr(self.norm_delta) if self._norm_fused_now else None, ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]),
-                 ptr(self.grad_sq["rel_emb"]), 0, self.num_rel)
+                 ptr(self.norm_delta) if self._norm_fused_now else None, *rel_job)
             if self._norm_fused_now:
                 self._norm_delta_n = bg.B
-        elif self._norm_fused_now:
-            call("coper_segscatter_add_norm", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), ptr(gsq_e), s.lo, s.hi,
-                 ptr(self.norm_delta))
-            self._norm_delta_n = bg.B
-        elif bg.B <= 4096:
-            call("coper_segscatter_add_sq", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), ptr(gsq_e), s.lo, s.hi)
         else:
             call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), s.lo, s.hi, ptr(bg.ws),
                  bg.ws_bytes)
@@ -1042,18 +1113,10 @@ class ConvE:
                 torch.mul(bg.dx0, bg.dx0, out=bg.dx0_sq)
                 call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0_sq), d, ptr(gsq_e), s.lo, s.hi, ptr(bg.ws),
                      bg.ws_bytes)
-        if self.rel_emb is None:
-            if dp:
-                raise NotImplementedError
-            return self._clip_and_apply()
-        if not pair:
-            if not rel_cleared:
-                g["rel_emb"].zero_()
-                self.grad_sq["rel_emb"].zero_()
-            if small:
+            if rel and small:
                 call("coper_segscatter_add_sq", ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]),
                      ptr(self.grad_sq["rel_emb"]), 0, self.num_rel)
-            else:
+            elif rel:
                 call("coper_segscatter_add", ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), 0, self.num_rel, ptr(b.ws),
                      b.ws_bytes)
                 torch.mul(b.dr, b.dr, out=b.dr_sq)
@@ -1065,23 +1128,8 @@ class ConvE:
                 big_work.wait()
             else:
                 sharding.reduce_replicated_grads(self.flat_grads, self.world, self.group)
-        self._clip_and_apply()
-
-    def _sampled_buffers(self, b, L):
-        if L not in b.samp:
-            f = dict(dtype=torch.float32, device=self.dev)
-            sb = type("Samp", (), {})()
-            sb.L = L
-            sb.lookup = torch.zeros(b.B, L, dtype=torch.int32, device=self.dev)
-            sb.labels, sb.scores, sb.g = (torch.zeros(b.B, L, **f) for _ in range(3))
-            sb.h_lookup = torch.zeros(b.B, L, dtype=torch.int32).pin_memory()
-            sb.h_labels = torch.zeros(b.B, L, dtype=torch.float32).pin_memory()
-            lib = _lib.load()
-            nbytes = lib.coper_score_sampled_sharded_workspace_bytes(b.B, L) if self.world > 1 else \
-                lib.coper_score_sampled_workspace_bytes(b.B, L)
-            sb.ws = torch.empty(nbytes, dtype=torch.uint8, device=self.dev)
-            b.samp[L] = sb
-        return b.samp[L]
+        if apply:
+            self._clip_and_apply()
 
     def _sampled_scorer(self, b):
         """models.py:438-443 + 448-453 on the staged [B, L] lookup ids / labels (b.cur_samp).  Entity-sharded: every
@@ -1171,18 +1219,18 @@ class ConvE:
         if self.use_negative_sampling:
             return self._train_step_sampled(batch, apply_update)
         b = self.stage_batch(batch)
-        if not apply_update:
-            saved = self._clip_and_apply
-            self._clip_and_apply = lambda: None
-            self._launch_mode()
-            try:
-                self._train_device(b)
-            finally:
-                self._clip_and_apply = saved
-        else:
-            self._run_graphed(("train", b.B), lambda: self._train_device(b))
-        self.global_step += 1
+        self._run_train(("train", b.B), b, apply_update)
         return b.loss_mean[0]
+
+    def _run_train(self, key, b, apply: bool):
+        """The device step on staged buffers b: graphed when it applies the update, eager when it only computes the
+        gradients (the caller applies them later with _clip_and_apply)."""
+        if apply:
+            self._run_graphed(key, lambda: self._train_device(b))
+        else:
+            self._launch_mode()
+            self._train_device(b, apply=False)
+        self.global_step += 1
 
     def _train_step_sampled(self, batch: Dict, apply_update: bool):
         """Sampled-label step: ``batch['lookup_values']`` int32 [B, L] entity ids and ``batch['e2_multi']`` fp32 [B, L]
@@ -1197,7 +1245,7 @@ class ConvE:
                                  "and 0 < num_labels <= num_ent")
             b = self.stage_batch({k: batch[k] for k in ("e1", "rel", "e2", "e2_multi_rowptr", "e2_multi_col")
                                   if k in batch})
-            sb = self._sampled_buffers(b, L)
+            sb = _slot(b.samp, L, _SampledSlot, self, b.B, L)
             b.cur_sampling = (L, float(sampling[1]))
         else:
             lookup, labels = batch["lookup_values"], batch["e2_multi"]
@@ -1206,7 +1254,8 @@ class ConvE:
                 raise ValueError("sampled-label training needs lookup_values [B, L] and e2_multi [B, L] "
                                  "(L = num_labels)")
             b = self.stage_batch({k: batch[k] for k in ("e1", "rel", "e2") if k in batch})
-            sb = self._sampled_buffers(b, int(lookup.shape[1]))
+            L = int(lookup.shape[1])
+            sb = _slot(b.samp, L, _SampledSlot, self, b.B, L)
             b.cur_sampling = None
             for src, dev_t, host_t, dt in ((lookup, sb.lookup, sb.h_lookup, torch.int32),
                                           (labels, sb.labels, sb.h_labels, torch.float32)):
@@ -1217,28 +1266,14 @@ class ConvE:
                     dev_t.copy_(host_t, non_blocking=True)
         b.h2d_event.record()
         b.cur_samp = sb
-        if not apply_update:
-            saved = self._clip_and_apply
-            self._clip_and_apply = lambda: None
-            self._launch_mode()
-            try:
-                self._train_device(b)
-            finally:
-                self._clip_and_apply = saved
-        else:
-            key = ("train_sampled", b.B, sb.L, b.cur_sampling, getattr(b, "csr_gen", 0) if b.cur_sampling else 0)
-            self._run_graphed(key, lambda: self._train_device(b))
-        self.global_step += 1
+        self._run_train(("train_sampled", b.B, L, b.cur_sampling, b.csr_gen if b.cur_sampling else 0), b, apply_update)
         return b.loss_sum[0] / (float(b.B) * float(sb.L))
 
     def predict_all(self, batch: Dict):
         """Logits of every query against this rank's entity rows: [B, rows] view (metrics.py:40-42)."""
         b = self.stage_batch(batch)
         self._launch_mode()
-        if self.dp and b.B % self.world == 0:
-            self._forward_q_dp(b, self._local_buffers(b), False)
-        else:
-            self._forward_q(b, False)
+        self._eval_q(b)
         self._score(b)
         return b.S[:, :self.shard.rows]
 
@@ -1256,40 +1291,16 @@ class ConvE:
             raise ValueError("k must be in [1, %d], got %d" % (_lib.TOPK_MAX, k))
         keys = ("e1", "rel")
         if filtered:
-            if "e2_multi_rowptr" not in batch and batch.get("e2_multi") is None:
+            if not has_known_tails(batch):
                 raise ValueError("filtered top-k needs the known true tails: e2_multi, or e2_multi_rowptr / e2_multi_col")
             keys += ("e2_multi_rowptr", "e2_multi_col", "e2_multi")
         b = self.stage_batch({key: batch[key] for key in keys if key in batch})
-        t = self._topk_buffers(b, k)
+        t = _slot(b.topk, k, _TopkSlot, self, b.B, k)
         self._run_graphed(("topk", b.B, k, bool(filtered)), lambda: self._topk_device(b, t, filtered))
         return t.scores, t.ids
 
-    def _topk_buffers(self, b, k):
-        if not hasattr(b, "topk"):
-            b.topk = {}
-        if k in b.topk:
-            return b.topk[k]
-        lib, dev, B, P = _lib.load(), self.dev, b.B, self.world
-        t = type("TopkBuf", (), {})()
-        t.scores = torch.empty(B, k, dtype=torch.float32, device=dev)
-        t.ids = torch.empty(B, k, dtype=torch.int64, device=dev)
-        if self.E_prep is not None:
-            t.ws_bytes = lib.coper_score1n_topk_workspace_bytes(B, self.shard.rows, self.ent_emb_size, k, self.prec)
-        else:
-            t.ws_bytes = lib.coper_topk_scores_workspace_bytes(B, self.shard.rows, k)
-        t.ws = torch.empty(t.ws_bytes, dtype=torch.uint8, device=dev)
-        if P > 1:        # this rank's list, and every rank's list after the exchange
-            t.local_scores, t.local_ids = torch.empty_like(t.scores), torch.empty_like(t.ids)
-            t.all_scores = torch.empty(P, B, k, dtype=torch.float32, device=dev)
-            t.all_ids = torch.empty(P, B, k, dtype=torch.int64, device=dev)
-        b.topk[k] = t
-        return t
-
     def _topk_device(self, b, t, filtered):
-        if self.dp and b.B % self.world == 0:
-            self._forward_q_dp(b, self._local_buffers(b), False)
-        else:
-            self._forward_q(b, False)
+        self._eval_q(b)
         s, d, k = self.shard, self.ent_emb_size, t.scores.shape[1]
         out_s, out_i = (t.local_scores, t.local_ids) if self.world > 1 else (t.scores, t.ids)
         if self.E_prep is not None:
@@ -1320,23 +1331,22 @@ class ConvE:
         ``batch['e2_multi*']`` is the filter set (all known true tails).  Returns int32 device tensors
         (rank, n_equal); rank == the reference's rank whenever n_equal == 0.  Both are buffers of the batch-size slot,
         overwritten by the next call with the same batch size (clone them to keep them, as metrics.py does)."""
-        if not (isinstance(batch["e2"], torch.Tensor) and batch["e2"].is_cuda):   # host batches are validated
-            e2 = np.asarray(batch["e2"])
-            if int(e2.min()) < 0 or int(e2.max()) >= self.num_ent:
-                raise ValueError("e2 out of range (train rows carry e2 = -1 in the reference; SURVEY Q17)")
+        self._check_e2(batch["e2"])
         b = self.stage_batch(batch, need_e2=True)
         if self.prec != 0:          # the gold entity joins the filter set (metrics.py:44-46 never compares it)
             call("coper_bits_t_set", ptr(b.e2), b.B, self.shard.lo, self.shard.hi, ptr(b.bitsT))
         self._run_graphed(("rank", b.B), lambda: self._rank_device(b))
         return b.rank, b.n_equal
 
+    def _check_e2(self, e2):
+        """Host gold tails must be entity ids (device ones are taken as they are)."""
+        if not (isinstance(e2, torch.Tensor) and e2.is_cuda):
+            e2 = np.asarray(e2)
+            if int(e2.min()) < 0 or int(e2.max()) >= self.num_ent:
+                raise ValueError("e2 out of range (train rows carry e2 = -1 in the reference; SURVEY Q17)")
+
     def _rank_device(self, b):
-        # (evaluation uses moving statistics and no dropout: a batch that does not split evenly over the ranks simply
-        # runs the front end replicated, with identical results)
-        if self.dp and b.B % self.world == 0:
-            self._forward_q_dp(b, self._local_buffers(b), False)
-        else:
-            self._forward_q(b, False)
+        self._eval_q(b)
         s = self.shard
         d = self.ent_emb_size
         b.rank_counts.zero_()
@@ -1380,40 +1390,16 @@ class ConvE:
         ``filtered=False`` excludes only the gold entity itself.  Scores as in ``score_candidates``.  Returns int32
         device tensors (rank, n_equal) [B], buffers of the (B, C) slot, overwritten by the next call with the same B
         and C (clone them to keep them)."""
-        if not (isinstance(batch["e2"], torch.Tensor) and batch["e2"].is_cuda):
-            e2 = np.asarray(batch["e2"])
-            if int(e2.min()) < 0 or int(e2.max()) >= self.num_ent:
-                raise ValueError("e2 out of range (train rows carry e2 = -1 in the reference; SURVEY Q17)")
+        self._check_e2(batch["e2"])
         keys = ("e1", "rel", "e2")
         if filtered:
-            if "e2_multi_rowptr" not in batch and batch.get("e2_multi") is None:
+            if not has_known_tails(batch):
                 raise ValueError("filtered candidate ranks need the known true tails: e2_multi, or e2_multi_rowptr / "
                                  "e2_multi_col")
             keys += ("e2_multi_rowptr", "e2_multi_col", "e2_multi")
         b, c = self._stage_candidates({k: batch[k] for k in keys if k in batch}, candidates, with_e2=True)
         self._run_graphed(("cand_rank", b.B, c.C, bool(filtered)), lambda: self._cand_rank_device(b, c, filtered))
         return c.rank, c.n_equal
-
-    def _cand_buffers(self, b, C):
-        """(B, C) slot: int32 [B, C] candidates followed by the [B] gold ids in one device block, staged through one
-        pinned host block (one copy per call), the [B, C] scores and the rank outputs."""
-        if not hasattr(b, "cand"):
-            b.cand = {}
-        if C not in b.cand:
-            B, dev = b.B, self.dev
-            t = type("CandBuf", (), {})()
-            t.C = C
-            t.d_ids = torch.zeros(B * C + B, dtype=torch.int32, device=dev)
-            t.cand, t.e2 = t.d_ids[:B * C].view(B, C), t.d_ids[B * C:]
-            t.h_ids = torch.zeros(B * C + B, dtype=torch.int32).pin_memory()
-            t.h_np = t.h_ids.numpy()
-            t.scores = torch.zeros(B, C, dtype=torch.float32, device=dev)
-            t.gold = torch.zeros(B, dtype=torch.float32, device=dev)
-            t.counts = torch.zeros(2, B, dtype=torch.int32, device=dev)
-            t.n_greater, t.n_equal = t.counts[0], t.counts[1]
-            t.rank = torch.zeros(B, dtype=torch.int32, device=dev)
-            b.cand[C] = t
-        return b.cand[C]
 
     def _stage_candidates(self, batch, candidates, with_e2):
         on_device = isinstance(candidates, torch.Tensor) and candidates.is_cuda
@@ -1425,7 +1411,7 @@ class ConvE:
             raise ValueError("candidate ids must lie in [0, %d) or be -1 (padding)" % self.num_ent)
         b = self.stage_batch(batch)             # e1, rel and the filter bits; e2 travels in the candidate block
         B, C = b.B, int(candidates.shape[1])
-        c = self._cand_buffers(b, C)
+        c = _slot(b.cand, C, _CandSlot, self, B, C)
         # each region of the block comes from where its ids live; two host regions travel in one copy
         e2 = batch["e2"] if with_e2 else None
         e2_on_device = isinstance(e2, torch.Tensor) and e2.is_cuda
@@ -1446,12 +1432,6 @@ class ConvE:
             c.e2.copy_(c.h_ids[B * C:], non_blocking=True)
         b.h2d_event.record()               # the next stage_batch waits for this copy before reusing pinned memory
         return b, c
-
-    def _eval_q(self, b):
-        if self.dp and b.B % self.world == 0:
-            self._forward_q_dp(b, self._local_buffers(b), False)
-        else:
-            self._forward_q(b, False)
 
     def _cand_score_device(self, b, c):
         s = self.shard

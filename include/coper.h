@@ -419,13 +419,12 @@ size_t coper_segscatter_workspace_bytes(int M);
  * Same summation order (index order) as coper_segscatter_add, which uses this path for small M. */
 int coper_segscatter_add_sq(const int64_t* idx, int M, const float* src, int width, float* dst, float* dst_sq,
                             int64_t row_lo, int64_t row_hi, coper_stream_t stream);
-/* coper_segscatter_add_sq that also reports, per position i of idx, norm_delta[i] = sum_c (new^2 - old^2) over the
- * destination row position i updated (0 for non-heads / rows of other shards): the correction of a squared gradient
- * norm that was taken before this scatter (tf.clip_by_global_norm over the dense ent_emb gradient, models.py:198-199). */
-int coper_segscatter_add_norm(const int64_t* idx, int M, const float* src, int width, float* dst, float* dst_sq,
-                              int64_t row_lo, int64_t row_hi, double* norm_delta, coper_stream_t stream);
-/* Two independent small scatters of one step in ONE launch: a = coper_segscatter_add_norm's arguments (norm_delta_a may
- * be NULL), b = coper_segscatter_add_sq's (the head-entity and relation gathers' gradients, models.py:176-178). */
+/* Two independent small scatters of one step in ONE launch, each with coper_segscatter_add_sq's arguments (the
+ * head-entity and relation gathers' gradients, models.py:176-178).  M_b == 0: job a alone (idx_b, src_b, dst_b may be
+ * NULL).  norm_delta_a (NULL = skip) receives, per position i of idx_a, norm_delta_a[i] = sum_c (new^2 - old^2) over
+ * the destination row position i updated (0 for non-heads / rows of other shards): the correction of a squared
+ * gradient norm that was taken before this scatter (tf.clip_by_global_norm over the dense ent_emb gradient,
+ * models.py:198-199). */
 int coper_segscatter_add_pair(const int64_t* idx_a, int M_a, const float* src_a, int width_a, float* dst_a,
                               float* dst_sq_a, int64_t lo_a, int64_t hi_a, double* norm_delta_a, const int64_t* idx_b,
                               int M_b, const float* src_b, int width_b, float* dst_b, float* dst_sq_b, int64_t lo_b,
@@ -488,7 +487,7 @@ int coper_amsgrad_step(float* theta, const float* grad, float* m, float* v, floa
 /* COPER_GRAD_NORM_EXTERNAL (OR-ed into mode): coper_mt_sumsq does not read this gradient - its squared norm is written
  * into tensor_sumsq[t] by coper_sumsq_combine AFTER coper_mt_sumsq, from the partial sums the kernel that produced the
  * gradient emitted (coper_score1n_bce_fwd_bwd_norm) and the corrections of the scatter that touched it afterwards
- * (coper_segscatter_add_norm): the [N, d] entity gradient is then read once (by the update), not twice. */
+ * (coper_segscatter_add_pair's norm_delta_a): the [N, d] entity gradient is then read once (by the update), not twice. */
 enum { COPER_GRAD_DENSE = 0, COPER_GRAD_INDEXED_SLICES = 1, COPER_GRAD_NORM_EXTERNAL = 2 };
 typedef struct {
   float* theta;

@@ -389,9 +389,7 @@ def test_multi_tensor_optimizer_matches_per_tensor(L, bug_compat):
     th2, vh2, m2, v2 = ([t.clone() for t in x] for x in (th, vh, m, v))
     prep = {0: (1, torch.zeros(lib.coper_prepared_bytes(40943, 200, 1), dtype=torch.uint8, device="cuda")),
             4: (2, torch.zeros(lib.coper_prepared_bytes(8 * 4608, 40, 2), dtype=torch.uint8, device="cuda"))}
-    desc = np.zeros(len(shapes), dtype=np.dtype([("theta", "<u8"), ("grad", "<u8"), ("m", "<u8"), ("v", "<u8"),
-                                                 ("vhat", "<u8"), ("prepared", "<u8"), ("grad_sq", "<u8"),
-                                                 ("n", "<i8"), ("prepared_prec", "<i4"), ("mode", "<i4")]))
+    desc = np.zeros(len(shapes), dtype=L.PARAM_DESC)
     chunks, offs = [], [0]
     for i in range(len(shapes)):
         desc[i]["theta"], desc[i]["grad"], desc[i]["vhat"] = th[i].data_ptr(), gr[i].data_ptr(), vh[i].data_ptr()

@@ -169,10 +169,7 @@ def test_reduce_partials2_equals_two_calls(L):
 def _descs(L, tensors, ext=None):
     """coper_param_desc array + chunk lists for a list of gradient tensors (dense mode)."""
     import ctypes as C
-    desc_dt = np.dtype([("theta", np.uint64), ("grad", np.uint64), ("m", np.uint64), ("v", np.uint64),
-                        ("vhat", np.uint64), ("prepared", np.uint64), ("grad_sq", np.uint64), ("n", np.int64),
-                        ("prepared_prec", np.int32), ("mode", np.int32)])
-    d = np.zeros(len(tensors), desc_dt)
+    d = np.zeros(len(tensors), L.PARAM_DESC)
     chunks, offsets = [], [0]
     for t, g in enumerate(tensors):
         d[t]["grad"] = g.data_ptr()
@@ -240,7 +237,8 @@ def test_segscatter_pair_equals_two_calls(L, with_norm, with_sq, R):
                    L.ptr(rel), B, L.ptr(drr), dr, L.ptr(dR), L.ptr(dRsq), 0, R)
         else:
             if with_norm:
-                L.call("coper_segscatter_add_norm", L.ptr(e1), B, L.ptr(dx0), d, L.ptr(dE), L.ptr(dEsq), lo, hi, L.ptr(nd))
+                L.call("coper_segscatter_add_pair", L.ptr(e1), B, L.ptr(dx0), d, L.ptr(dE), L.ptr(dEsq), lo, hi, L.ptr(nd),
+                       None, 0, None, 0, None, None, 0, 0)
             else:
                 L.call("coper_segscatter_add_sq", L.ptr(e1), B, L.ptr(dx0), d, L.ptr(dE), L.ptr(dEsq), lo, hi)
             L.call("coper_segscatter_add_sq", L.ptr(rel), B, L.ptr(drr), dr, L.ptr(dR), L.ptr(dRsq), 0, R)

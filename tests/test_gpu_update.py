@@ -135,7 +135,7 @@ def test_scorer_norm_and_split_form(L, prec, B, N, d):
 @pytest.mark.parametrize("M", [1, 130, 4096])
 @pytest.mark.parametrize("pair", [False, True])
 def test_head_scatter_norm_delta(L, M, pair):
-    """norm_delta of coper_segscatter_add_norm / the a half of coper_segscatter_add_pair: the change of the squared
+    """norm_delta of coper_segscatter_add_pair's a job, alone and beside a b job: the change of the squared
     norm of the shard's rows, reported once per destination row by its writer (the first position that holds it)."""
     rng = np.random.default_rng(M * 3 + pair)
     d, lo, hi, R, dr = 200, 100, 500, 22, 8
@@ -157,7 +157,8 @@ def test_head_scatter_norm_delta(L, M, pair):
         L.call("coper_segscatter_add_pair", L.ptr(te1), M, L.ptr(tsrc), d, L.ptr(tdst), L.ptr(tsq), lo, hi, L.ptr(nd),
                L.ptr(trel), M, L.ptr(tdrr), dr, L.ptr(dR), L.ptr(dRsq), 0, R)
     else:
-        L.call("coper_segscatter_add_norm", L.ptr(te1), M, L.ptr(tsrc), d, L.ptr(tdst), L.ptr(tsq), lo, hi, L.ptr(nd))
+        L.call("coper_segscatter_add_pair", L.ptr(te1), M, L.ptr(tsrc), d, L.ptr(tdst), L.ptr(tsq), lo, hi, L.ptr(nd),
+               None, 0, None, 0, None, None, 0, 0)
     torch.cuda.synchronize()
     delta = nd.cpu().numpy()
     after = tdst.cpu().numpy().astype(np.float64)
