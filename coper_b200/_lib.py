@@ -109,6 +109,7 @@ SIGNATURES = {
 }
 SUMSQ_BLOCKS = 256
 TOPK_MAX = 128  # COPER_TOPK_MAX
+SEGSCATTER_SMALL_M = 4096  # COPER_SEGSCATTER_SMALL_M
 MT_CHUNK = 16384
 # mirrors coper_param_desc (include/coper.h): one record per tensor of the multi-tensor clip / AMSGrad launches
 PARAM_DESC = np.dtype([("theta", "<u8"), ("grad", "<u8"), ("m", "<u8"), ("v", "<u8"), ("vhat", "<u8"), ("prepared", "<u8"),

@@ -41,7 +41,7 @@ __global__ void segscatter_kernel(const int64_t* __restrict__ keys, const int32_
 // not a segment head and exits - and otherwise sums every later member of its row in INDEX order (the order a stable
 // sort would give): same result bit for bit as the sorted path, one launch, no workspace.
 // dst_sq (optional): sum of the SQUARED source rows per destination row (the IndexedSlices bookkeeping).
-constexpr int kSegSmallM = 4096;
+constexpr int kSegSmallM = COPER_SEGSCATTER_SMALL_M;
 // norm_delta (optional, [M] doubles): position i receives sum_c (new_c^2 - old_c^2) of the destination row it updated
 // (0 if it is not a segment head / not owned) - the correction that turns a sum of squares taken BEFORE the scatter
 // (by the kernel that produced dst) into the sum of squares of the final gradient.

@@ -32,6 +32,7 @@ one fused kernel).
 """
 from __future__ import annotations
 
+import contextlib
 import math
 from typing import Dict, List, Optional
 
@@ -437,6 +438,20 @@ class ConvE:
         self._bufs = {}
         self._graphs = {}
         self._build_trainables()
+        # per-model constants of the training step: the BCE targets in fp32 (models.py:450)
+        self._pos = float(np.float32(np.float32(1.0 - self.label_smoothing_epsilon) * np.float32(1.0)
+                                     + np.float32(1.0 / self.num_ent)))
+        self._neg = float(np.float32(1.0 / self.num_ent))
+        # g_linear (no hidden generator layers: both contexts ARE the relation embedding): d rel_emb = dc + dcb is
+        # formed by the CPG-FC backward itself - dc lands in b.dr, the bias generator's dcb is added to it
+        self._linear = self.variant == "cpg" and not self.fc_weights.hidden and not self.fc_bias.hidden
+        self._cpg_bwd_flags = (CPG_BWD_REUSE_FWD if self.prec != 0 else 0) | \
+            (CPG_BWD_DCB_ACCUMULATE if self._linear else 0)
+        # the generator's weight gradients (dP^, dPb) feed nothing but the clip / optimizer: they are computed on the
+        # side stream while the chain through df / dc continues (DESIGN 4.5)
+        self._split_w = not self.dp and self.variant != "param_lookup"
+        # shared conv filters: the Conv1BN backward is folded into the conv backward (dz never goes to HBM)
+        self._fold = self.conv_w_gen is None
         self.refresh_prepared()
         # device-resident step state: {lr_t, beta1^t, beta2^t, -} and the dropout seed
         self.step_state = torch.tensor([0.0, self.beta1, self.beta2, 0.0], dtype=f32, device=dev)
@@ -563,7 +578,7 @@ class ConvE:
         self.dE_sumsq = torch.zeros(1, dtype=torch.float64, device=self.dev)
         # arrival counter of the single-launch batch-norm statistics (coper_bn_stats_finalize); zero between launches
         self.sync_word = torch.zeros(1, dtype=torch.int32, device=self.dev)
-        self.norm_delta = torch.zeros(4096, dtype=torch.float64, device=self.dev)
+        self.norm_delta = torch.zeros(_lib.SEGSCATTER_SMALL_M, dtype=torch.float64, device=self.dev)
         self._norm_fused_now = False
         self._norm_delta_n = 0
         self.mt_chunks = torch.tensor(chunks, dtype=torch.int32).to(self.dev)
@@ -952,36 +967,52 @@ class ConvE:
     def _train_device(self, b, apply: bool = True):
         """fwd + bwd (+ clip + AMSGrad when apply) on staged buffers; everything is enqueued, nothing syncs.
         apply=False leaves the gradients for a later _clip_and_apply()."""
-        self._train_device_impl(b, self._local_buffers(b) if self.dp else b, apply)
-
-    def _train_device_impl(self, bg, b, apply):
-        """bg: buffers of the batch the scorer sees; b: buffers of the rows this rank's front end owns
-        (b is bg unless the front end is data-parallel)."""
-        dp = b is not bg
-        B, d, dr, F, C = b.B, self.ent_emb_size, self.rel_emb_size, self.F, self.C
-        s, g = self.shard, self.grads
-        Ns = s.rows
-        if dp:
+        # bg: buffers of the batch the scorer sees; b: buffers of the rows this rank's front end owns
+        bg, b = b, (self._local_buffers(b) if self.dp else b)
+        # the fused norm needs the scatter's norm correction, which only the small-M scatter kernel writes
+        self._norm_fused_now = self._norm_fused and bg.B <= _lib.SEGSCATTER_SMALL_M
+        inv_count = 1.0 / (float(bg.B) * float(self.num_ent))                # mean over B*N (models.py:451)
+        if self.dp:
             call("coper_step_state_advance", ptr(self.step_state), ptr(self.seed_dev), self.learning_rate, self.beta1,
                  self.beta2)
             self._forward_q_dp(bg, b, True)
         else:
             self._forward_q(b, True, advance=True)
-        pos = np.float32(np.float32(1.0 - self.label_smoothing_epsilon) * np.float32(1.0)
-                         + np.float32(1.0 / self.num_ent))                     # models.py:450 in fp32
-        neg = np.float32(1.0 / self.num_ent)
-        inv_count = 1.0 / (float(bg.B) * float(self.num_ent))                # mean over B*N (models.py:451)
-        self._norm_fused_now = self._norm_fused and bg.B <= 4096       # (the scatter correction is the small-M kernel's)
+        rel_cleared = self._scorer_backward(bg, b, inv_count)
+        big_work = self._fc_backward(b)
+        self._conv_backward(b)
+        self._lookup_grad_scatter(bg, b, rel_cleared)
+        if self.dp:      # partial sums over this rank's rows -> all-reduce of the flat bucket
+            if big_work is not None:
+                sharding.reduce_replicated_grads(self.flat_small, self.world, self.group)
+                big_work.wait()
+            else:
+                sharding.reduce_replicated_grads(self.flat_grads, self.world, self.group)
+        if apply:
+            self._clip_and_apply()
+
+    @contextlib.contextmanager
+    def _on_side(self):
+        """Fork: the body is enqueued on the side stream, after everything enqueued so far on the current one.  The
+        step joins the side stream before the lookup-gradient scatter."""
+        self._side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(self._side):
+            yield
+        self._side_pending = True
+
+    def _scorer_backward(self, bg, b, inv_count):
+        """Scorer + BCE loss + dq / dE / dbias for the bg.B queries, then the entity-sharded scorer's exchange and the
+        mean loss.  Returns whether the relation gradient was cleared (on the side stream, for the scatter)."""
+        g, Ns, d = self.grads, self.shard.rows, self.ent_emb_size
         rel_cleared = loss_done = False
         if self.use_negative_sampling:
             self._sampled_scorer(bg)
         elif self._norm_fused_now:
             call("coper_score1n_bce_fwd_bwd_norm", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
-                 ptr(bg.bitsT), bg.B, Ns, d, float(pos), float(neg), inv_count, ptr(bg.loss_sum),
+                 ptr(bg.bitsT), bg.B, Ns, d, self._pos, self._neg, inv_count, ptr(bg.loss_sum),
                  ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), None, ptr(g["pred_bias"]), ptr(self.dE_sumsq), ptr(bg.ws),
                  bg.ws_bytes, self.prec)
-            self._side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(self._side):
+            with self._on_side():
                 if self.rel_emb is not None:     # cleared here, off the main chain, for the scatter after the join
                     g["rel_emb"].zero_()
                     self.grad_sq["rel_emb"].zero_()
@@ -991,45 +1022,38 @@ class ConvE:
                 if self.world == 1:              # the mean loss the caller reads (models.py:451)
                     torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
                     loss_done = True
-            self._side_pending = True
         else:
             call("coper_score1n_bce_fwd_bwd", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
-                 ptr(bg.bits if self.prec == 0 else bg.bitsT), bg.B, Ns, d, float(pos), float(neg), inv_count,
+                 ptr(bg.bits if self.prec == 0 else bg.bitsT), bg.B, Ns, d, self._pos, self._neg, inv_count,
                  ptr(bg.loss_sum), ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), ptr(g["ent_emb"]),
                  ptr(g["pred_bias"]), ptr(bg.ws), bg.ws_bytes, self.prec)
         # entity-sharded scorer: every rank scored all B queries against its rows -> sum the partial loss and
         # the partial dq = G_shard . E_shard (SURVEY §8e step 4); dE / dbias stay local.
-        if dp:      # each rank only needs the summed dq of its own rows
+        if self.dp:      # each rank only needs the summed dq of its own rows
             sharding.scatter_dq(bg.dq, b.dq, bg.loss_sum, self.world, self.group)
         else:
             sharding.reduce_scorer_partials(b.loss_sum, b.dq, self.world, self.group)
         if not loss_done and not self.use_negative_sampling:
             torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
-        use_batch = self.batch_norm_train_stats
-        keep1, keep2 = 1.0 - self.hidden_dropout, 1.0 - self.output_dropout
+        return rel_cleared
+
+    def _fc_backward(self, b):
+        """FC block and CPG-FC backward, then the FC generators' context nets.  Returns the all-reduce of the big
+        gradient bucket, left in flight under the rest of the backward pass, or None."""
+        B, d, F, g = b.B, self.ent_emb_size, self.F, self.grads
         # FC block backward: relu -> FCBN -> output dropout (models.py:414-419)
-        self._bn_backward(self.fc_bn, b.dq, b.y, B, d, b, use_batch, True, 1.0, 0, keep2, SALT_OUTPUT, b.dy)
+        self._bn_backward(self.fc_bn, b.dq, b.y, B, d, b, self.batch_norm_train_stats, True, 1.0, 0,
+                          1.0 - self.output_dropout, SALT_OUTPUT, b.dy)
         Pw, Pb = self.fc_weights.projections[-1], self.fc_bias.projections[-1]
-        nw, nb = len(self.fc_weights.projections) - 1, len(self.fc_bias.projections) - 1
-        # the generator's weight gradients (dP^, dPb) feed nothing but the clip / optimizer: they are computed on the
-        # side stream while the chain through df / dc continues (DESIGN 4.5)
-        split_w = not dp and self.variant != "param_lookup"
-        reuse = CPG_BWD_REUSE_FWD if self.prec != 0 else 0
-        # g_linear (no hidden generator layers: both contexts ARE the relation embedding): d rel_emb = dc + dcb is formed
-        # by the call itself - dc lands in b.dr, the bias generator's dcb is added to it
-        linear = self.variant == "cpg" and not self.fc_weights.hidden and not self.fc_bias.hidden
-        if linear:
-            reuse |= CPG_BWD_DCB_ACCUMULATE
-        dcw_out, dcb_out = (b.dr, b.dr) if linear else (b.dcw, b.dcb)
+        dcw_out, dcb_out = (b.dr, b.dr) if self._linear else (b.dcw, b.dcb)
         cpg_bwd_args = (ptr(b.cw), ptr(b.f), ptr(Pw), ptr(self.P_prep), ptr(b.cb), ptr(Pb), ptr(b.dy), B,
                         Pw.shape[0], F, d, Pb.shape[0], ptr(g[self._last_w_name]), ptr(g[self._last_b_name]),
                         ptr(b.df), ptr(dcw_out), ptr(dcb_out), ptr(b.ws_cpg), b.ws_cpg_bytes, self.prec)
-        call("coper_cpg_fc_bwd", *cpg_bwd_args, reuse | (CPG_BWD_INPUT_GRADS_ONLY if split_w else 0))
-        if split_w:
-            self._side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(self._side):
-                call("coper_cpg_fc_bwd", *cpg_bwd_args, reuse | CPG_BWD_WEIGHT_GRADS_ONLY)
-            self._side_pending = True
+        flags = self._cpg_bwd_flags
+        call("coper_cpg_fc_bwd", *cpg_bwd_args, flags | (CPG_BWD_INPUT_GRADS_ONLY if self._split_w else 0))
+        if self._split_w:
+            with self._on_side():
+                call("coper_cpg_fc_bwd", *cpg_bwd_args, flags | CPG_BWD_WEIGHT_GRADS_ONLY)
         if self.variant == "param_lookup":
             # the tables are read through embedding_lookup (models.py:91): IndexedSlices gradients, one [F*d] / [d]
             # slice per query.  The slice-wise norm and the sparse AMSGrad rule need, per table row, the sum of the
@@ -1041,24 +1065,27 @@ class ConvE:
                  ptr(self.grad_sq["fc_bias"]), ptr(b.df_scratch), ptr(b.dcw), ptr(b.dcb), ptr(b.ws_cpg),
                  b.ws_cpg_bytes, self.prec, 0)
         big_work = None
-        if dp and self.group_big is not None:
+        if self.dp and self.group_big is not None:
             big_work = sharding.reduce_replicated_grads(self.flat_big, self.world, self.group_big, async_op=True)
-        if self.variant == "cpg" and not linear:
+        if self.variant == "cpg" and not self._linear:
             self._ctx_backward(self.fc_weights, 0, b, b.dcw, b.dr, False)
             self._ctx_backward(self.fc_bias, 1, b, b.dcb, b.dr, True)
-        # conv block backward: feature-map dropout -> relu -> Conv1BN -> conv (models.py:373-391)
-        R1 = B * self.OH * self.OW
+        return big_work
+
+    def _conv_backward(self, b):
+        """Conv block backward: feature-map dropout -> relu -> Conv1BN -> conv (models.py:373-391), then the conv
+        filter generators.  Leaves d x0 in b.dx0 and the conv block's share of d rel_emb in b.dr."""
+        B, d, C, g = b.B, self.ent_emb_size, self.C, self.grads
+        keep1 = 1.0 - self.hidden_dropout
         if self.concat_rel:                  # tf.concat backward: conv part | d rel_emb (added to the generators' part)
             b.dfconv.copy_(b.df[:, :self.F_conv])
             if self.variant == "cpg":
                 b.dr.add_(b.df[:, self.F_conv:])
-        # shared filters: the Conv1BN backward is folded into the conv backward (dz never goes to HBM)
-        fold = self.conv_w_gen is None
-        self._bn_backward(self.conv1_bn, b.dfconv, b.z, R1, C, b, use_batch, True, keep1, SALT_FEATURE_MAP, 1.0, 0, b.dz,
-                          apply=not fold)
+        self._bn_backward(self.conv1_bn, b.dfconv, b.z, B * self.OH * self.OW, C, b, self.batch_norm_train_stats, True,
+                          keep1, SALT_FEATURE_MAP, 1.0, 0, b.dz, apply=not self._fold)
         plain = self.variant == "plain"
         KK = self.conv_filter_height * self.conv_filter_width * C
-        if self.conv_w_gen is not None:
+        if not self._fold:
             # per-example filters: dz -> dx0 and, per query, dWq [B, KK] / dbq [B, C]; then back through the generators
             call("coper_conv_bwd", ptr(b.dz), ptr(b.x0), B, self.H, self.W, ptr(b.wq), self.conv_filter_height,
                  self.conv_filter_width, C, 1, ptr(b.dx0), ptr(b.dwc_part), ptr(b.dbc_part))
@@ -1085,12 +1112,16 @@ class ConvE:
                                                      self.conv_filter_width, C, 0)
             call("coper_reduce_partials2", ptr(b.dwc_part), KK, ptr(g["conv1_weights"]), ptr(b.dbc_part), C,
                  ptr(g["conv1_bias"]), slabs, 1.0, 0)
-        # gradients of the two embedding gathers (models.py:176-178): deterministic segmented scatter
-        # IndexedSlices bookkeeping (rel_emb always; ent_emb with sampled labels): the same pass also accumulates the
-        # per-row sums of the SQUARED slices (slice-wise global norm + sparse AMSGrad rule)
-        small = B <= 4096
-        gsq_e = self.grad_sq["ent_emb"] if self.use_negative_sampling else None
-        if dp:      # every shard needs dx0 of ALL queries whose head entity it owns
+
+    def _lookup_grad_scatter(self, bg, b, rel_cleared):
+        """Gradients of the two embedding gathers (models.py:176-178): deterministic segmented scatters, after the join
+        of the side stream.  IndexedSlices bookkeeping (rel_emb always; ent_emb with sampled labels): the same pass also
+        accumulates the per-row sums of the SQUARED slices (slice-wise global norm + sparse AMSGrad rule)."""
+        s, g, gsq = self.shard, self.grads, self.grad_sq
+        B, d, dr = b.B, self.ent_emb_size, self.rel_emb_size
+        small = _lib.SEGSCATTER_SMALL_M
+        gsq_e = gsq["ent_emb"] if self.use_negative_sampling else None
+        if self.dp:      # every shard needs dx0 of ALL queries whose head entity it owns
             sharding.gather_batch(bg.dx0, b.dx0, self.world, self.group)
         if self._side_pending:      # join: the scatter below adds into dE, the clip reads every gradient
             torch.cuda.current_stream().wait_stream(self._side)
@@ -1098,38 +1129,30 @@ class ConvE:
         rel = self.rel_emb is not None
         if rel and not rel_cleared:
             g["rel_emb"].zero_()
-            self.grad_sq["rel_emb"].zero_()
-        if bg.B <= 4096:      # head-entity scatter, with the relation scatter as its second job: one launch
-            rel_job = (ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), ptr(self.grad_sq["rel_emb"]), 0, self.num_rel) \
+            gsq["rel_emb"].zero_()
+        if bg.B <= small:      # head-entity scatter, with the relation scatter as its second job: one launch
+            rel_job = (ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), ptr(gsq["rel_emb"]), 0, self.num_rel) \
                 if rel else (None, 0, None, 0, None, None, 0, 0)
             call("coper_segscatter_add_pair", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), ptr(gsq_e), s.lo, s.hi,
                  ptr(self.norm_delta) if self._norm_fused_now else None, *rel_job)
             if self._norm_fused_now:
                 self._norm_delta_n = bg.B
-        else:
-            call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0), d, ptr(g["ent_emb"]), s.lo, s.hi, ptr(bg.ws),
-                 bg.ws_bytes)
-            if gsq_e is not None:
-                torch.mul(bg.dx0, bg.dx0, out=bg.dx0_sq)
-                call("coper_segscatter_add", ptr(bg.e1), bg.B, ptr(bg.dx0_sq), d, ptr(gsq_e), s.lo, s.hi, ptr(bg.ws),
-                     bg.ws_bytes)
-            if rel and small:
-                call("coper_segscatter_add_sq", ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]),
-                     ptr(self.grad_sq["rel_emb"]), 0, self.num_rel)
-            elif rel:
-                call("coper_segscatter_add", ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), 0, self.num_rel, ptr(b.ws),
-                     b.ws_bytes)
-                torch.mul(b.dr, b.dr, out=b.dr_sq)
-                call("coper_segscatter_add", ptr(b.rel), B, ptr(b.dr_sq), dr, ptr(self.grad_sq["rel_emb"]), 0,
-                     self.num_rel, ptr(b.ws), b.ws_bytes)
-        if dp:      # partial sums over this rank's rows -> all-reduce of the flat bucket
-            if big_work is not None:
-                sharding.reduce_replicated_grads(self.flat_small, self.world, self.group)
-                big_work.wait()
-            else:
-                sharding.reduce_replicated_grads(self.flat_grads, self.world, self.group)
-        if apply:
-            self._clip_and_apply()
+            return
+        self._scatter_with_squares(bg, bg.e1, bg.dx0, bg.dx0_sq, g["ent_emb"], gsq_e, s.lo, s.hi)
+        if rel and B <= small:       # a data-parallel rank's share of a large batch
+            call("coper_segscatter_add_sq", ptr(b.rel), B, ptr(b.dr), dr, ptr(g["rel_emb"]), ptr(gsq["rel_emb"]), 0,
+                 self.num_rel)
+        elif rel:
+            self._scatter_with_squares(b, b.rel, b.dr, b.dr_sq, g["rel_emb"], gsq["rel_emb"], 0, self.num_rel)
+
+    def _scatter_with_squares(self, sl, idx, src, src_sq, dst, dst_sq, lo, hi):
+        """Sorted scatter-add of the [sl.B, w] rows src into dst and, unless dst_sq is None, of their squares (formed in
+        src_sq) into dst_sq; the workspace is sl's."""
+        w = src.shape[1]
+        call("coper_segscatter_add", ptr(idx), sl.B, ptr(src), w, ptr(dst), lo, hi, ptr(sl.ws), sl.ws_bytes)
+        if dst_sq is not None:
+            torch.mul(src, src, out=src_sq)
+            call("coper_segscatter_add", ptr(idx), sl.B, ptr(src_sq), w, ptr(dst_sq), lo, hi, ptr(sl.ws), sl.ws_bytes)
 
     def _sampled_scorer(self, b):
         """models.py:438-443 + 448-453 on the staged [B, L] lookup ids / labels (b.cur_samp).  Entity-sharded: every

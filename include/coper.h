@@ -413,18 +413,20 @@ int coper_topk_merge(const float* in_scores, const int64_t* in_ids, int n_lists,
  *   dst[idx[i] - row_lo, :] += src[i, :] for row_lo <= idx[i] < row_hi; one writer per destination row
  *   (sort by key, warp per segment, fixed summation order) -> deterministic. */
 size_t coper_segscatter_workspace_bytes(int M);
-/* M <= 4096 (one batch of gathers): sort-free variant that can also accumulate the per-row sums of the SQUARED source
- * rows into dst_sq (NULL = skip) - the IndexedSlices bookkeeping of the sparse AMSGrad rule (utils/amsgrad.py:161-189)
- * and of tf.clip_by_global_norm's slice-wise norm (models.py:199).
+/* M <= COPER_SEGSCATTER_SMALL_M (one batch of gathers): sort-free variant that can also accumulate the per-row sums of
+ * the SQUARED source rows into dst_sq (NULL = skip) - the IndexedSlices bookkeeping of the sparse AMSGrad rule
+ * (utils/amsgrad.py:161-189) and of tf.clip_by_global_norm's slice-wise norm (models.py:199).  Larger M returns
+ * COPER_ERR_UNSUPPORTED.
  * Same summation order (index order) as coper_segscatter_add, which uses this path for small M. */
+#define COPER_SEGSCATTER_SMALL_M 4096
 int coper_segscatter_add_sq(const int64_t* idx, int M, const float* src, int width, float* dst, float* dst_sq,
                             int64_t row_lo, int64_t row_hi, coper_stream_t stream);
 /* Two independent small scatters of one step in ONE launch, each with coper_segscatter_add_sq's arguments (the
- * head-entity and relation gathers' gradients, models.py:176-178).  M_b == 0: job a alone (idx_b, src_b, dst_b may be
- * NULL).  norm_delta_a (NULL = skip) receives, per position i of idx_a, norm_delta_a[i] = sum_c (new^2 - old^2) over
- * the destination row position i updated (0 for non-heads / rows of other shards): the correction of a squared
- * gradient norm that was taken before this scatter (tf.clip_by_global_norm over the dense ent_emb gradient,
- * models.py:198-199). */
+ * head-entity and relation gathers' gradients, models.py:176-178); M_a, M_b <= COPER_SEGSCATTER_SMALL_M, else
+ * COPER_ERR_UNSUPPORTED.  M_b == 0: job a alone (idx_b, src_b, dst_b may be NULL).  norm_delta_a (NULL = skip)
+ * receives, per position i of idx_a, norm_delta_a[i] = sum_c (new^2 - old^2) over the destination row position i
+ * updated (0 for non-heads / rows of other shards): the correction of a squared gradient norm that was taken before
+ * this scatter (tf.clip_by_global_norm over the dense ent_emb gradient, models.py:198-199). */
 int coper_segscatter_add_pair(const int64_t* idx_a, int M_a, const float* src_a, int width_a, float* dst_a,
                               float* dst_sq_a, int64_t lo_a, int64_t hi_a, double* norm_delta_a, const int64_t* idx_b,
                               int M_b, const float* src_b, int width_b, float* dst_b, float* dst_sq_b, int64_t lo_b,

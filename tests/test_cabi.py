@@ -32,6 +32,15 @@ def test_every_declared_symbol_is_exported_and_bound():
         assert n in names, "bound but not declared in coper.h: " + n
 
 
+def test_python_constants_mirror_the_header():
+    """The limits and flags _lib repeats for its callers equal the values include/coper.h defines."""
+    src = open(os.path.join(ROOT, "include", "coper.h")).read()
+    defs = {k: int(v) for k, v in re.findall(r"#define (COPER_\w+) (\d+)", src)}
+    for name in ("TOPK_MAX", "SEGSCATTER_SMALL_M", "SUMSQ_BLOCKS", "MT_CHUNK", "CPG_BWD_REUSE_FWD",
+                 "CPG_BWD_INPUT_GRADS_ONLY", "CPG_BWD_WEIGHT_GRADS_ONLY", "CPG_BWD_DCB_ACCUMULATE"):
+        assert defs["COPER_" + name] == getattr(_lib, name), name
+
+
 def test_workspace_queries_run_without_gpu():
     lib = _lib.load()
     assert lib.coper_colstats_chunks(1000) == 16
