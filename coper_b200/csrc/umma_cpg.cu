@@ -54,6 +54,8 @@ struct CpgFwdEpi : EpiBase {
 
 // N = d <= 256 in one tile.  tf32x3: chains cut every 4 k-blocks (see umma_gemm.cuh)
 // fp16x3: 64 k-elements per k-block (two fp16 planes) -> the same chain length is 2 k-blocks
+// f does not depend on the context group, but a resident f (RES_A_KB) made this kernel 1-4 us SLOWER at every
+// benchmark shape (B200, DESIGN §4.7): both operands stream.
 template <int PREC>
 using CpgFwdCfg = GemmCfg<PREC, 256, (PREC == PREC_BF16 ? 4 : 2), 8, false, true,
                           (PREC == PREC_BF16 ? 0 : PREC == PREC_FP16X3 ? 2 : 4)>;
@@ -131,8 +133,12 @@ struct CpgBwdTEpi : EpiBase {
 };
 constexpr int kBwdTEpiWarps = 16;
 constexpr int kBwdTBlockN = 128;
+// The dy tile does not depend on the context group: bf16 / fp16x3 keep its whole K extent (d <= 256: 4 k-blocks) resident
+// (64 / 128 KB) and stream only P[k] (8 x 16 KB / 3 x 32 KB stages).  tf32x3 (d = 200: 7 k-blocks x 2 planes x 16 KB)
+// does not fit and streams both.
 template <int PREC>
-using CpgBwdTCfg = GemmCfg<PREC, kBwdTBlockN, (PREC == PREC_BF16 ? 4 : 3), kBwdTEpiWarps, false, false, 0>;
+using CpgBwdTCfg = GemmCfg<PREC, kBwdTBlockN, (PREC == PREC_BF16 ? 8 : 3), kBwdTEpiWarps, false, false, 0, 0,
+                           (PREC == PREC_TF32X3 ? 0 : 4)>;
 
 // fp16x3: max |dy[b,j] * c[b,g]| = max_b (max_j |dy[b,:]| * max_g |c[b,:]|); one warp per row, result (float bits) in
 // trailer[1] (zeroed before the launch)

@@ -30,11 +30,17 @@ constexpr int NUM_NON_EPI_THREADS = 128;
 // a dedicated shared-memory region and reused by every tile of the CTA that shares the n-block; only A tiles stream
 // through the stage ring.  For the entity-major scorers (B = the query block) this cuts the L2->SM traffic per tile
 // from (A + B) to A, which is what bounds a 128 x 128 x 256 bf16 tile on B200 (~42 B/clk/SM of TMA throughput).
+// RES_A_KB > 0 ("resident A"): for problems whose A coordinates do not depend on the group (the generator backward's
+// T-kernel loops over dc groups with the same dy tile): the A k-blocks of one (m-block, split), at most RES_A_KB of
+// them, are loaded ONCE into a dedicated region, one mbarrier per k-block, and serve every group; only B tiles stream
+// through the stage ring.  The region is refilled for the next (m-block, split) only after every MMA reading it has
+// completed.
 template <int PREC_, int BLOCK_N_, int STAGES_, int EPI_WARPS_, bool A_MN_, bool B_MN_, int PROMOTE_KB_ = 0,
-          int RES_KB_ = 0>
+          int RES_KB_ = 0, int RES_A_KB_ = 0>
 struct GemmCfg {
   static constexpr int PROMOTE_KB = PROMOTE_KB_;
   static constexpr int RES_KB = RES_KB_;
+  static constexpr int RES_A_KB = RES_A_KB_;
   static constexpr int PREC = PREC_, BLOCK_N = BLOCK_N_, STAGES = STAGES_, EPI_WARPS = EPI_WARPS_;
   static constexpr bool A_MN = A_MN_, B_MN = B_MN_;
   static constexpr int ELEM = (PREC == PREC_TF32X3) ? 4 : 2;
@@ -45,12 +51,19 @@ struct GemmCfg {
   static constexpr bool SCALED = (PREC == PREC_FP16X3);         // accumulators carry 2^(ea+eb)
   static constexpr int A_BYTES = BLOCK_M * 128;     // one plane of the A tile (BLOCK_M x BLOCK_K or BLOCK_K x BLOCK_M)
   static constexpr int B_BYTES = BLOCK_N * 128;
-  static constexpr int STAGE_BYTES = RES_KB_ > 0 ? TERMS * A_BYTES : TERMS * (A_BYTES + B_BYTES);
-  static constexpr int RES_BYTES = RES_KB_ * TERMS * B_BYTES;
+  static constexpr int STAGE_BYTES = RES_KB_ > 0     ? TERMS * A_BYTES
+                                     : RES_A_KB_ > 0 ? TERMS * B_BYTES
+                                                     : TERMS * (A_BYTES + B_BYTES);
+  static constexpr int RES_PLANE_BYTES = RES_KB_ > 0 ? B_BYTES : A_BYTES;
+  static constexpr int RES_BYTES = (RES_KB_ + RES_A_KB_) * TERMS * RES_PLANE_BYTES;
+  static constexpr int BARRIERS = 2 * STAGES + 2 + 2 + 1 + RES_A_KB_;   // full, empty, tfull, tempty, bfull, afull
   static constexpr int TMEM_COLS = (2 * BLOCK_N <= 32) ? 32 : (2 * BLOCK_N <= 64) ? 64 : (2 * BLOCK_N <= 128) ? 128
                                    : (2 * BLOCK_N <= 256) ? 256 : 512;
   static constexpr int THREADS = NUM_NON_EPI_THREADS + EPI_WARPS * 32;
   static constexpr size_t SMEM_BYTES = (size_t)STAGES * STAGE_BYTES + RES_BYTES + 1024 /*align*/ + 256 /*barriers*/;
+  static_assert(RES_KB_ == 0 || RES_A_KB_ == 0, "one resident operand");
+  static_assert(BARRIERS * 8 + 4 <= 256, "barriers + TMEM address");
+  static_assert(SMEM_BYTES <= 227 * 1024, "dynamic shared memory of one CTA");
 
   static constexpr uint32_t FMT = (PREC == PREC_BF16) ? FMT_BF16 : (PREC == PREC_FP16X3) ? FMT_F16 : FMT_TF32;
   // MN-major smem layout: 16-bit types use the plain 128B swizzle (8-row k atoms); tf32 must use the
@@ -73,8 +86,9 @@ struct SmemLayout {
   uint64_t* tfull;      // [2]
   uint64_t* tempty;     // [2]
   uint64_t* bfull;      // [1] resident B loaded
+  uint64_t* afull;      // [RES_A_KB] resident A k-block loaded
   uint32_t* tmem_ptr;
-  uint8_t* res;         // resident B region: [RES_KB][TERMS][B_BYTES]
+  uint8_t* res;         // resident region: B [RES_KB][TERMS][B_BYTES] or A [RES_A_KB][TERMS][A_BYTES]
   __device__ __forceinline__ explicit SmemLayout(uint8_t* raw) {
     base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~uintptr_t(1023));
     res = base + (size_t)Cfg::STAGES * Cfg::STAGE_BYTES;
@@ -84,16 +98,18 @@ struct SmemLayout {
     tfull = bars + 2 * Cfg::STAGES;
     tempty = tfull + 2;
     bfull = tempty + 2;
-    tmem_ptr = reinterpret_cast<uint32_t*>(bfull + 1);
+    afull = bfull + 1;
+    tmem_ptr = reinterpret_cast<uint32_t*>(afull + Cfg::RES_A_KB);
   }
   __device__ __forceinline__ uint8_t* res_plane(int kb, int term) const {
-    return res + ((size_t)kb * Cfg::TERMS + term) * Cfg::B_BYTES;
+    return res + ((size_t)kb * Cfg::TERMS + term) * Cfg::RES_PLANE_BYTES;
   }
-  __device__ __forceinline__ uint8_t* a_plane(int stage, int term) const {
+  __device__ __forceinline__ uint8_t* a_plane(int stage, int term) const {   // streaming-A configurations only
     return base + (size_t)stage * Cfg::STAGE_BYTES + term * Cfg::A_BYTES;
   }
   __device__ __forceinline__ uint8_t* b_plane(int stage, int term) const {   // streaming-B configurations only
-    return base + (size_t)stage * Cfg::STAGE_BYTES + Cfg::TERMS * Cfg::A_BYTES + term * Cfg::B_BYTES;
+    return base + (size_t)stage * Cfg::STAGE_BYTES + (Cfg::RES_A_KB > 0 ? 0 : Cfg::TERMS * Cfg::A_BYTES) +
+           term * Cfg::B_BYTES;
   }
 };
 
@@ -105,6 +121,7 @@ __device__ __forceinline__ uint32_t cta_setup(const SmemLayout<Cfg>& sm) {
     for (int i = 0; i < Cfg::STAGES; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&sm.tfull[i], 1); mbar_init(&sm.tempty[i], Cfg::EPI_WARPS); }
     mbar_init(sm.bfull, 1);
+    for (int i = 0; i < Cfg::RES_A_KB; ++i) mbar_init(&sm.afull[i], 1);
     fence_barrier_init();
   } else if (warp == 2) {
     tmem_alloc(sm.tmem_ptr, Cfg::TMEM_COLS);
@@ -125,9 +142,22 @@ __device__ __forceinline__ void cta_teardown(uint32_t tmem_base) {
   }
 }
 
-// Producer: fill one stage.  (a_mn0, b_mn0) = first row (M / N index) of the tiles, k0 = first k element.
+// One plane of the A tile (a_mn0 = first M index, a_k0 = first k element) into dst, completing on bar.
 // K-major operand: tensor map over [rows = MN, cols = K], one box {BLOCK_K, rows}.
 // MN-major operand: tensor map over [rows = K, cols = MN], boxes {CHUNK, BLOCK_K} per 128-byte MN chunk.
+template <class Cfg>
+__device__ __forceinline__ void load_a_plane(uint8_t* dst, const CUtensorMap* ma, uint64_t* bar, int a_mn0, int a_k0,
+                                             bool leader) {
+  if (!Cfg::A_MN) {
+    if (leader) tma_load_2d(dst, ma, bar, a_k0, a_mn0);
+  } else {
+#pragma unroll
+    for (int c = 0; c < BLOCK_M / Cfg::CHUNK; ++c)
+      if (leader) tma_load_2d(dst + c * (Cfg::BLOCK_K * 128), ma, bar, a_mn0 + c * Cfg::CHUNK, a_k0);
+  }
+}
+
+// Producer: fill one stage.  (a_mn0, b_mn0) = first row (M / N index) of the tiles, k0 = first k element.
 template <class Cfg>
 __device__ __forceinline__ void produce_stage(const SmemLayout<Cfg>& sm, int stage, const CUtensorMap* tA,
                                               const CUtensorMap* tAlo, const CUtensorMap* tB, const CUtensorMap* tBlo,
@@ -137,15 +167,8 @@ __device__ __forceinline__ void produce_stage(const SmemLayout<Cfg>& sm, int sta
   if (leader) mbar_expect_tx(bar, Cfg::STAGE_BYTES);
 #pragma unroll
   for (int t = 0; t < Cfg::TERMS; ++t) {
-    const CUtensorMap* ma = t ? tAlo : tA;
     const CUtensorMap* mb = t ? tBlo : tB;
-    if (!Cfg::A_MN) {
-      if (leader) tma_load_2d(sm.a_plane(stage, t), ma, bar, a_k0, a_mn0);
-    } else {
-#pragma unroll
-      for (int c = 0; c < BLOCK_M / Cfg::CHUNK; ++c)
-        if (leader) tma_load_2d(sm.a_plane(stage, t) + c * (Cfg::BLOCK_K * 128), ma, bar, a_mn0 + c * Cfg::CHUNK, a_k0);
-    }
+    if (Cfg::RES_A_KB == 0) load_a_plane<Cfg>(sm.a_plane(stage, t), t ? tAlo : tA, bar, a_mn0, a_k0, leader);
     if (Cfg::RES_KB > 0) {
       // B is resident: nothing to stream
     } else if (!Cfg::B_MN) {
@@ -168,7 +191,7 @@ __device__ __forceinline__ void issue_stage_rt(const SmemLayout<Cfg>& sm, int st
   uint64_t da[2], db[2];
 #pragma unroll
   for (int t = 0; t < Cfg::TERMS; ++t) {
-    const uint32_t a_addr = smem_u32(sm.a_plane(stage, t));
+    const uint32_t a_addr = smem_u32(Cfg::RES_A_KB > 0 ? sm.res_plane(kb_res, t) : sm.a_plane(stage, t));
     const uint32_t b_addr = smem_u32(Cfg::RES_KB > 0 ? sm.res_plane(kb_res, t) : sm.b_plane(stage, t));
     da[t] = Cfg::A_MN ? make_desc(a_addr, Cfg::BLOCK_K * 128, Cfg::MN_SBO, Cfg::MN_LAYOUT) : make_desc_kmajor(a_addr);
     db[t] = Cfg::B_MN ? make_desc(b_addr, Cfg::BLOCK_K * 128, Cfg::MN_SBO, Cfg::MN_LAYOUT) : make_desc_kmajor(b_addr);
@@ -206,6 +229,16 @@ struct PipeState {
     if (++stage == STAGES) { stage = 0; phase ^= 1; }
   }
 };
+
+// Producer, before refilling a resident region: every stage of the ring has been released, i.e. every MMA issued so
+// far (all of which may read the resident region) has completed.
+template <class Cfg>
+__device__ __forceinline__ void wait_ring_drained(const SmemLayout<Cfg>& sm, PipeState q) {
+  for (int i = 0; i < Cfg::STAGES; ++i) {
+    mbar_wait(&sm.empty[q.stage], q.phase ^ 1);
+    q.template advance<Cfg::STAGES>();
+  }
+}
 
 }  // namespace umma
 }  // namespace coper
@@ -306,20 +339,22 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tA, const __grid_constant__
       tma_prefetch_desc(&tB);
     }
     PipeState ps;
-    int res_nblk = -1;
+    int res_nblk = -1, res_a_key = -1;
     for (long long s = blockIdx.x; s < supers; s += gridDim.x) {
       for (int g = 0; g < g_loop; ++g) {
         TileCoord t = gemm_decode(p, s, g, Cfg::BLOCK_K);
         int a_mn0 = t.m_blk * BLOCK_M + t.group * p.a_group_mn;
         int b_mn0 = t.n_blk * Cfg::BLOCK_N + t.group * p.b_group_mn;
+        bool load_a = false;       // resident A: this group pass also loads the A k-blocks of (m_blk, split)
+        if (Cfg::RES_A_KB > 0 && g == 0 && t.split * p.m_tiles + t.m_blk != res_a_key) {
+          wait_ring_drained<Cfg>(sm, ps);
+          res_a_key = t.split * p.m_tiles + t.m_blk;
+          load_a = true;
+        }
         if (Cfg::RES_KB > 0 && t.n_blk != res_nblk) {
           // new n-block: wait until every MMA that reads the old resident B has completed (all stages drained),
           // then load the whole K extent of the new B tile
-          PipeState q = ps;
-          for (int i = 0; i < Cfg::STAGES; ++i) {
-            mbar_wait(&sm.empty[q.stage], q.phase ^ 1);
-            q.template advance<Cfg::STAGES>();
-          }
+          wait_ring_drained<Cfg>(sm, ps);
           const int kbn = t.kb1 - t.kb0;
           if (leader) mbar_expect_tx(sm.bfull, (uint32_t)(kbn * Cfg::TERMS * Cfg::B_BYTES));
           for (int kb = t.kb0; kb < t.kb1; ++kb)
@@ -339,6 +374,15 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tA, const __grid_constant__
           res_nblk = t.n_blk;
         }
         for (int kb = t.kb0; kb < t.kb1; ++kb) {
+          if (Cfg::RES_A_KB > 0 && load_a) {
+            // issued ahead of the stage's B tile and without waiting for a free stage: the first MMA waits only for
+            // its own A k-block
+            uint64_t* bar = &sm.afull[kb - t.kb0];
+            if (leader) mbar_expect_tx(bar, Cfg::TERMS * Cfg::A_BYTES);
+#pragma unroll
+            for (int tm = 0; tm < Cfg::TERMS; ++tm)
+              load_a_plane<Cfg>(sm.res_plane(kb - t.kb0, tm), tm ? &tAlo : &tA, bar, a_mn0, kb * Cfg::BLOCK_K, leader);
+          }
           mbar_wait(&sm.empty[ps.stage], ps.phase ^ 1);
           produce_stage<Cfg>(sm, ps.stage, &tA, &tAlo, &tB, &tBlo, a_mn0, b_mn0,
                              kb * Cfg::BLOCK_K + t.group * p.a_group_k, kb * Cfg::BLOCK_K + t.group * p.b_group_k, leader);
@@ -353,11 +397,17 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tA, const __grid_constant__
     PipeState ps;
     int as = 0;
     uint32_t aphase = 0;
-    int res_nblk = -1;
+    int res_nblk = -1, res_a_key = -1;
     uint32_t bphase = 0;
+    uint32_t a_parity = 0;         // bit i: parity of the next completion of afull[i] (a short last split skips some)
     for (long long s = blockIdx.x; s < supers; s += gridDim.x) {
       for (int g = 0; g < g_loop; ++g) {
         TileCoord t = gemm_decode(p, s, g, Cfg::BLOCK_K);
+        bool wait_a = false;       // the same decision as the producer's load_a
+        if (Cfg::RES_A_KB > 0 && g == 0 && t.split * p.m_tiles + t.m_blk != res_a_key) {
+          res_a_key = t.split * p.m_tiles + t.m_blk;
+          wait_a = true;
+        }
         if (Cfg::RES_KB > 0 && t.n_blk != res_nblk) {
           mbar_wait(sm.bfull, bphase);
           bphase ^= 1;
@@ -372,6 +422,11 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tA, const __grid_constant__
           mbar_wait(&sm.tempty[as], aphase ^ 1);
           tc_fence_after();
           for (int kb = kc; kb < kce; ++kb) {
+            if (Cfg::RES_A_KB > 0 && wait_a) {
+              const int i = kb - t.kb0;
+              mbar_wait(&sm.afull[i], (a_parity >> i) & 1u);
+              a_parity ^= 1u << i;
+            }
             mbar_wait(&sm.full[ps.stage], ps.phase);
             tc_fence_after();
             int kvalid = min(Cfg::BLOCK_K, p.K - kb * Cfg::BLOCK_K);
@@ -530,6 +585,8 @@ int launch_gemm(const TcOperand& A, const TcOperand& B, const GemmProblem& p, co
                 int grid_override = 0) {
   if (p.groups_inner && !Epi::kAccumulate) return COPER_ERR_INVALID_ARG;
   if (Cfg::RES_KB > 0 && (p.splits != 1 || p.groups != 1 || (p.K + Cfg::BLOCK_K - 1) / Cfg::BLOCK_K > Cfg::RES_KB))
+    return COPER_ERR_UNSUPPORTED;
+  if (Cfg::RES_A_KB > 0 && (p.kb_per_split > Cfg::RES_A_KB || p.a_group_mn != 0 || p.a_group_k != 0))
     return COPER_ERR_UNSUPPORTED;
   CUtensorMap tA, tAlo, tB, tBlo;
   int rc = make_gemm_tmaps<Cfg>(A, B, &tA, &tAlo, &tB, &tBlo);
