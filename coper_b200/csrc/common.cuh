@@ -136,19 +136,6 @@ __device__ __forceinline__ T block_sum(T v, T* smem32) {
   return r;
 }
 
-// COPER_PREC_FP16X3 operand scaling (umma_score.cu): x is stored as hi / lo fp16 planes of x * 2^e with e chosen so that
-// the operand's max |x| lands in [2^10, 2^11).  Trailer of a prepared operand (uint32 words, 256 bytes after the planes):
-// [0] e (int32), [1] max |x| of the last full preparation (float bits), [2] max |x| accumulated by the optimizer kernel
-// while it re-emits the operand (float bits; rolled into [0] before the next optimizer pass).
-constexpr int kFp16x3TargetExp = 10;
-__host__ __device__ __forceinline__ int fp16x3_exponent_of(float absmax) {
-  if (!(absmax > 0.f) || !(absmax < 3.0e38f)) return 0;
-  int ex;
-  frexpf(absmax, &ex);                       // absmax = f * 2^ex, f in [0.5, 1)  ->  ilogb = ex - 1
-  int e = kFp16x3TargetExp - (ex - 1);
-  return e < -100 ? -100 : (e > 100 ? 100 : e);
-}
-
 // SMs of the current device (148 on B200), queried once per device: grids of the persistent kernels are sized from it
 inline int sm_count() {
   static int cached[64] = {};

@@ -1,9 +1,7 @@
 // HBM-bound pieces of the CoPER-ConvE hot path: lookups, batch-norm/relu/dropout, label bit rows,
 // deterministic reductions, global-norm clip and AMSGrad.  All kernels are streaming: coalesced,
 // 128-bit vectorised where the shape allows, grids sized in multiples of the SM count.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-#include "common.cuh"
+#include "operand.cuh"
 
 namespace coper {
 thread_local int g_last_cuda_error = 0;
@@ -713,10 +711,6 @@ __global__ void __launch_bounds__(256) mt_sumsq_kernel(const coper_param_desc* _
   if (threadIdx.x == 0) chunk_partials[blockIdx.x] = tsum;
 }
 // tensor_sumsq[t] = sum of the chunk partials of tensor t (fixed order); chunk_offsets [n_tensors + 1]
-__device__ __forceinline__ uint32_t* fp16x3_trailer_of(const coper_param_desc& d) {
-  // the optimizer emits operands whose pitch equals the row length: 2 fp16 planes of n elements, then the trailer
-  return reinterpret_cast<uint32_t*>(static_cast<char*>(d.prepared) + (((size_t)d.n * 4 + 255) / 256) * 256);
-}
 __global__ void mt_tensor_sums_kernel(const coper_param_desc* __restrict__ descs, const double* __restrict__ chunk_partials,
                                       const int32_t* __restrict__ chunk_offsets, int n_tensors,
                                       double* __restrict__ tensor_sumsq) {
@@ -734,11 +728,7 @@ __global__ void mt_tensor_sums_kernel(const coper_param_desc* __restrict__ descs
     // fp16x3 operand copies re-emitted by the update kernel that follows: roll the exponent to the magnitude the
     // variable has NOW (running max of the previous emission / of the full preparation) and restart the running max
     const coper_param_desc d = descs[t];
-    if (d.prepared && d.prepared_prec == COPER_PREC_FP16X3) {
-      uint32_t* tr = fp16x3_trailer_of(d);
-      reinterpret_cast<int*>(tr)[0] = fp16x3_exponent_of(__uint_as_float(tr[2]));
-      tr[2] = 0u;
-    }
+    if (d.prepared && d.prepared_prec == COPER_PREC_FP16X3) fp16x3_roll(fp16x3_trailer(d.prepared, d.n));
   }
 }
 // mt_tensor_sums_kernel + sumsq_combine_kernel + clip_scale_kernel in ONE block (same summation orders): per-tensor sums
@@ -762,11 +752,8 @@ __global__ void __launch_bounds__(256) mt_sumsq_finish_kernel(const coper_param_
     acc = warp_sum_d(acc);
     if (lane == 0) {
       if (t != ext_tensor) tensor_sumsq[t] = acc;
-      if (d.prepared && d.prepared_prec == COPER_PREC_FP16X3) {      // see mt_tensor_sums_kernel
-        uint32_t* tr = fp16x3_trailer_of(d);
-        reinterpret_cast<int*>(tr)[0] = fp16x3_exponent_of(__uint_as_float(tr[2]));
-        tr[2] = 0u;
-      }
+      if (d.prepared && d.prepared_prec == COPER_PREC_FP16X3)       // see mt_tensor_sums_kernel
+        fp16x3_roll(fp16x3_trailer(d.prepared, d.n));
     }
   }
   if (ext_tensor >= 0) {
@@ -803,22 +790,6 @@ __device__ __forceinline__ void amsgrad_elem(float g, float& th, float* m, float
   vh = fmaxf(vh, vt);
   th -= lr_t * mt / (sqrtf(vh) + eps);
 }
-__device__ __forceinline__ void emit_prepared(const coper_param_desc& d, int64_t i, float th, float sc = 1.0f) {
-  if (d.prepared_prec == COPER_PREC_BF16) {
-    static_cast<__nv_bfloat16*>(d.prepared)[i] = __float2bfloat16_rn(th);
-  } else if (d.prepared_prec == COPER_PREC_FP16X3) {
-    const float xs = th * sc;
-    const __half h = __float2half_rn(xs);
-    static_cast<__half*>(d.prepared)[i] = h;
-    static_cast<__half*>(d.prepared)[d.n + i] = __float2half_rn(xs - __half2float(h));
-  } else {
-    uint32_t h;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(th));
-    float hf = __uint_as_float(h);
-    static_cast<float*>(d.prepared)[i] = hf;
-    static_cast<float*>(d.prepared)[d.n + i] = th - hf;
-  }
-}
 __global__ void __launch_bounds__(256) mt_amsgrad_kernel(const coper_param_desc* __restrict__ descs,
                                                          const int32_t* __restrict__ chunks,
                                                          const float* __restrict__ step_state, float b1, float b2,
@@ -834,8 +805,9 @@ __global__ void __launch_bounds__(256) mt_amsgrad_kernel(const coper_param_desc*
   const float omb1 = 1.0f - b1, omb2 = 1.0f - b2;
   // fp16x3 operand copy: the exponent was rolled by mt_tensor_sums_kernel; max |theta_new| goes to the running max
   const bool f16x3 = d.prepared && d.prepared_prec == COPER_PREC_FP16X3;
-  uint32_t* trailer = f16x3 ? fp16x3_trailer_of(d) : nullptr;
-  const float sc = f16x3 ? exp2f((float)reinterpret_cast<const int*>(trailer)[0]) : 1.0f;
+  // the optimizer's operand copies have pitch == row length: planes of n elements
+  uint32_t* trailer = f16x3 ? fp16x3_trailer(d.prepared, d.n) : nullptr;
+  const float sc = f16x3 ? exp2f((float)reinterpret_cast<const int*>(trailer)[kTrExp]) : 1.0f;
   float amax = 0.f;
   if ((d.mode & 1) == COPER_GRAD_INDEXED_SLICES) {           // utils/amsgrad.py:161-189 (slots accumulate)
     for (int64_t i = start + threadIdx.x; i < end; i += 256) {
@@ -848,13 +820,10 @@ __global__ void __launch_bounds__(256) mt_amsgrad_kernel(const coper_param_desc*
       d.vhat[i] = vh;
       const float th = d.theta[i] - lr_t * mt / (sqrtf(vh) + eps);
       d.theta[i] = th;
-      if (d.prepared) emit_prepared(d, i, th, sc);
+      if (d.prepared) emit_prepared(d.prepared_prec, d.prepared, d.n, i, th, sc);
       amax = fmaxf(amax, fabsf(th));
     }
-    if (f16x3) {
-      amax = warp_max(amax);
-      if ((threadIdx.x & 31) == 0 && amax > 0.f) atomicMax(trailer + 2, __float_as_uint(amax));
-    }
+    if (f16x3) warp_trailer_max(trailer + kTrRunMax, amax);
     return;
   }
   const bool vec = end - start == COPER_MT_CHUNK && bug_compat &&
@@ -874,44 +843,8 @@ __global__ void __launch_bounds__(256) mt_amsgrad_kernel(const coper_param_desc*
       th4[j] = th;
       vh4[j] = vh;
       if (d.prepared) {
-        int64_t i = start + 4 * (int64_t)j;
-        if (d.prepared_prec == COPER_PREC_BF16) {
-          __nv_bfloat162 p0 = __floats2bfloat162_rn(th.x, th.y), p1 = __floats2bfloat162_rn(th.z, th.w);
-          uint2 u;
-          u.x = *reinterpret_cast<uint32_t*>(&p0);
-          u.y = *reinterpret_cast<uint32_t*>(&p1);
-          *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(d.prepared) + i) = u;
-        } else if (d.prepared_prec == COPER_PREC_FP16X3 && (d.n & 3) == 0) {
-          const float a0 = th.x * sc, a1 = th.y * sc, a2 = th.z * sc, a3 = th.w * sc;
-          const __half2 h0 = __floats2half2_rn(a0, a1), h1 = __floats2half2_rn(a2, a3);
-          const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
-          const __half2 l0 = __floats2half2_rn(a0 - f0.x, a1 - f0.y), l1 = __floats2half2_rn(a2 - f1.x, a3 - f1.y);
-          uint2 uh, ul;
-          uh.x = *reinterpret_cast<const uint32_t*>(&h0); uh.y = *reinterpret_cast<const uint32_t*>(&h1);
-          ul.x = *reinterpret_cast<const uint32_t*>(&l0); ul.y = *reinterpret_cast<const uint32_t*>(&l1);
-          *reinterpret_cast<uint2*>(static_cast<__half*>(d.prepared) + i) = uh;
-          *reinterpret_cast<uint2*>(static_cast<__half*>(d.prepared) + d.n + i) = ul;
-          amax = fmaxf(fmaxf(amax, fmaxf(fabsf(th.x), fabsf(th.y))), fmaxf(fabsf(th.z), fabsf(th.w)));
-        } else if (d.prepared_prec == COPER_PREC_FP16X3) {
-          emit_prepared(d, i, th.x, sc); emit_prepared(d, i + 1, th.y, sc); emit_prepared(d, i + 2, th.z, sc);
-          emit_prepared(d, i + 3, th.w, sc);
-          amax = fmaxf(fmaxf(amax, fmaxf(fabsf(th.x), fabsf(th.y))), fmaxf(fabsf(th.z), fabsf(th.w)));
-        } else if ((d.n & 3) == 0) {
-          float h[4] = {th.x, th.y, th.z, th.w}, l[4];
-#pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            uint32_t hb;
-            asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(h[k]));
-            l[k] = h[k] - __uint_as_float(hb);
-            h[k] = __uint_as_float(hb);
-          }
-          float* hi = static_cast<float*>(d.prepared) + i;
-          *reinterpret_cast<float4*>(hi) = make_float4(h[0], h[1], h[2], h[3]);
-          *reinterpret_cast<float4*>(hi + d.n) = make_float4(l[0], l[1], l[2], l[3]);
-        } else {
-          emit_prepared(d, i, th.x); emit_prepared(d, i + 1, th.y); emit_prepared(d, i + 2, th.z);
-          emit_prepared(d, i + 3, th.w);
-        }
+        emit_prepared4(d.prepared_prec, d.prepared, d.n, start + 4 * (int64_t)j, th, sc);
+        if (f16x3) amax = fmaxf(fmaxf(amax, fmaxf(fabsf(th.x), fabsf(th.y))), fmaxf(fabsf(th.z), fabsf(th.w)));
       }
     }
   } else {
@@ -920,14 +853,11 @@ __global__ void __launch_bounds__(256) mt_amsgrad_kernel(const coper_param_desc*
       amsgrad_elem(d.grad[i] * cs, th, d.m, d.v, vh, i, lr_t, b1, b2, omb1, omb2, eps, bug_compat);
       d.theta[i] = th;
       d.vhat[i] = vh;
-      if (d.prepared) emit_prepared(d, i, th, sc);
+      if (d.prepared) emit_prepared(d.prepared_prec, d.prepared, d.n, i, th, sc);
       amax = fmaxf(amax, fabsf(th));
     }
   }
-  if (f16x3) {
-    amax = warp_max(amax);
-    if ((threadIdx.x & 31) == 0 && amax > 0.f) atomicMax(trailer + 2, __float_as_uint(amax));
-  }
+  if (f16x3) warp_trailer_max(trailer + kTrRunMax, amax);
 }
 
 // out[0] = sum(parts[0..n_parts)) + sum(deltas[0..n_deltas)) in a fixed order (one block)

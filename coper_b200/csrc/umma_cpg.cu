@@ -11,19 +11,10 @@
 // Backward:
 //   T_k = dy . P[k]^T  (per group, never stored)   df = sum_k c[:,k] * T_k     dc[:,k] = rowsum(f * T_k)
 //   dP[k] = f^T . (c[:,k] * dy)                     (grouped GEMM over k with a pre-scaled dy operand)
-#include <cuda_fp16.h>
 #include "umma_gemm.cuh"
 
 namespace coper {
 using namespace umma;
-
-size_t tc_prepared_bytes(int64_t rows, int cols, int prec);                     // umma_score.cu
-int tc_prepare(const float* src, int64_t rows, int cols, int64_t ld_src, int prec, void* dst, cudaStream_t st);
-int64_t tc_prepared_ld(int cols, int prec);
-TcOperand tc_operand(const void* prep, int64_t rows, int cols, int prec);       // umma_gemm.cu
-void* tc_fp16x3_trailer(const void* prep, int64_t rows, int cols);
-int tc_gemm_store(int prec, bool a_mn, bool b_mn, const TcOperand& A, const TcOperand& B, const GemmProblem& p,
-                  bool split, const StoreEpi& epi, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------ forward
 struct CpgFwdEpi : EpiBase {
@@ -74,8 +65,8 @@ static CpgFwdPlan cpg_fwd_plan(int B, int dc, int F, int d, int prec) {
   else plan_gemm<CpgFwdCfg<PREC_TF32X3>>(p, true);
   L.p = p;
   size_t o = 0;
-  L.off_f = o; o = align_up(o + tc_prepared_bytes(B, F, prec), 256);
-  L.off_P = o; o = align_up(o + tc_prepared_bytes((int64_t)dc * F, d, prec), 256);
+  L.off_f = o; o = align_up(o + prepared_bytes(B, F, prec), 256);
+  L.off_P = o; o = align_up(o + prepared_bytes((int64_t)dc * F, d, prec), 256);
   L.off_slabs = o; o = align_up(o + (size_t)p.splits * B * d * sizeof(float), 256);
   L.total = o;
   return L;
@@ -140,8 +131,8 @@ template <int PREC>
 using CpgBwdTCfg = GemmCfg<PREC, kBwdTBlockN, (PREC == PREC_BF16 ? 8 : 3), kBwdTEpiWarps, false, false, 0, 0,
                            (PREC == PREC_TF32X3 ? 0 : 4)>;
 
-// fp16x3: max |dy[b,j] * c[b,g]| = max_b (max_j |dy[b,:]| * max_g |c[b,:]|); one warp per row, result (float bits) in
-// trailer[1] (zeroed before the launch)
+// fp16x3: max |dy[b,j] * c[b,g]| = max_b (max_j |dy[b,:]| * max_g |c[b,:]|); one warp per row, result in the trailer's
+// max word (zeroed before the launch)
 __global__ void absmax_scaled_kernel(const float* __restrict__ dy, const float* __restrict__ c, int B, int d, int dc,
                                      uint32_t* __restrict__ trailer) {
   pdl_enter();
@@ -155,8 +146,7 @@ __global__ void absmax_scaled_kernel(const float* __restrict__ dy, const float* 
       my = fmaxf(my, __shfl_xor_sync(0xffffffffu, my, o));
       mc = fmaxf(mc, __shfl_xor_sync(0xffffffffu, mc, o));
     }
-    const float m = my * mc;
-    if (lane == 0 && m > 0.f) atomicMax(trailer + 1, __float_as_uint(m));
+    if (lane == 0) trailer_max(trailer + kTrMax, my * mc);
   }
 }
 // dyc[(g*B + b), j] = dy[b,j] * c[b,g] in prepared operand form
@@ -166,38 +156,21 @@ __global__ void prepare_scaled_kernel(const float* __restrict__ dy, const float*
   int64_t n = (int64_t)dc * B * ldp;
   int64_t stride = (int64_t)gridDim.x * blockDim.x;
   float sc = 1.0f;
-  if (prec == COPER_PREC_FP16X3) {                      // same exponent rule as coper_prepare_operand (umma_score.cu)
-    const int ex = fp16x3_exponent_of(__uint_as_float(trailer[1]));
-    if (blockIdx.x == 0 && threadIdx.x == 0) reinterpret_cast<int*>(trailer)[0] = ex;
-    sc = exp2f((float)ex);
-  }
+  if (prec == COPER_PREC_FP16X3) sc = fp16x3_publish(trailer, trailer[kTrMax], -1, blockIdx.x == 0 && threadIdx.x == 0);
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += stride) {
     int64_t r = e / ldp;
     int j = (int)(e - r * ldp);
     int g = (int)(r / B), b = (int)(r - (int64_t)g * B);
     float x = j < d ? __ldg(dy + (int64_t)b * d + j) * __ldg(c + (int64_t)b * dc + g) : 0.f;
-    if (prec == COPER_PREC_BF16) {
-      static_cast<__nv_bfloat16*>(dst)[e] = __float2bfloat16_rn(x);
-    } else if (prec == COPER_PREC_FP16X3) {
-      const float xs = x * sc;
-      const __half h = __float2half_rn(xs);
-      static_cast<__half*>(dst)[e] = h;
-      static_cast<__half*>(dst)[n + e] = __float2half_rn(xs - __half2float(h));
-    } else {
-      uint32_t h;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x));
-      float hf = __uint_as_float(h);
-      static_cast<float*>(dst)[e] = hf;
-      static_cast<float*>(dst)[n + e] = x - hf;
-    }
+    emit_prepared(prec, dst, n, e, x, sc);
   }
 }
 
 // fp16x3, one batch (B <= a few thousand rows): both backward operands - dy and dy scaled by the context - in ONE launch
-// instead of prepare(dy) + absmax_scaled + prepare_scaled.  Every block reduces its rows' maxima into tr_dy[1] (max |dy|)
-// and tr_dy[4] (max |dy| * max |c| per row), a grid-wide arrive counter (tr_dy[3]) tells when all are in, then the
-// blocks emit the planes.  tr_dy words 0..7 are zero on entry; the grid is capped so that all blocks are co-resident.
-// Same maxima, same exponent rule, same rounding as the three kernels it replaces -> same bits.
+// instead of prepare(dy) + absmax_scaled + prepare_scaled.  Every block reduces its rows' maxima into dy's trailer
+// (kTrMax: max |dy|, kTrMax2: max |dy| * max |c| per row) and waits at the grid barrier, then the blocks emit the planes.
+// tr_dy words 0..7 are zero on entry.  Same maxima, same exponent rule, same rounding as the three kernels it replaces
+// -> same bits.
 __global__ void __launch_bounds__(256) cpg_bwd_prepare_fp16x3_kernel(const float* __restrict__ dy,
                                                                      const float* __restrict__ c, int B, int d, int dc,
                                                                      int64_t ldp, __half* __restrict__ dyp,
@@ -222,53 +195,33 @@ __global__ void __launch_bounds__(256) cpg_bwd_prepare_fp16x3_kernel(const float
   if (threadIdx.x == 0) {
 #pragma unroll
     for (int w = 1; w < 8; ++w) { m_dy = fmaxf(m_dy, wmax[0][w]); m_dyc = fmaxf(m_dyc, wmax[1][w]); }
-    if (m_dy > 0.f) atomicMax(tr_dy + 1, __float_as_uint(m_dy));
-    if (m_dyc > 0.f) atomicMax(tr_dy + 4, __float_as_uint(m_dyc));
-    __threadfence();
-    atomicAdd(tr_dy + 3, 1u);
-    const long long t0 = clock64();
-    while (*reinterpret_cast<volatile uint32_t*>(tr_dy + 3) < gridDim.x) {
-      if (clock64() - t0 > 4000000000ll) __trap();
-    }
-    __threadfence();
+    trailer_max(tr_dy + kTrMax, m_dy);
+    trailer_max(tr_dy + kTrMax2, m_dyc);
+    grid_arrive_wait(tr_dy + kTrArrive);
   }
   __syncthreads();
-  const uint32_t bits_dy = *reinterpret_cast<volatile uint32_t*>(tr_dy + 1);
-  const uint32_t bits_dyc = *reinterpret_cast<volatile uint32_t*>(tr_dy + 4);
-  const int e_dy = fp16x3_exponent_of(__uint_as_float(bits_dy)), e_dyc = fp16x3_exponent_of(__uint_as_float(bits_dyc));
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    reinterpret_cast<int*>(tr_dy)[0] = e_dy;
-    tr_dy[2] = bits_dy;
-    reinterpret_cast<int*>(tr_dyc)[0] = e_dyc;
-    tr_dyc[1] = bits_dyc;
-  }
-  const float sc_dy = exp2f((float)e_dy), sc_dyc = exp2f((float)e_dyc);
+  const bool leader = blockIdx.x == 0 && threadIdx.x == 0;
+  const float sc_dy = fp16x3_publish(tr_dy, *reinterpret_cast<volatile uint32_t*>(tr_dy + kTrMax), kTrRunMax, leader);
+  const float sc_dyc = fp16x3_publish(tr_dyc, *reinterpret_cast<volatile uint32_t*>(tr_dy + kTrMax2), kTrMax, leader);
   // work unit = one 8-column group of one row of plane-set p (p = 0: dy, p = 1 + g: dy * c[:, g])
   const int gpr = (int)(ldp / 8);
   const int64_t per = (int64_t)B * gpr, units = per * (1 + dc);
-  __half* const dy_lo = dyp + (int64_t)B * ldp;
-  __half* const dyc_lo = dycp + (int64_t)dc * B * ldp;
   for (int64_t u = (int64_t)blockIdx.x * 256 + threadIdx.x; u < units; u += (int64_t)gridDim.x * 256) {
     const int p = (int)(u / per);
     const int64_t v = u - (int64_t)p * per;
     const int b = (int)(v / gpr), c0 = (int)(v - (int64_t)b * gpr) * 8;
     const float cs = p == 0 ? 1.0f : __ldg(c + (int64_t)b * dc + (p - 1));
-    const float sc = p == 0 ? sc_dy : sc_dyc;
-    __half2 h[4], l[4];
+    float x[8];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int j = c0 + 2 * k;
+    for (int k = 0; k < 8; k += 2) {
+      const int j = c0 + k;
       float x0 = j < d ? __ldg(dy + (int64_t)b * d + j) : 0.f, x1 = j + 1 < d ? __ldg(dy + (int64_t)b * d + j + 1) : 0.f;
       if (p != 0) { x0 = j < d ? x0 * cs : 0.f; x1 = j + 1 < d ? x1 * cs : 0.f; }
-      const float a0 = x0 * sc, a1 = x1 * sc;
-      h[k] = __floats2half2_rn(a0, a1);
-      const float2 hf = __half22float2(h[k]);
-      l[k] = __floats2half2_rn(a0 - hf.x, a1 - hf.y);
+      x[k] = x0;
+      x[k + 1] = x1;
     }
-    __half* hi = p == 0 ? dyp + v * 8 : dycp + ((int64_t)(p - 1) * per + v) * 8;
-    __half* lo = p == 0 ? dy_lo + v * 8 : dyc_lo + ((int64_t)(p - 1) * per + v) * 8;
-    *reinterpret_cast<uint4*>(hi) = *reinterpret_cast<uint4*>(h);
-    *reinterpret_cast<uint4*>(lo) = *reinterpret_cast<uint4*>(l);
+    emit_prepared_vec<COPER_PREC_FP16X3, 8>(p == 0 ? dyp : dycp, p == 0 ? (int64_t)B * ldp : (int64_t)dc * B * ldp,
+                                            (p == 0 ? v : (int64_t)(p - 1) * per + v) * 8, x, p == 0 ? sc_dy : sc_dyc);
   }
 }
 
@@ -280,10 +233,10 @@ static CpgBwdPlan cpg_bwd_plan(int B, int dc, int F, int d, int prec) {
   CpgBwdPlan L;
   size_t o = 0;
   // [f][P] first, at the same offsets as the forward plan (so a backward call may reuse them)
-  L.off_f = o; o = align_up(o + tc_prepared_bytes(B, F, prec), 256);
-  L.off_P = o; o = align_up(o + tc_prepared_bytes((int64_t)dc * F, d, prec), 256);
-  L.off_dy = o; o = align_up(o + tc_prepared_bytes(B, d, prec), 256);
-  L.off_dyc = o; o = align_up(o + tc_prepared_bytes((int64_t)dc * B, d, prec), 256);
+  L.off_f = o; o = align_up(o + prepared_bytes(B, F, prec), 256);
+  L.off_P = o; o = align_up(o + prepared_bytes((int64_t)dc * F, d, prec), 256);
+  L.off_dy = o; o = align_up(o + prepared_bytes(B, d, prec), 256);
+  L.off_dyc = o; o = align_up(o + prepared_bytes((int64_t)dc * B, d, prec), 256);
   L.dc_slabs = ((F + kBwdTBlockN - 1) / kBwdTBlockN) * (kBwdTEpiWarps / 4);
   L.off_dcpart = o; o = align_up(o + (size_t)L.dc_slabs * B * dc * sizeof(float), 256);
   L.total = o;
@@ -344,12 +297,12 @@ int umma_cpg_bwd(const float* c, const float* f, const float* P, const void* P_p
       if ((rc = tc_prepare(f, B, F, F, prec, fp, st))) return rc;
       if (!P_prepared && (rc = tc_prepare(P, (int64_t)dc * F, d, d, prec, w + L.off_P, st))) return rc;
     }
-    int64_t ldp = tc_prepared_ld(d, prec);
+    int64_t ldp = prepared_ld(d, prec);
     int64_t n = (int64_t)dc * B * ldp;
     if (prec == COPER_PREC_FP16X3 && n <= ((int64_t)8 << 20)) {
       // one launch for both operands (grid barrier: <= 2 co-resident blocks per SM)
-      uint32_t* tr_dy = static_cast<uint32_t*>(tc_fp16x3_trailer(dyp, B, d));
-      uint32_t* tr_dyc = static_cast<uint32_t*>(tc_fp16x3_trailer(dycp, (int64_t)dc * B, d));
+      uint32_t* tr_dy = fp16x3_trailer(dyp, B, d);
+      uint32_t* tr_dyc = fp16x3_trailer(dycp, (int64_t)dc * B, d);
       if ((rc = check_cuda(cudaMemsetAsync(tr_dy, 0, 32, st)))) return rc;
       const int64_t want = ((int64_t)(1 + dc) * B * (ldp / 8) + 256 * 4 - 1) / (256 * 4);
       int g = (int)(want < (int64_t)sm_count() * 2 ? want : (int64_t)sm_count() * 2);
@@ -362,7 +315,7 @@ int umma_cpg_bwd(const float* c, const float* f, const float* P, const void* P_p
       int grid = (int)((n + 255) / 256 < sm_count() * 8 ? (n + 255) / 256 : sm_count() * 8);
       uint32_t* trailer = nullptr;
       if (prec == COPER_PREC_FP16X3) {
-        trailer = static_cast<uint32_t*>(tc_fp16x3_trailer(dycp, (int64_t)dc * B, d));
+        trailer = fp16x3_trailer(dycp, (int64_t)dc * B, d);
         if ((rc = check_cuda(cudaMemsetAsync(trailer, 0, 8, st)))) return rc;
         launch_pdl(absmax_scaled_kernel, (B + 7) / 8, 256, 0, st, dy, c, B, d, dc, trailer);
         if ((rc = check_launch())) return rc;

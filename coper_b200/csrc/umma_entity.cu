@@ -12,21 +12,12 @@
 //
 // Three epilogues share the pipeline (umma_gemm.cuh):  ScoreEpiT (logits out), BceEpiT (loss + G + dbias partials),
 // RankEpiT (filtered-rank counts; logits never leave TMEM) plus DiagEpiT for the bit-identical gold logits.
-#include <cuda_fp16.h>
 #include "umma_gemm.cuh"
 #include "bce_math.cuh"
 
 namespace coper {
 using namespace umma;
 
-size_t tc_prepared_bytes(int64_t rows, int cols, int prec);                     // umma_score.cu
-int tc_prepare(const float* src, int64_t rows, int cols, int64_t ld_src, int prec, void* dst, cudaStream_t st);
-int64_t tc_prepared_ld(int cols, int prec);
-TcOperand tc_operand(const void* prep, int64_t rows, int cols, int prec);       // umma_gemm.cu
-void* tc_fp16x3_trailer(const void* prep, int64_t rows, int cols);
-int tc_gemm_store(int prec, bool a_mn, bool b_mn, const TcOperand& A, const TcOperand& B, const GemmProblem& p,
-                  bool split, const StoreEpi& epi, cudaStream_t st);
-int tc_plan_splits(int prec, GemmProblem p, bool split);
 // fused scorer + BCE + dq kernel (umma_fused.cu)
 bool umma_fused_ok(int B, int64_t Ns, int d, int prec);
 void umma_fused_plan(int B, int64_t Ns, int* QB, int* R);
@@ -151,30 +142,10 @@ struct BceEpiT : EpiBase {
       if (PREC == PREC_FP16X3) {
         // (sigmoid - z') * 2^10 as fp16 hi / lo planes, entity-major like the bf16 path
 #pragma unroll
-        for (int v = 0; v < 4; ++v) {
-          uint32_t hw[4], lw[4];
-#pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            const float a = g[8 * v + 2 * k], b = g[8 * v + 2 * k + 1];
-            const __half2 h = __floats2half2_rn(a, b);
-            const float2 hf = __half22float2(h);
-            const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-            hw[k] = *reinterpret_cast<const uint32_t*>(&h);
-            lw[k] = *reinterpret_cast<const uint32_t*>(&l);
-          }
-          pk[v] = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-          pk2[v] = make_uint4(lw[0], lw[1], lw[2], lw[3]);
-        }
+        for (int v = 0; v < 4; ++v) fp16_split8(g + 8 * v, pk[v], pk2[v]);
       } else if (PREC == PREC_BF16) {
 #pragma unroll
-        for (int v = 0; v < 4; ++v) {
-          __nv_bfloat162 t0 = __floats2bfloat162_rn(g[8 * v], g[8 * v + 1]);
-          __nv_bfloat162 t1 = __floats2bfloat162_rn(g[8 * v + 2], g[8 * v + 3]);
-          __nv_bfloat162 t2 = __floats2bfloat162_rn(g[8 * v + 4], g[8 * v + 5]);
-          __nv_bfloat162 t3 = __floats2bfloat162_rn(g[8 * v + 6], g[8 * v + 7]);
-          pk[v].x = *reinterpret_cast<uint32_t*>(&t0); pk[v].y = *reinterpret_cast<uint32_t*>(&t1);
-          pk[v].z = *reinterpret_cast<uint32_t*>(&t2); pk[v].w = *reinterpret_cast<uint32_t*>(&t3);
-        }
+        for (int v = 0; v < 4; ++v) pk[v] = bf16_pack8(g + 8 * v);
       } else if (PREC == PREC_TF32X3) {
         // tf32x3: 8 bytes per element in two planes - QUERY-major G[b, n] so that every store instruction of the warp
         // covers 32 consecutive entities (128 B); ldGT is the [N, ld] pitch here
@@ -183,10 +154,9 @@ struct BceEpiT : EpiBase {
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           if (j < ncol) {
-            uint32_t hb;
-            asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(g[j]));
-            *hi = __uint_as_float(hb);
-            *lo = g[j] - __uint_as_float(hb);
+            const float h = tf32_hi(g[j]);
+            *hi = h;
+            *lo = g[j] - h;
           }
           hi += ldGT;
           lo += ldGT;
@@ -475,10 +445,10 @@ struct TopkEpiT : EpiBase {
 // rows e2[b] - ent_lo of a prepared operand [Ns, ldp] -> [B, ldp] (zero rows when not owned); 16-byte vectors
 __global__ void gather_prepared_kernel(const uint4* __restrict__ src, int64_t Ns, int vec_per_row, int planes,
                                        const int64_t* __restrict__ e2, int64_t ent_lo, int B, uint4* __restrict__ dst,
-                                       const int* __restrict__ src_exp, int* __restrict__ dst_exp) {
+                                       const uint32_t* __restrict__ src_tr, uint32_t* __restrict__ dst_tr) {
   pdl_enter();
   int b = blockIdx.x;
-  if (src_exp && b == 0 && threadIdx.x == 0) *dst_exp = *src_exp;      // fp16x3: the gathered rows keep E's exponent
+  if (src_tr && b == 0 && threadIdx.x == 0) dst_tr[kTrExp] = src_tr[kTrExp];    // fp16x3: the rows keep E's exponent
   int64_t l = e2[b] - ent_lo;
   bool owned = l >= 0 && l < Ns;
   for (int pl = 0; pl < planes; ++pl) {
@@ -591,7 +561,7 @@ int umma_score1n_fwd_prepared(const void* q_prep, const void* E_prep, const floa
 }
 
 // ------------------------------------------------------------------------------------------ gold + rank
-size_t umma_rank_workspace_bytes(int B, int d, int prec) { return align_up(tc_prepared_bytes(B, d, prec), 256); }
+size_t umma_rank_workspace_bytes(int B, int d, int prec) { return align_up(prepared_bytes(B, d, prec), 256); }
 
 template <class Cfg>
 static int gold_impl(const TcOperand& Eg, const TcOperand& Q, const float* bias, int B, int64_t Ns, int d,
@@ -606,17 +576,11 @@ int umma_score1n_gold(const void* q_prep, const void* E_prep, const float* bias,
                       cudaStream_t st) {
   if (!ws || ws_bytes < umma_rank_workspace_bytes(B, d, prec) || (reinterpret_cast<uintptr_t>(ws) & 255))
     return COPER_ERR_WORKSPACE;
-  int64_t ldp = tc_prepared_ld(d, prec);
-  int elem = prec == COPER_PREC_TF32X3 ? 4 : 2;
-  int vec_per_row = (int)(ldp * elem / 16);
-  const int* src_exp = nullptr;
-  int* dst_exp = nullptr;
-  if (prec == COPER_PREC_FP16X3) {
-    src_exp = static_cast<const int*>(tc_fp16x3_trailer(E_prep, Ns, d));
-    dst_exp = static_cast<int*>(tc_fp16x3_trailer(ws, B, d));
-  }
-  launch_pdl(gather_prepared_kernel, B, 64, 0, st, static_cast<const uint4*>(E_prep), Ns, vec_per_row, prec ==
-             COPER_PREC_BF16 ? 1 : 2, e2, ent_lo, B, static_cast<uint4*>(ws), src_exp, dst_exp);
+  const int vec_per_row = (int)(prepared_ld(d, prec) * prepared_elem_bytes(prec) / 16);
+  const bool f16x3 = prec == COPER_PREC_FP16X3;
+  launch_pdl(gather_prepared_kernel, B, 64, 0, st, static_cast<const uint4*>(E_prep), Ns, vec_per_row,
+             prepared_planes(prec), e2, ent_lo, B, static_cast<uint4*>(ws), f16x3 ? fp16x3_trailer(E_prep, Ns, d) : nullptr,
+             f16x3 ? fp16x3_trailer(ws, B, d) : nullptr);
   int rc = check_launch();
   if (rc) return rc;
   TcOperand Q = tc_operand(q_prep, B, d, prec), Eg = tc_operand(ws, B, d, prec);
@@ -721,8 +685,8 @@ static BceTcLayout bce_tc_layout(int B, int64_t Ns, int d, int prec) {
     if (QB > L.dbias_slabs) L.dbias_slabs = QB;
   }
   size_t o = 0;
-  L.off_q = o; o = align_up(o + tc_prepared_bytes(B, d, prec), 256);
-  L.off_E = o; o = align_up(o + tc_prepared_bytes(Ns, d, prec), 256);
+  L.off_q = o; o = align_up(o + prepared_bytes(B, d, prec), 256);
+  L.off_E = o; o = align_up(o + prepared_bytes(Ns, d, prec), 256);
   L.off_dq = o; o = align_up(o + dq_rows * d * sizeof(float), 256);
   L.off_dbias = o; o = align_up(o + (size_t)L.dbias_slabs * Ns * sizeof(float), 256);
   L.off_loss = o; o = align_up(o + (size_t)sm_count() * kBceEpiWarps * sizeof(double), 256);

@@ -249,14 +249,7 @@ bce_dq_fused_kernel(const __grid_constant__ CUtensorMap tE, const __grid_constan
       const float rsum = rowok ? gsum : 0.f;
       uint4 pk[4];
 #pragma unroll
-      for (int v = 0; v < 4; ++v) {
-        __nv_bfloat162 a0 = __floats2bfloat162_rn(g[8 * v], g[8 * v + 1]);
-        __nv_bfloat162 a1 = __floats2bfloat162_rn(g[8 * v + 2], g[8 * v + 3]);
-        __nv_bfloat162 a2 = __floats2bfloat162_rn(g[8 * v + 4], g[8 * v + 5]);
-        __nv_bfloat162 a3 = __floats2bfloat162_rn(g[8 * v + 6], g[8 * v + 7]);
-        pk[v].x = *reinterpret_cast<uint32_t*>(&a0); pk[v].y = *reinterpret_cast<uint32_t*>(&a1);
-        pk[v].z = *reinterpret_cast<uint32_t*>(&a2); pk[v].w = *reinterpret_cast<uint32_t*>(&a3);
-      }
+      for (int v = 0; v < 4; ++v) pk[v] = bf16_pack8(g + 8 * v);
       if (tr) p.trace[i * 8 + TR_EPI_MATH_DONE] = clock64();
       // the G tile of the previous entity tile must have been consumed (dq MMAs + TMA store) before it is overwritten
       mbar_wait_guarded(&bar[B_GEMPTY], (uint32_t)((i & 1) ^ 1));

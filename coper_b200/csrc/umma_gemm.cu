@@ -5,11 +5,6 @@
 namespace coper {
 using namespace umma;
 
-size_t tc_prepared_bytes(int64_t rows, int cols, int prec);                     // umma_score.cu
-int tc_prepare(const float* src, int64_t rows, int cols, int64_t ld_src, int prec, void* dst, cudaStream_t st);
-int64_t tc_prepared_ld(int cols, int prec);
-void* tc_fp16x3_trailer(const void* prep, int64_t rows, int cols);
-
 // N-is-small configurations (N = d <= 256 in one tile): BLOCK_N = 256
 // tf32x3: 8 epilogue warps (128 promoted accumulators per thread), chains cut every 4 k-blocks (48 MMAs)
 // fp16x3: a k-block holds 64 k-elements (2 x 16 KB planes per operand tile row block): chains cut every 2 k-blocks
@@ -39,8 +34,6 @@ bool tc_resident_b_ok(int prec, bool a_mn, bool b_mn, const GemmProblem& p) {
          p.M >= 16 * BLOCK_M;
 }
 
-// p: M, N, K, groups, groups_inner and group offsets filled by the caller; tiling is planned here.
-// With split == true the caller must size `epi.out` for plan_splits() partial slabs.
 int tc_gemm_store(int prec, bool a_mn, bool b_mn, const TcOperand& A, const TcOperand& B, const GemmProblem& p,
                   bool split, const StoreEpi& epi, cudaStream_t st) {
   // (the resident-B variant measured slower than the streaming one for dE - the output stores dominate - and is kept
@@ -60,12 +53,12 @@ int tc_plan_splits(int prec, GemmProblem p, bool split) {
 
 TcOperand tc_operand(const void* prep, int64_t rows, int cols, int prec) {
   TcOperand o;
-  int64_t ldp = tc_prepared_ld(cols, prec);
+  int64_t ldp = prepared_ld(cols, prec);
   o.main = prep;
   o.lo = prec == COPER_PREC_TF32X3 ? static_cast<const void*>(static_cast<const float*>(prep) + rows * ldp)
          : prec == COPER_PREC_FP16X3 ? static_cast<const void*>(static_cast<const uint16_t*>(prep) + rows * ldp)
                                      : nullptr;
-  o.exp = prec == COPER_PREC_FP16X3 ? static_cast<const int*>(tc_fp16x3_trailer(prep, rows, cols)) : nullptr;
+  o.exp = prec == COPER_PREC_FP16X3 ? reinterpret_cast<const int*>(fp16x3_trailer(prep, rows, cols) + kTrExp) : nullptr;
   o.rows = (uint64_t)rows;
   o.cols = (uint64_t)cols;
   o.pitch = (uint64_t)ldp;
@@ -79,8 +72,8 @@ extern "C" {
 
 size_t coper_tc_gemm_workspace_bytes(int M, int N, int K, int prec) {
   // operands are prepared as stored: [M,K] or [K,M] / [K,N] or [N,K] -> same byte count either way (upper bound)
-  size_t a = tc_prepared_bytes(M > K ? M : K, M > K ? K : M, prec) + tc_prepared_bytes(K, M, prec);
-  size_t b = tc_prepared_bytes(N > K ? N : K, N > K ? K : N, prec) + tc_prepared_bytes(K, N, prec);
+  size_t a = prepared_bytes(M > K ? M : K, M > K ? K : M, prec) + prepared_bytes(K, M, prec);
+  size_t b = prepared_bytes(N > K ? N : K, N > K ? K : N, prec) + prepared_bytes(K, N, prec);
   return a + b + 1024;
 }
 
@@ -96,7 +89,7 @@ int coper_tc_gemm(int transA, int transB, int M, int N, int K, const float* A, i
   // operand B(k,n): !transB -> stored [K,N] (MN-major); transB -> stored [N,K] (K-major)
   int64_t b_rows = transB ? N : K, b_cols = transB ? K : N;
   void* Ap = p;
-  void* Bp = p + tc_prepared_bytes(a_rows, (int)a_cols, prec);
+  void* Bp = p + prepared_bytes(a_rows, (int)a_cols, prec);
   int rc;
   if ((rc = tc_prepare(A, a_rows, (int)a_cols, lda, prec, Ap, st))) return rc;
   if ((rc = tc_prepare(B, b_rows, (int)b_cols, ldb, prec, Bp, st))) return rc;

@@ -14,6 +14,7 @@
 //                right after they are read from TMEM (acc * 2^-(ea+eb) * post_scale).
 // Operands may be K-major (rows x 128 B tiles) or MN-major (k-rows x 128 B chunks); see umma.cuh.
 #pragma once
+#include "operand.cuh"
 #include "umma.cuh"
 
 namespace coper {
@@ -724,4 +725,13 @@ inline StoreEpi make_store_epi(float* out, long long ld, long long group_stride,
 }
 
 }  // namespace umma
+
+// ---- host entry points of the generic GEMM (umma_gemm.cu)
+// a prepared operand (operand.cuh) of a stored [rows, cols] matrix, as the kernels read it
+umma::TcOperand tc_operand(const void* prep, int64_t rows, int cols, int prec);
+// p: M, N, K, groups, groups_inner and group offsets filled by the caller; tiling is planned here.  With split == true
+// the caller must size `epi.out` for tc_plan_splits() partial slabs.
+int tc_gemm_store(int prec, bool a_mn, bool b_mn, const umma::TcOperand& A, const umma::TcOperand& B,
+                  const umma::GemmProblem& p, bool split, const umma::StoreEpi& epi, cudaStream_t st);
+int tc_plan_splits(int prec, umma::GemmProblem p, bool split);
 }  // namespace coper

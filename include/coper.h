@@ -204,12 +204,14 @@ size_t coper_score1n_workspace_bytes(int B, int64_t Ns, int d, int prec);
 int coper_score1n_fwd(const float* q, const float* E, const float* bias, int B, int64_t Ns, int d, float* scores,
                       int64_t ld_scores, void* workspace, size_t workspace_bytes, int prec, coper_stream_t stream);
 
-/* Tensor-pipe operand preparation (COPER_PREC_BF16 / COPER_PREC_TF32X3) for the operands of the tf.matmul calls
- * at models.py:70-73,412,433-437.  The tcgen05 kernels consume operands in
- * "prepared" form: a bf16 copy [rows, ldp] (ldp = cols rounded up to 8), or two fp32 planes (hi = tf32-rounded value,
- * lo = x - hi) of [rows, ldp] (ldp = cols rounded up to 4), or (FP16X3) two fp16 planes of [rows, ldp] (ldp = cols
- * rounded up to 8) holding hi / lo of x * 2^e followed by a 256-byte trailer whose first int32 is e.  Prepare the entity table once per evaluation pass /
- * optimizer step and reuse it across calls with coper_score1n_fwd_prepared (coper_score1n_fwd prepares per call). */
+/* Tensor-pipe operand preparation (COPER_PREC_BF16 / COPER_PREC_TF32X3 / COPER_PREC_FP16X3) for the operands of the
+ * tf.matmul calls at models.py:70-73,412,433-437.  The tcgen05 kernels consume operands in "prepared" form
+ * (csrc/operand.cuh): a bf16 copy [rows, ldp] (ldp = cols rounded up to 8), or two fp32 planes (hi = tf32-rounded
+ * value, lo = x - hi) of [rows, ldp] (ldp = cols rounded up to 4), or (FP16X3) two fp16 planes of [rows, ldp] (ldp =
+ * cols rounded up to 8) holding hi / lo of x * 2^e followed, 256-byte aligned, by a 256-byte trailer of uint32 words
+ * {e, max |x|, running max, ...}; e puts max |x| in [2^10, 2^11).  Padding columns are zero.  Prepare the entity
+ * table once per evaluation pass / optimizer step and reuse it across calls with coper_score1n_fwd_prepared
+ * (coper_score1n_fwd prepares per call). */
 size_t coper_prepared_bytes(int64_t rows, int cols, int prec);
 int coper_prepare_operand(const float* src, int64_t rows, int cols, int64_t ld_src, int prec, void* dst,
                           coper_stream_t stream);
@@ -218,7 +220,7 @@ int coper_score1n_fwd_prepared(const void* q_prep, const void* E_prep, const flo
 
 /* C = op(A).op(B) on the tensor pipe (tcgen05, fp32 accumulate in TMEM); same layout flags as coper_sgemm
  * (tf.matmul, models.py:60, and its autodiff twins).
- * Operands are prepared into the workspace on every call (bf16 copy or tf32 hi/lo planes). */
+ * Operands are prepared into the workspace on every call (coper_prepare_operand's format). */
 size_t coper_tc_gemm_workspace_bytes(int M, int N, int K, int prec);
 int coper_tc_gemm(int transA, int transB, int M, int N, int K, const float* A, int lda, const float* B, int ldb,
                   float* C, int ldc, int prec, void* workspace, size_t workspace_bytes, coper_stream_t stream);
@@ -469,8 +471,10 @@ int coper_amsgrad_step(float* theta, const float* grad, float* m, float* v, floa
  * multi-tensor form of the clip + AMSGrad tail (models.py:199, utils/amsgrad.py:130-159): the whole
  * variable list is processed by ONE launch per phase instead of one per variable.
  *   descs         device array [n_tensors] describing every trainable (pointers as in coper_amsgrad_step);
- *                 `prepared` (optional) is refreshed with the tensor-pipe operand form of the UPDATED variable
- *                 (bf16 copy, or tf32 hi plane followed by the lo plane; requires row pitch == row length),
+ *                 `prepared` (optional) is refreshed with the tensor-pipe operand form of the UPDATED variable in
+ *                 precision prepared_prec (coper_prepare_operand's format with row pitch == row length: the lo
+ *                 plane starts n elements after the hi plane, and an FP16X3 copy's trailer follows at n * 4 bytes
+ *                 rounded up to 256; it must hold a preparation's trailer, whose exponent the update keeps current),
  *                 so the next step's GEMMs need no separate conversion pass.
  *                 mode = COPER_GRAD_DENSE: the dense rule of coper_amsgrad_step.  mode = COPER_GRAD_INDEXED_SLICES: the
  *                 variable is read only through tf.nn.embedding_lookup (rel_emb, models.py:178), TF hands the

@@ -388,7 +388,9 @@ def test_multi_tensor_optimizer_matches_per_tensor(L, bug_compat):
     v = [torch.rand(*s, device="cuda", generator=g) for s in shapes]
     th2, vh2, m2, v2 = ([t.clone() for t in x] for x in (th, vh, m, v))
     prep = {0: (1, torch.zeros(lib.coper_prepared_bytes(40943, 200, 1), dtype=torch.uint8, device="cuda")),
-            4: (2, torch.zeros(lib.coper_prepared_bytes(8 * 4608, 40, 2), dtype=torch.uint8, device="cuda"))}
+            4: (2, torch.zeros(lib.coper_prepared_bytes(8 * 4608, 40, 2), dtype=torch.uint8, device="cuda")),
+            # n % 4 != 0: the 4-wide emission of a full chunk falls back to one element at a time
+            3: (2, torch.zeros(lib.coper_prepared_bytes(1, 16385, 2), dtype=torch.uint8, device="cuda"))}
     desc = np.zeros(len(shapes), dtype=L.PARAM_DESC)
     chunks, offs = [], [0]
     for i in range(len(shapes)):
@@ -431,12 +433,15 @@ def test_multi_tensor_optimizer_matches_per_tensor(L, bug_compat):
         assert torch.equal(th[i], th2[i]) and torch.equal(vh[i], vh2[i]), i
         if not bug_compat:
             assert torch.equal(m[i], m2[i]) and torch.equal(v[i], v2[i]), i
-    for i, (rows, cols) in ((0, (40943, 200)), (4, (8 * 4608, 40))):
+    for i, (rows, cols) in ((0, (40943, 200)), (4, (8 * 4608, 40)), (3, (1, 16385))):
         pr, buf = prep[i]
         chk = torch.zeros_like(buf)
         L.call("coper_prepare_operand", L.ptr(th[i]), rows, cols, cols, pr, L.ptr(chk))
-        n_bytes = rows * cols * (2 if pr == 1 else 8)
-        assert torch.equal(buf[:n_bytes], chk[:n_bytes]), i
+        # the optimizer's planes have pitch n; coper_prepare_operand's have pitch cols rounded up to 8 (bf16) / 4 (tf32)
+        esz, ldp = (2, -(-cols // 8) * 8) if pr == 1 else (4, -(-cols // 4) * 4)
+        n = rows * cols
+        for pl in range(1 if pr == 1 else 2):
+            assert torch.equal(buf[pl * n * esz:(pl + 1) * n * esz], chk[pl * rows * ldp * esz:pl * rows * ldp * esz + n * esz]), (i, pl)
 
 
 def test_reduce_partials_fixed_order(L):
