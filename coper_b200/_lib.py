@@ -67,6 +67,14 @@ SIGNATURES = {
     "coper_score1n_bce_fwd_bwd_norm": (i32, [vp, vp, vp, vp, vp, i32, i64, i32, f32, f32, f32, vp, vp, i64, vp, vp, vp, vp,
                                              vp, sz, i32, vp]),
     "coper_score1n_bce_dE": (i32, [vp, i32, i64, i32, f32, vp, vp, vp, vp, sz, i32, vp]),
+    "coper_score1n_lse_workspace_bytes": (sz, [i32, i64, i32, i32]),
+    "coper_score1n_lse": (i32, [vp, vp, vp, vp, i32, i64, i32, vp, vp, sz, i32, vp]),
+    "coper_lse_finalize": (i32, [vp, i32, i32, vp, vp]),
+    "coper_score1n_ce_dE_inv_count": (f32, [f32, i64, i32]),
+    "coper_score1n_ce_fwd_bwd": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, i64, f32, f32, vp, vp, i64, vp, vp, vp,
+                                       vp, sz, i32, vp]),
+    "coper_score1n_ce_fwd_bwd_norm": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i64, i32, i64, f32, f32, vp, vp, i64, vp, vp,
+                                            vp, vp, vp, sz, i32, vp]),
     "coper_sample_labels": (i32, [vp, vp, i32, i64, i32, i32, vp, u64, vp, vp, vp]),
     "coper_score_sampled_workspace_bytes": (sz, [i32, i32]),
     "coper_score_sampled_bce_fwd_bwd": (i32, [vp, vp, vp, vp, vp, i32, i32, i64, i32, f32, f32, f32, vp, vp, vp, vp, vp,

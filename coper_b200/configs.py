@@ -163,4 +163,5 @@ def model_descriptors(cfg: AttributeDict, num_ent: int, num_rel: int, use_cpg: b
         "batch_norm_momentum": m.get("batch_norm_momentum", 0.1),
         "batch_norm_train_stats": m.get("batch_norm_train_stats", False),
         "do_parameter_lookup": use_parameter_lookup,
+        "loss": m.get("loss", "bce"),       # "bce" (the reference's objective) or "softmax_ce" (include/coper.h)
     }

@@ -25,6 +25,18 @@ int umma_score1n_bce_fwd_bwd(const float* q, const float* E, const void* E_prepa
 int umma_score1n_dE(const void* G, int B, int64_t Ns, int d, float inv_count, float* dE, double* dE_sumsq, float* dbias,
                     void* ws, size_t ws_bytes, int prec, cudaStream_t st);
 
+// implemented in umma_entity.cu (tcgen05 path): softmax cross-entropy over all entities
+size_t umma_lse_workspace_bytes(int B, int64_t Ns, int d, int prec);
+int umma_score1n_lse(const float* q, const float* E, const void* E_prepared, const float* bias, int B, int64_t Ns, int d,
+                     float* ml, void* ws, size_t ws_bytes, int prec, cudaStream_t st);
+int lse_reduce(const float* parts, int S, int B, float* ml, float* lse, cudaStream_t st);
+float umma_ce_dE_inv_count(float inv_count, int64_t num_ent, int prec);
+int umma_score1n_ce_fwd_bwd(const float* q, const float* E, const void* E_prepared, const float* bias,
+                            const uint32_t* label_bits_t, const int32_t* rowptr, const float* lse, int B, int64_t Ns,
+                            int d, int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G, float* dq,
+                            float* dE, float* dbias, void* ws, size_t ws_bytes, int prec, double* dE_sumsq,
+                            cudaStream_t st);
+
 using namespace simt;
 
 struct BceArgs {
@@ -127,6 +139,126 @@ __global__ void __launch_bounds__(THREADS) score_kernel(const float* __restrict_
       int64_t n = n0 + threadIdx.x;
       if (n < Ns) bce.dbias_part[(int64_t)blockIdx.y * Ns + n] = s;
     }
+  }
+}
+
+// ---- softmax cross-entropy (include/coper.h), exact-fp32 engine
+// (m, l) = (max, sum exp(s - max)) of the logits of one batch row over one 128-entity tile: per thread over its 8
+// columns, then over the 16 threads that share the row in a fixed order
+__device__ __forceinline__ void lse_pair_combine(float& m, float& l, float m2, float l2) {
+  const float hi = fmaxf(m, m2);
+  l = l * expf(m - hi) + l2 * expf(m2 - hi);
+  m = hi;
+}
+__global__ void __launch_bounds__(THREADS, 1) score_lse_kernel(const float* __restrict__ q, const float* __restrict__ E,
+                                                            const float* __restrict__ bias, int B, int64_t Ns, int d,
+                                                            float2* __restrict__ part) {
+  pdl_enter();
+  __shared__ Smem sm;
+  int64_t n0 = (int64_t)blockIdx.x * BN;
+  int m0 = blockIdx.y * BM;
+  SrcK A{q, d, B, d};
+  SrcK Bs{E + n0 * d, d, Ns - n0, d};
+  float acc[8][8];
+  zero_acc(acc);
+  mainloop(A, Bs, m0, 0, 0, (d + BK - 1) / BK, acc, sm);
+  __syncthreads();                                  // the operand tiles are free: per-thread pairs [BM][16]
+  float2(*pairs)[16] = reinterpret_cast<float2(*)[16]>(&sm);
+  // logits in place; columns past the shard's last entity become -1e30 (exp = 0; the pair of a row without an
+  // entity here is (-1e30, 0) after the fixed combine below)
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int64_t n = n0 + mt_col(j);
+    const float bj = (n < Ns) ? __ldg(bias + n) : -1e30f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) acc[i][j] += bj;
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    float m = acc[i][0], l = 0.f;
+#pragma unroll
+    for (int j = 1; j < 8; ++j) m = fmaxf(m, acc[i][j]);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) l += (acc[i][j] > -1e30f) ? __expf(acc[i][j] - m) : 0.f;   // x <= 0: abs. error ~1e-7
+    pairs[mt_row(i)][threadIdx.x & 15] = make_float2(m, l);
+  }
+  __syncthreads();
+  if (threadIdx.x < BM && m0 + (int)threadIdx.x < B) {   // one thread per batch row: its 16 pairs in a fixed order
+    float2 acc2 = pairs[threadIdx.x][0];
+    for (int k = 1; k < 16; ++k) lse_pair_combine(acc2.x, acc2.y, pairs[threadIdx.x][k].x, pairs[threadIdx.x][k].y);
+    part[(int64_t)blockIdx.x * B + m0 + threadIdx.x] = acc2;
+  }
+}
+
+struct CeArgs {
+  const uint32_t* bits;
+  int64_t words;
+  const int32_t* rowptr;
+  const float* lse;
+  float eps, eN, inv_count;
+  float* loss_partials;  // [gridDim.y * gridDim.x]
+  float* dbias_part;     // [gridDim.y, Ns]
+};
+// G = (tau exp(s - lse) - t) * inv_count, loss = t (lse - s)
+__global__ void __launch_bounds__(THREADS) score_ce_kernel(const float* __restrict__ q, const float* __restrict__ E,
+                                                           const float* __restrict__ bias, int B, int64_t Ns, int d,
+                                                           float* __restrict__ out, int64_t ld, CeArgs ce) {
+  pdl_enter();
+  __shared__ Smem sm;
+  __shared__ float red32[32];
+  int64_t n0 = (int64_t)blockIdx.x * BN;
+  int m0 = blockIdx.y * BM;
+  SrcK A{q, d, B, d};
+  SrcK Bs{E + n0 * d, d, Ns - n0, d};
+  float acc[8][8];
+  zero_acc(acc);
+  mainloop(A, Bs, m0, 0, 0, (d + BK - 1) / BK, acc, sm);
+  float bj[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    int64_t n = n0 + mt_col(j);
+    bj[j] = (n < Ns) ? __ldg(bias + n) : 0.f;
+  }
+  float lsum = 0.f;
+  float cs[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) cs[j] = 0.f;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    int b = m0 + mt_row(i);
+    if (b >= B) continue;
+    const int nb = __ldg(ce.rowptr + b + 1) - __ldg(ce.rowptr + b);
+    const float tau = nb > 0 ? 1.0f : ce.eps;
+    const float pw = (1.0f - ce.eps) / (float)max(nb, 1);
+    const float lse = __ldg(ce.lse + b);
+    const uint32_t* brow = ce.bits + (int64_t)b * ce.words;
+    float* grow = out + (int64_t)b * ld + n0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      int64_t n = n0 + mt_col(j);
+      if (n >= Ns) continue;
+      uint32_t w = __ldg(brow + (n >> 5));
+      const float t = (((w >> (n & 31)) & 1u) ? pw : 0.f) + ce.eN;
+      const float s = acc[i][j] + bj[j];
+      const float g = (tau * expf(s - lse) - t) * ce.inv_count;
+      lsum += t * (lse - s);
+      cs[j] += g;
+      grow[mt_col(j)] = g;
+    }
+  }
+  float t = block_sum<float>(lsum, red32);
+  if (threadIdx.x == 0) ce.loss_partials[(int64_t)blockIdx.y * gridDim.x + blockIdx.x] = t;
+  float(*red)[BN] = reinterpret_cast<float(*)[BN]>(&sm.a[0][0][0]);
+  int ty = threadIdx.x >> 4;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) red[ty][mt_col(j)] = cs[j];
+  __syncthreads();
+  if (threadIdx.x < BN) {
+    float s = 0.f;
+#pragma unroll
+    for (int r = 0; r < 16; ++r) s += red[r][threadIdx.x];
+    int64_t n = n0 + threadIdx.x;
+    if (n < Ns) ce.dbias_part[(int64_t)blockIdx.y * Ns + n] = s;
   }
 }
 
@@ -245,6 +377,9 @@ size_t coper_score1n_bce_G_bytes(int B, int64_t Ns, int prec) {
   return (size_t)B * ((Ns + 31) / 32 * 32) * sizeof(float);
 }
 
+static int fp32_grad_tail(const float* q, const float* E, int B, int64_t Ns, int d, double* loss_sum, const float* G,
+                          int64_t ldG, float* dq, float* dE, float* dbias, void* workspace, coper_stream_t stream);
+
 static int score1n_bce_impl(const float* q, const float* E, const void* E_prepared, const float* bias,
                             const uint32_t* label_bits, int B, int64_t Ns, int d, float pos_target, float neg_target,
                             float inv_count, double* loss_sum, void* Gv, int64_t ldG, float* dq, float* dE, float* dbias,
@@ -264,11 +399,23 @@ static int score1n_bce_impl(const float* q, const float* E, const void* E_prepar
   char* ws = static_cast<char*>(workspace);
   float* loss_part = reinterpret_cast<float*>(ws + L.off_loss);
   float* dbias_part = reinterpret_cast<float*>(ws + L.off_dbias);
-  float* dq_part = reinterpret_cast<float*>(ws + L.off_dq);
   BceArgs bce{label_bits, (Ns + 31) / 32, pos_target, neg_target, inv_count, loss_part, dbias_part};
   launch_pdl(score_kernel<1>, dim3(L.gx, L.gy), THREADS, 0, st, q, E, bias, B, Ns, d, G, ldG, bce);
   int rc = check_launch();
   if (rc) return rc;
+  return fp32_grad_tail(q, E, B, Ns, d, loss_sum, G, ldG, dq, dE, dbias, workspace, stream);
+}
+
+// after the fp32 scorer pass (loss / dbias partials in the workspace, G): loss sum, dbias, dq = G.E, dE = G^T.q
+static int fp32_grad_tail(const float* q, const float* E, int B, int64_t Ns, int d, double* loss_sum, const float* G,
+                          int64_t ldG, float* dq, float* dE, float* dbias, void* workspace, coper_stream_t stream) {
+  BceLayout L = bce_layout(B, Ns, d);
+  cudaStream_t st = as_stream(stream);
+  char* ws = static_cast<char*>(workspace);
+  float* loss_part = reinterpret_cast<float*>(ws + L.off_loss);
+  float* dbias_part = reinterpret_cast<float*>(ws + L.off_dbias);
+  float* dq_part = reinterpret_cast<float*>(ws + L.off_dq);
+  int rc;
   launch_pdl(sum_to_double_kernel, 1, 1024, 0, st, loss_part, (int64_t)L.gx * L.gy, loss_sum);
   if ((rc = check_launch())) return rc;
   rc = coper_reduce_partials(dbias_part, L.gy, Ns, 1.0f, 0, dbias, stream);
@@ -303,6 +450,78 @@ int coper_score1n_bce_fwd_bwd_norm(const float* q, const float* E, const void* E
   COPER_CHECK_ARG(dE_sumsq);
   return score1n_bce_impl(q, E, E_prepared, bias, label_bits, B, Ns, d, pos_target, neg_target, inv_count, loss_sum, Gv,
                           ldG, dq, dE, dbias, workspace, workspace_bytes, prec, dE_sumsq, stream);
+}
+
+// ---- softmax cross-entropy over all entities
+size_t coper_score1n_lse_workspace_bytes(int B, int64_t Ns, int d, int prec) {
+  if (prec == COPER_PREC_FP32) return align_up((size_t)ceil_div(Ns, BN) * B * sizeof(float2), 256);
+  if (prec != COPER_PREC_BF16 && prec != COPER_PREC_TF32X3 && prec != COPER_PREC_FP16X3) return 0;
+  return umma_lse_workspace_bytes(B, Ns, d, prec);
+}
+int coper_score1n_lse(const float* q, const float* E, const void* E_prepared, const float* bias, int B, int64_t Ns, int d,
+                      float* ml, void* workspace, size_t workspace_bytes, int prec, coper_stream_t stream) {
+  COPER_CHECK_ARG(q && E && bias && ml && workspace && B > 0 && Ns > 0 && d > 0);
+  if (prec == COPER_PREC_BF16 || prec == COPER_PREC_TF32X3 || prec == COPER_PREC_FP16X3)
+    return umma_score1n_lse(q, E, E_prepared, bias, B, Ns, d, ml, workspace, workspace_bytes, prec, as_stream(stream));
+  if (prec != COPER_PREC_FP32) return COPER_ERR_UNSUPPORTED;
+  if (workspace_bytes < coper_score1n_lse_workspace_bytes(B, Ns, d, prec)) return COPER_ERR_WORKSPACE;
+  const int gx = ceil_div(Ns, BN);
+  cudaStream_t st = as_stream(stream);
+  float2* part = static_cast<float2*>(workspace);
+  launch_pdl(score_lse_kernel, dim3(gx, ceil_div(B, BM)), THREADS, 0, st, q, E, bias, B, Ns, d, part);
+  int rc = check_launch();
+  if (rc) return rc;
+  return lse_reduce(reinterpret_cast<const float*>(part), gx, B, ml, nullptr, st);
+}
+int coper_lse_finalize(const float* parts, int P, int B, float* lse, coper_stream_t stream) {
+  COPER_CHECK_ARG(parts && lse && P > 0 && B > 0);
+  return lse_reduce(parts, P, B, nullptr, lse, as_stream(stream));
+}
+float coper_score1n_ce_dE_inv_count(float inv_count, int64_t num_ent, int prec) {
+  return umma_ce_dE_inv_count(inv_count, num_ent, prec);
+}
+
+static int score1n_ce_impl(const float* q, const float* E, const void* E_prepared, const float* bias,
+                           const uint32_t* label_bits, const int32_t* rowptr, const float* lse, int B, int64_t Ns, int d,
+                           int64_t num_ent, float eps, float inv_count, double* loss_sum, void* Gv, int64_t ldG, float* dq,
+                           float* dE, float* dbias, void* workspace, size_t workspace_bytes, int prec, double* dE_sumsq,
+                           coper_stream_t stream) {
+  COPER_CHECK_ARG(q && E && bias && label_bits && rowptr && lse && loss_sum && Gv && dq && dbias && workspace);
+  COPER_CHECK_ARG(B > 0 && Ns > 0 && d > 0 && ldG >= Ns && num_ent >= Ns && eps >= 0.f && eps <= 1.f);
+  COPER_CHECK_ARG(dE || (prec != COPER_PREC_FP32 && dE_sumsq));   // dE == NULL: split call, see coper_score1n_bce_dE
+  if (prec == COPER_PREC_BF16 || prec == COPER_PREC_TF32X3 || prec == COPER_PREC_FP16X3)
+    return umma_score1n_ce_fwd_bwd(q, E, E_prepared, bias, label_bits, rowptr, lse, B, Ns, d, num_ent, eps, inv_count,
+                                   loss_sum, Gv, dq, dE, dbias, workspace, workspace_bytes, prec, dE_sumsq,
+                                   as_stream(stream));
+  if (prec != COPER_PREC_FP32) return COPER_ERR_UNSUPPORTED;
+  if (dE_sumsq) return COPER_ERR_UNSUPPORTED;
+  float* G = static_cast<float*>(Gv);
+  BceLayout L = bce_layout(B, Ns, d);
+  if (workspace_bytes < L.total) return COPER_ERR_WORKSPACE;
+  char* ws = static_cast<char*>(workspace);
+  CeArgs ce{label_bits, (Ns + 31) / 32, rowptr, lse, eps, (float)((double)eps / (double)num_ent), inv_count,
+            reinterpret_cast<float*>(ws + L.off_loss), reinterpret_cast<float*>(ws + L.off_dbias)};
+  launch_pdl(score_ce_kernel, dim3(L.gx, L.gy), THREADS, 0, as_stream(stream), q, E, bias, B, Ns, d, G, ldG, ce);
+  int rc = check_launch();
+  if (rc) return rc;
+  return fp32_grad_tail(q, E, B, Ns, d, loss_sum, G, ldG, dq, dE, dbias, workspace, stream);
+}
+int coper_score1n_ce_fwd_bwd(const float* q, const float* E, const void* E_prepared, const float* bias,
+                             const uint32_t* label_bits, const int32_t* rowptr, const float* lse, int B, int64_t Ns, int d,
+                             int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G, int64_t ldG,
+                             float* dq, float* dE, float* dbias, void* workspace, size_t workspace_bytes, int prec,
+                             coper_stream_t stream) {
+  return score1n_ce_impl(q, E, E_prepared, bias, label_bits, rowptr, lse, B, Ns, d, num_ent, eps, inv_count, loss_sum, G,
+                         ldG, dq, dE, dbias, workspace, workspace_bytes, prec, nullptr, stream);
+}
+int coper_score1n_ce_fwd_bwd_norm(const float* q, const float* E, const void* E_prepared, const float* bias,
+                                  const uint32_t* label_bits, const int32_t* rowptr, const float* lse, int B, int64_t Ns,
+                                  int d, int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G,
+                                  int64_t ldG, float* dq, float* dE, float* dbias, double* dE_sumsq, void* workspace,
+                                  size_t workspace_bytes, int prec, coper_stream_t stream) {
+  COPER_CHECK_ARG(dE_sumsq);
+  return score1n_ce_impl(q, E, E_prepared, bias, label_bits, rowptr, lse, B, Ns, d, num_ent, eps, inv_count, loss_sum, G,
+                         ldG, dq, dE, dbias, workspace, workspace_bytes, prec, dE_sumsq, stream);
 }
 
 }  // extern "C"

@@ -95,6 +95,66 @@ struct ScoreEpiT : EpiBase {
 // GEMMs read GT through TMA as an MN-major (dq) / K-major (dE) A operand.
 // Positives are sparse (a few per query out of N): the dense loop treats every element as a negative (no bit test) and
 // chunks that do contain a positive (warp vote) take the general path.
+// The warp's 32 entity rows x 32 query columns of dL/dS (g: this thread's row, 32 columns; ncol < 32 only in the last
+// query chunk) stored in the scorer-gradient operand form the dq / dE GEMMs read (CeEpiT).  BceEpiT keeps its own copy
+// of these lines inline: calling this helper from it reschedules the BCE kernels' SASS.
+template <int PREC>
+__device__ __forceinline__ void store_g(void* GT, int64_t ldGT, const GemmProblem& p, int row, int col, int ncol,
+                                        bool rowok, const float (&g)[32]) {
+  uint4 pk[4];
+  uint4 pk2[4];
+  if (rowok) {
+    if (PREC == PREC_FP16X3) {
+      // g (scaled by a power of two, see bce_impl / ce_impl) as fp16 hi / lo planes, entity-major like the bf16 path
+#pragma unroll
+      for (int v = 0; v < 4; ++v) fp16_split8(g + 8 * v, pk[v], pk2[v]);
+    } else if (PREC == PREC_BF16) {
+#pragma unroll
+      for (int v = 0; v < 4; ++v) pk[v] = bf16_pack8(g + 8 * v);
+    } else if (PREC == PREC_TF32X3) {
+      // tf32x3: 8 bytes per element in two planes - QUERY-major G[b, n] so that every store instruction of the warp
+      // covers 32 consecutive entities (128 B); ldGT is the [N, ld] pitch here
+      float* hi = static_cast<float*>(GT) + (int64_t)col * ldGT + row;
+      float* lo = hi + (int64_t)p.N * ldGT;
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        if (j < ncol) {
+          const float h = tf32_hi(g[j]);
+          *hi = h;
+          *lo = g[j] - h;
+        }
+        hi += ldGT;
+        lo += ldGT;
+      }
+    }
+  }
+  if (PREC == PREC_BF16 || PREC == PREC_FP16X3) {
+    // stage the warp's [32 entities x 32 queries] 16-bit block (64 B per row) through shared memory so that every
+    // store instruction writes 8 rows x 64 contiguous bytes (full sectors) instead of 32 rows x 16 bytes
+    __shared__ uint4 stage_g[kBceEpiWarps][128];
+    uint4* st = stage_g[(threadIdx.x >> 5) - 4];
+    const int lane = threadIdx.x & 31;
+    const int row0 = row - lane;
+    const int64_t ld16 = ldGT / 8;                    // row pitch in 16-byte units
+    const int gq = lane & 3;
+#pragma unroll
+    for (int plane = 0; plane < (PREC == PREC_FP16X3 ? 2 : 1); ++plane) {
+#pragma unroll
+      for (int v = 0; v < 4; ++v) st[lane * 4 + (v ^ ((lane >> 1) & 3))] = plane ? pk2[v] : pk[v];
+      __syncwarp();
+      uint4* o0 = reinterpret_cast<uint4*>(static_cast<uint16_t*>(GT) + ((int64_t)plane * p.M + row0) * ldGT + col);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const int rr = 8 * k + (lane >> 2);
+        const uint4 x = st[rr * 4 + (gq ^ ((rr >> 1) & 3))];
+        if (row0 + rr < p.M) o0[(int64_t)rr * ld16 + gq] = x;   // the pitch is padded to 32 queries: whole chunks writable
+      }
+      __syncwarp();
+    }
+  }
+}
+
+// (its G store is repeated in store_g, which CeEpiT calls: a change to one copy belongs in the other)
 template <int PREC, int NCH>
 struct BceEpiT : EpiBase {
   RowState<NCH> rs;
@@ -442,6 +502,187 @@ struct TopkEpiT : EpiBase {
   }
 };
 
+// ------------------------------------------------------------------------------------------ softmax cross-entropy
+// (include/coper.h, "Softmax cross-entropy over all entities").  Two passes over E: LseEpiT reduces each query column
+// to the pair (m, l) = (max_n s, sum_n exp(s - m)) over the CTA's entity rows - the logits never leave TMEM - and,
+// once lse_b is known across every shard, CeEpiT writes G = (tau_b exp(s - lse_b) - t_bn) / B in BCE's operand form.
+constexpr float kLseEmpty = -1e30f;   // m of a pair that has seen no logit (l = 0); exp(kLseEmpty - s) == 0
+__device__ __forceinline__ void lse_combine(float& m, float& l, float m2, float l2) {
+  const float hi = fmaxf(m, m2), lo = fminf(m, m2);
+  const float e = mufu_ex2((lo - hi) * 1.4426950408889634f);
+  l = (m >= m2) ? fmaf(l2, e, l) : fmaf(l, e, l2);
+  m = hi;
+}
+// Per chunk: the thread's 32 logits become pairs (s, 1) (padding rows and columns past the last query: (empty, 0)),
+// then a transposing warp reduction - 31 pair-combining shuffle steps per 32 columns - leaves in lane j the pair of
+// column chunk*32 + j over the warp's 32 entity rows, which is folded into the lane's running pair.  Every CTA keeps
+// one query block (lse_plan), so finish() writes each (CTA row group, lane quadrant, query) slot exactly once.
+template <int NCH>
+struct LseEpiT : EpiBase {
+  RowState<NCH> rs;
+  float2* part;             // [R * 4][N]: R = grid / n_tiles
+  float run_m[NCH], run_l[NCH];
+  int cur_col0;
+  __device__ __forceinline__ void tile_begin(const GemmProblem& p, const TileCoord&, int row, int col0) {
+    cur_col0 = col0;
+    rs.begin(p, row, col0);
+  }
+  __device__ __forceinline__ void tile_prefetch(const GemmProblem& p, const TileCoord&, int row, int col0) { rs.prefetch(p, row, col0); }
+  __device__ __forceinline__ void chunk(const GemmProblem& p, const TileCoord&, int row, int col, const uint32_t (&r)[32], int ci) {
+    const int lane = threadIdx.x & 31;
+    const bool rowok = row < p.M;
+    const int ncol = p.N - col;
+    float m[32], l[32];
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const bool ok = rowok && j < ncol;             // stale TMEM columns past the last query are never read as logits
+      m[j] = ok ? __uint_as_float(r[j]) + rs.bias_cur : kLseEmpty;
+      l[j] = ok ? 1.f : 0.f;
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) {
+      const bool upper = (lane & off) != 0;
+#pragma unroll
+      for (int q = 0; q < off; ++q) {
+        const float sm = upper ? m[q] : m[q + off], sl = upper ? l[q] : l[q + off];
+        float km = upper ? m[q + off] : m[q], kl = upper ? l[q + off] : l[q];
+        lse_combine(km, kl, __shfl_xor_sync(0xffffffffu, sm, off), __shfl_xor_sync(0xffffffffu, sl, off));
+        m[q] = km;
+        l[q] = kl;
+      }
+    }
+    lse_combine(run_m[ci], run_l[ci], m[0], l[0]);
+  }
+  __device__ __forceinline__ void finish(int, int) {
+    if (cur_col0 < 0) return;
+    const int lane = threadIdx.x & 31;
+    const int slot = (blockIdx.x / n_tiles) * 4 + ((threadIdx.x >> 5) & 3);
+#pragma unroll
+    for (int i = 0; i < NCH; ++i) {
+      const int c = cur_col0 + i * 32 + lane;
+      if (c < n_queries) part[(int64_t)slot * n_queries + c] = make_float2(run_m[i], run_l[i]);
+    }
+  }
+  int n_tiles, n_queries;
+};
+
+// G = (tau_b exp(s - lse_b) - t_bn) * ic with t_bn = [n in P_b] pw_b + eps/N, tau_b = eps + (1 - eps)[n_b > 0],
+// pw_b = (1 - eps) / max(n_b, 1); loss = sum t (lse - s).  Per query column the owning lane holds lse' = lse - log tau
+// (+inf for tau = 0), lse and pw; elements read them by broadcast shuffle (no shared memory: the resident fp16x3
+// configuration has none to spare).  Dense chunks (no positive, all 32 columns, warp vote as in BceEpiT):
+// g = exp(s - lse') ic - eN ic and the chunk's loss eN (sum_j lse_j - sum_j s_j) with the warp-uniform sum_j lse_j.
+template <int PREC, int NCH>
+struct CeEpiT : EpiBase {
+  RowState<NCH> rs;
+  const float* lse;         // [N]
+  const int32_t* rowptr;    // [N + 1]: global positive counts n_b = rowptr[b+1] - rowptr[b]
+  float eps, eN, ic;        // ic: factor applied to g (1/B, or fp16x3: a power of two from num_ent, see ce_g_scale)
+  float rsum_scale;         // dbias = rsum_scale * sum g
+  void* GT;
+  int64_t ldGT;
+  float* dbias_part;        // [n_tiles * col_groups][M]
+  double* loss_part;        // [grid * epi_warps]
+  double loss_acc;
+  float rsum;
+  int cur_col0;
+  float lsep[NCH], lsev[NCH], pw[NCH], slse[NCH];
+  __device__ __forceinline__ void tile_begin(const GemmProblem& p, const TileCoord&, int row, int col0) {
+    if (col0 != cur_col0) {
+      cur_col0 = col0;
+      const int lane = threadIdx.x & 31;
+#pragma unroll
+      for (int i = 0; i < NCH; ++i) {
+        const int c = col0 + i * 32 + lane;
+        float lv = 0.f, lp = INFINITY, w = 0.f;
+        if (c < p.N) {
+          const int nb = __ldg(rowptr + c + 1) - __ldg(rowptr + c);
+          const float tau = nb > 0 ? 1.0f : eps;
+          lv = __ldg(lse + c);
+          lp = tau > 0.f ? lv - logf(tau) : INFINITY;
+          w = (1.0f - eps) / (float)max(nb, 1);
+        }
+        lsep[i] = lp; lsev[i] = lv; pw[i] = w;
+        slse[i] = warp_sum(lv);
+      }
+    }
+    rs.begin(p, row, col0);
+    rsum = 0.f;
+  }
+  __device__ __forceinline__ void tile_prefetch(const GemmProblem& p, const TileCoord&, int row, int col0) { rs.prefetch(p, row, col0); }
+  __device__ __forceinline__ void chunk(const GemmProblem& p, const TileCoord&, int row, int col, const uint32_t (&r)[32],
+                                        int ci) {
+    const bool rowok = row < p.M;
+    const int ncol = p.N - col;
+    const uint32_t vm = ncol >= 32 ? 0xFFFFFFFFu : ((1u << ncol) - 1u);
+    const uint32_t w = rowok ? (rs.w_cur[ci] & vm) : 0u;
+    float g[32];
+    float lsum = 0.f, gsum = 0.f;
+    const float lp = lsep[ci];
+    if (ncol < 32 || __any_sync(0xffffffffu, w != 0u)) {
+      const float lv = lsev[ci], pwv = pw[ci];
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        const float s = __uint_as_float(r[j]) + rs.bias_cur;
+        const float lpj = __shfl_sync(0xffffffffu, lp, j), lvj = __shfl_sync(0xffffffffu, lv, j);
+        const float pwj = __shfl_sync(0xffffffffu, pwv, j);
+        const bool ok = (vm >> j) & 1u;
+        const float t = (((w >> j) & 1u) ? pwj : 0.f) + eN;
+        const float gj = ok ? (mufu_ex2((s - lpj) * 1.4426950408889634f) - t) * ic : 0.f;
+        lsum += ok ? t * (lvj - s) : 0.f;
+        g[j] = gj;
+        gsum += gj;
+      }
+    } else {
+      float ssum = 0.f;
+      const float c0 = -eN * ic;
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        const float s = __uint_as_float(r[j]) + rs.bias_cur;
+        const float e = mufu_ex2((s - __shfl_sync(0xffffffffu, lp, j)) * 1.4426950408889634f);
+        const float gj = fmaf(e, ic, c0);
+        ssum += s;
+        g[j] = gj;
+        gsum += gj;
+      }
+      lsum = eN * (slse[ci] - ssum);
+    }
+    if (rowok) {
+      loss_acc += (double)lsum;
+      rsum += gsum * rsum_scale;
+    }
+    store_g<PREC>(GT, ldGT, p, row, col, ncol, rowok, g);
+  }
+  __device__ __forceinline__ void tile_done(const GemmProblem& p, const TileCoord& t, int row, int col_group, int col_groups) {
+    if (row < p.M) dbias_part[(int64_t)(t.n_blk * col_groups + col_group) * p.M + row] = rsum;
+  }
+  __device__ __forceinline__ void finish(int epi_thread, int epi_threads) {
+    double t = warp_sum_d(loss_acc);
+    if ((epi_thread & 31) == 0) loss_part[(int64_t)blockIdx.x * (epi_threads >> 5) + (epi_thread >> 5)] = t;
+  }
+};
+
+// parts [S][B] (m, l) -> fixed-order combine per query (fp64 sum): ml [B] pairs, or (final) lse [B] = m + log l
+__global__ void lse_reduce_kernel(const float2* __restrict__ parts, int S, int B, float2* __restrict__ ml,
+                                  float* __restrict__ lse) {
+  pdl_enter();
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  float m = kLseEmpty;
+  for (int s = 0; s < S; ++s) m = fmaxf(m, parts[(int64_t)s * B + b].x);
+  double l = 0.0;
+  for (int s = 0; s < S; ++s) {
+    const float2 v = parts[(int64_t)s * B + b];
+    l += (double)v.y * exp((double)v.x - (double)m);
+  }
+  if (lse) lse[b] = (float)((double)m + log(l));
+  else ml[b] = make_float2(m, (float)l);
+}
+int lse_reduce(const float* parts, int S, int B, float* ml, float* lse, cudaStream_t st) {
+  launch_pdl(lse_reduce_kernel, (B + 127) / 128, 128, 0, st, reinterpret_cast<const float2*>(parts), S, B,
+             reinterpret_cast<float2*>(ml), lse);
+  return check_launch();
+}
+
 // rows e2[b] - ent_lo of a prepared operand [Ns, ldp] -> [B, ldp] (zero rows when not owned); 16-byte vectors
 __global__ void gather_prepared_kernel(const uint4* __restrict__ src, int64_t Ns, int vec_per_row, int planes,
                                        const int64_t* __restrict__ e2, int64_t ent_lo, int B, uint4* __restrict__ dst,
@@ -774,6 +1015,36 @@ int umma_score1n_dE(const void* G, int B, int64_t Ns, int d, float inv_count, fl
   return dE_gemm(prec, prec == COPER_PREC_TF32X3, Go, Qo, p, epi, dE_sumsq, reinterpret_cast<double*>(w + L.off_ss), st);
 }
 
+// Passes 2 and 3 of the unfused scorer gradient, after the scorer pass left G, the loss partials of its `grid` CTAs
+// and the dbias slabs: dq = g_post-scaled G . E and the loss sum, then (dE != NULL) dbias and dE = G^T . q.
+static int grad_gemms(void* G, const TcOperand& Eo, int B, int64_t Ns, int d, float g_post, float inv_count,
+                      double* loss_sum, float* dq, float* dE, float* dbias, void* ws, size_t ws_bytes, int prec,
+                      double* dE_sumsq, int grid, cudaStream_t st) {
+  const bool entity_major = prec != COPER_PREC_TF32X3;
+  BceTcLayout L = bce_tc_layout(B, Ns, d, prec);
+  char* w = static_cast<char*>(ws);
+  float* dq_part = reinterpret_cast<float*>(w + L.off_dq);
+  double* loss_part = reinterpret_cast<double*>(w + L.off_loss);
+  TcOperand Go = g_operand(G, B, Ns, prec);
+  int rc;
+  // ---- pass 2: dq = G . E   (A(b, n): GT is the MN-major form, G the K-major form; B = E stored [K, N] -> MN-major)
+  {
+    GemmProblem p{};
+    p.M = B; p.N = d; p.K = (int)Ns; p.groups = 1; p.groups_inner = 0;
+    p.post_scale = g_post;
+    StoreEpi epi = make_store_epi(dq_part, d, 0, (long long)B * d);
+    if ((rc = tc_gemm_store(prec, entity_major, true, Go, Eo, p, true, epi, st))) return rc;
+    // dq slabs and the loss partials of pass 1: one launch
+    if ((rc = reduce_partials_and_sum(dq_part, L.splits, (int64_t)B * d, 1.0f, 0, dq, loss_part, grid * kBceEpiWarps,
+                                      loss_sum, st)))
+      return rc;
+  }
+  // ---- pass 3: dE = G^T . q (A(n, b): GT is the K-major form, G the MN-major form; B = q stored [K, N] -> MN-major),
+  // preceded by the dbias slab reduction
+  if (!dE) return COPER_OK;                            // the caller runs umma_score1n_dE itself (second stream)
+  return umma_score1n_dE(G, B, Ns, d, inv_count, dE, dE_sumsq, dbias, ws, ws_bytes, prec, st);
+}
+
 int umma_score1n_bce_fwd_bwd(const float* q, const float* E, const void* E_prepared, const float* bias,
                              const uint32_t* label_bits_t, int B, int64_t Ns, int d, float pos, float neg,
                              float inv_count, double* loss_sum, void* G, int64_t ldG, float* dq, float* dE,
@@ -781,8 +1052,7 @@ int umma_score1n_bce_fwd_bwd(const float* q, const float* E, const void* E_prepa
   if (Ns > 0x7fffffff - 512) return COPER_ERR_UNSUPPORTED;
   (void)ldG;                                          // the tensor-pipe engines lay G out entity-major themselves
   if (reinterpret_cast<uintptr_t>(G) & 127) return COPER_ERR_INVALID_ARG;
-  const bool entity_major = prec != COPER_PREC_TF32X3;
-  const int64_t ldGT = entity_major ? gt_pitch(B) : (Ns + 31) / 32 * 32;
+  const int64_t ldGT = prec != COPER_PREC_TF32X3 ? gt_pitch(B) : (Ns + 31) / 32 * 32;
   const float g_post = prec == COPER_PREC_FP16X3 ? inv_count * (1.0f / 1024.0f) : 0.f;   // see bce_impl
   BceTcLayout L = bce_tc_layout(B, Ns, d, prec);
   if (!ws || ws_bytes < L.total) return COPER_ERR_WORKSPACE;
@@ -830,23 +1100,145 @@ int umma_score1n_bce_fwd_bwd(const float* q, const float* E, const void* E_prepa
                                                      dbias_part, loss_part, st, &grid);
   };
   if ((rc = run_bce())) return rc;
-  TcOperand Go = g_operand(G, B, Ns, prec);
-  // ---- pass 2: dq = G . E   (A(b, n): GT is the MN-major form, G the K-major form; B = E stored [K, N] -> MN-major)
-  {
-    GemmProblem p{};
-    p.M = B; p.N = d; p.K = (int)Ns; p.groups = 1; p.groups_inner = 0;
-    p.post_scale = g_post;
-    StoreEpi epi = make_store_epi(dq_part, d, 0, (long long)B * d);
-    if ((rc = tc_gemm_store(prec, entity_major, true, Go, Eo, p, true, epi, st))) return rc;
-    // dq slabs and the loss partials of pass 1: one launch
-    if ((rc = reduce_partials_and_sum(dq_part, L.splits, (int64_t)B * d, 1.0f, 0, dq, loss_part, grid * kBceEpiWarps,
-                                      loss_sum, st)))
+  return grad_gemms(G, Eo, B, Ns, d, g_post, inv_count, loss_sum, dq, dE, dbias, ws, ws_bytes, prec, dE_sumsq, grid, st);
+}
+
+// ------------------------------------------------------------------------------------------ softmax cross-entropy
+// Every CTA keeps one query block (n_tiles <= SMs): R CTA row groups x n_tiles query blocks, 4 slots per CTA
+static bool lse_plan(int B, int64_t Ns, int d, int prec, int* R) {
+  const int bn = ent_block_n(d, prec, Ns, B);
+  const int n_tiles = (B + bn - 1) / bn, sms = sm_count();
+  const int64_t m_tiles = (Ns + BLOCK_M - 1) / BLOCK_M;
+  if (n_tiles > sms) return false;
+  *R = (int)std::min<int64_t>(m_tiles, sms / n_tiles);
+  return true;
+}
+struct LseTcLayout {
+  size_t off_q, off_E, off_part, total;
+  int slots;
+};
+static LseTcLayout lse_tc_layout(int B, int64_t Ns, int d, int prec) {
+  LseTcLayout L{};
+  int R = 1;
+  lse_plan(B, Ns, d, prec, &R);
+  L.slots = 4 * R;
+  size_t o = 0;
+  L.off_q = o; o = align_up(o + prepared_bytes(B, d, prec), 256);
+  L.off_E = o; o = align_up(o + prepared_bytes(Ns, d, prec), 256);
+  L.off_part = o; o = align_up(o + (size_t)L.slots * B * sizeof(float2), 256);
+  L.total = o;
+  return L;
+}
+size_t umma_lse_workspace_bytes(int B, int64_t Ns, int d, int prec) { return lse_tc_layout(B, Ns, d, prec).total; }
+
+template <class Cfg>
+static int lse_impl(const TcOperand& E, const TcOperand& Q, const float* bias, int B, int64_t Ns, int d, float2* part,
+                    int R, cudaStream_t st) {
+  GemmProblem p = ent_problem(B, Ns, d, Cfg::BLOCK_N);
+  constexpr int kEntNCH = ent_nch<Cfg>();
+  LseEpiT<kEntNCH> epi;
+  epi.rs.init(bias, nullptr, 0);
+  epi.part = part;
+  for (int i = 0; i < kEntNCH; ++i) { epi.run_m[i] = kLseEmpty; epi.run_l[i] = 0.f; }
+  epi.cur_col0 = -1;
+  epi.n_tiles = p.n_tiles;
+  epi.n_queries = B;
+  return launch_gemm<Cfg, LseEpiT<kEntNCH>>(E, Q, p, epi, st, R * p.n_tiles);
+}
+int umma_score1n_lse(const float* q, const float* E, const void* E_prepared, const float* bias, int B, int64_t Ns, int d,
+                     float* ml, void* ws, size_t ws_bytes, int prec, cudaStream_t st) {
+  if (Ns > 0x7fffffff - 512) return COPER_ERR_UNSUPPORTED;
+  int R;
+  if (!lse_plan(B, Ns, d, prec, &R)) return COPER_ERR_UNSUPPORTED;
+  LseTcLayout L = lse_tc_layout(B, Ns, d, prec);
+  if (!ws || ws_bytes < L.total) return COPER_ERR_WORKSPACE;
+  if (reinterpret_cast<uintptr_t>(ws) & 255) return COPER_ERR_INVALID_ARG;
+  char* w = static_cast<char*>(ws);
+  int rc;
+  if ((rc = tc_prepare(q, B, d, d, prec, w + L.off_q, st))) return rc;
+  if (!E_prepared && (rc = tc_prepare(E, Ns, d, d, prec, w + L.off_E, st))) return rc;
+  TcOperand Q = tc_operand(w + L.off_q, B, d, prec), Eo = tc_operand(E_prepared ? E_prepared : w + L.off_E, Ns, d, prec);
+  float2* part = reinterpret_cast<float2*>(w + L.off_part);
+  rc = [&]() -> int { ENT_DISPATCH(lse_impl, Eo, Q, bias, B, Ns, d, part, R, st); }();
+  if (rc) return rc;
+  return lse_reduce(reinterpret_cast<const float*>(part), L.slots, B, ml, nullptr, st);
+}
+
+// fp16x3 carries the CE gradient times 2^k in fp16 planes: most entries are ~1/N, and 2^10 (BCE) would push the lo plane
+// of a 10 M-entity table into fp16 subnormals.  |g| <= 1, so 2^15 still leaves room below the fp16 maximum.
+static float ce_g_scale(int64_t num_ent) {
+  int k = 10;
+  while (k < 15 && ((int64_t)1 << k) < num_ent) ++k;
+  return (float)(1 << k);
+}
+float umma_ce_dE_inv_count(float inv_count, int64_t num_ent, int prec) {
+  return prec == COPER_PREC_FP16X3 ? inv_count * (1024.0f / ce_g_scale(num_ent)) : inv_count;
+}
+
+template <class Cfg>
+static int ce_impl(const TcOperand& E, const TcOperand& Q, const float* bias, const uint32_t* bitsT, const int32_t* rowptr,
+                   const float* lse, int B, int64_t Ns, int d, int64_t num_ent, float eps, float inv_count, void* GT,
+                   int64_t ldGT, float* dbias_part, double* loss_part, cudaStream_t st, int* grid_out) {
+  GemmProblem p = ent_problem(B, Ns, d, Cfg::BLOCK_N);
+  constexpr int kEntNCH = ent_nch<Cfg>();
+  constexpr int PREC = Cfg::PREC;
+  CeEpiT<PREC, kEntNCH> epi;
+  epi.rs.init(bias, bitsT, (B + 31) / 32);
+  epi.lse = lse; epi.rowptr = rowptr;
+  epi.eps = eps; epi.eN = (float)((double)eps / (double)num_ent);
+  epi.ic = PREC == PREC_FP16X3 ? ce_g_scale(num_ent) : inv_count;
+  epi.rsum_scale = PREC == PREC_FP16X3 ? inv_count / ce_g_scale(num_ent) : 1.0f;
+  epi.GT = GT; epi.ldGT = ldGT;
+  epi.dbias_part = dbias_part; epi.loss_part = loss_part; epi.loss_acc = 0.0; epi.rsum = 0.f;
+  epi.cur_col0 = -1;
+  for (int i = 0; i < kEntNCH; ++i) epi.lsep[i] = epi.lsev[i] = epi.pw[i] = epi.slse[i] = 0.f;
+  *grid_out = ent_grid(p);
+  return launch_gemm<Cfg, CeEpiT<PREC, kEntNCH>>(E, Q, p, epi, st, *grid_out);
+}
+
+int umma_score1n_ce_fwd_bwd(const float* q, const float* E, const void* E_prepared, const float* bias,
+                            const uint32_t* label_bits_t, const int32_t* rowptr, const float* lse, int B, int64_t Ns,
+                            int d, int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G, float* dq,
+                            float* dE, float* dbias, void* ws, size_t ws_bytes, int prec, double* dE_sumsq,
+                            cudaStream_t st) {
+  if (Ns > 0x7fffffff - 512) return COPER_ERR_UNSUPPORTED;
+  if (reinterpret_cast<uintptr_t>(G) & 127) return COPER_ERR_INVALID_ARG;
+  const int64_t ldGT = prec != COPER_PREC_TF32X3 ? gt_pitch(B) : (Ns + 31) / 32 * 32;
+  const float ic_dE = umma_ce_dE_inv_count(inv_count, num_ent, prec);
+  const float g_post = prec == COPER_PREC_FP16X3 ? ic_dE * (1.0f / 1024.0f) : 0.f;
+  BceTcLayout L = bce_tc_layout(B, Ns, d, prec);
+  if (!ws || ws_bytes < L.total) return COPER_ERR_WORKSPACE;
+  if (reinterpret_cast<uintptr_t>(ws) & 255) return COPER_ERR_INVALID_ARG;
+  char* w = static_cast<char*>(ws);
+  void* qp = w + L.off_q;
+  const void* Ep = E_prepared ? E_prepared : w + L.off_E;
+  float* dbias_part = reinterpret_cast<float*>(w + L.off_dbias);
+  double* loss_part = reinterpret_cast<double*>(w + L.off_loss);
+  int rc;
+  if ((rc = tc_prepare(q, B, d, d, prec, qp, st))) return rc;
+  if (!E_prepared && (rc = tc_prepare(E, Ns, d, d, prec, w + L.off_E, st))) return rc;
+  TcOperand Qo = tc_operand(qp, B, d, prec), Eo = tc_operand(Ep, Ns, d, prec);
+  int grid = 0;
+  const bool res = ent_resident(d, prec, Ns, B);
+#define CE_RUN(P, RES) ce_impl<BceSel<P, RES>::Cfg>(Eo, Qo, bias, label_bits_t, rowptr, lse, B, Ns, d, num_ent, eps, \
+                                                    inv_count, G, ldGT, dbias_part, loss_part, st, &grid)
+  if (prec == COPER_PREC_BF16) rc = res ? CE_RUN(PREC_BF16, true) : CE_RUN(PREC_BF16, false);
+  else if (prec == COPER_PREC_FP16X3) rc = res ? CE_RUN(PREC_FP16X3, true) : CE_RUN(PREC_FP16X3, false);
+  else rc = CE_RUN(PREC_TF32X3, false);
+#undef CE_RUN
+  if (rc) return rc;
+  if (umma_fused_ok(B, Ns, d, prec)) {
+    // umma_score1n_dE reduces the QB dbias slabs the fused BCE kernel writes for these arguments; the CE pass wrote the
+    // unfused slab set (always more than QB slabs): fold slabs 1.. into slab 0 and zero slabs 1..QB-1, so that the later
+    // QB-slab sum is exact and the same for the split and the unsplit call
+    int QB, R;
+    umma_fused_plan(B, Ns, &QB, &R);
+    const int slabs = ((B + ent_block_n(d, prec, Ns, B) - 1) / ent_block_n(d, prec, Ns, B)) * (kBceEpiWarps / 4);
+    if ((rc = coper_reduce_partials(dbias_part + Ns, slabs - 1, Ns, 1.0f, 1, dbias_part, (coper_stream_t)st))) return rc;
+    if (QB > 1 && (rc = check_cuda(cudaMemsetAsync(dbias_part + Ns, 0, (size_t)(QB - 1) * Ns * sizeof(float), st))))
       return rc;
   }
-  // ---- pass 3: dE = G^T . q (A(n, b): GT is the K-major form, G the MN-major form; B = q stored [K, N] -> MN-major),
-  // preceded by the dbias slab reduction
-  if (!dE) return COPER_OK;                            // the caller runs umma_score1n_dE itself (second stream)
-  return umma_score1n_dE(G, B, Ns, d, inv_count, dE, dE_sumsq, dbias, ws, ws_bytes, prec, st);
+  return grad_gemms(G, Eo, B, Ns, d, g_post, ic_dE, loss_sum, dq, dE, dbias, ws, ws_bytes, prec, dE_sumsq, grid, st);
 }
 
 }  // namespace coper

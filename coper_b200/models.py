@@ -163,6 +163,12 @@ class _BatchSlot:
         ws = max(lib.coper_score1n_bce_workspace_bytes(B, Ns, d, m.prec),
                  lib.coper_score1n_workspace_bytes(B, Ns, d, m.prec),
                  lib.coper_segscatter_workspace_bytes(B), lib.coper_score1n_rank_workspace_bytes(B, d, m.prec))
+        # softmax cross-entropy: this rank's log-sum-exp pairs, every rank's pairs and the finalised lse per query
+        self.ml = self.ml_all = self.lse = None
+        if m.loss == "softmax_ce":
+            ws = max(ws, lib.coper_score1n_lse_workspace_bytes(B, Ns, d, m.prec))
+            self.ml, self.lse = z(B, 2), z(B)
+            self.ml_all = z(m.world, B, 2) if m.world > 1 else None
         self.ws = torch.empty(ws, dtype=torch.uint8, device=dev)
         self.ws_bytes = ws
         # context nets: activations per hidden layer for the two generators
@@ -279,6 +285,14 @@ class ConvE:
         # ---- descriptors (models.py:98-128)
         self.use_negative_sampling = md.get("use_negative_sampling", False)
         self.label_smoothing_epsilon = float(md["label_smoothing_epsilon"])
+        # training objective over the full 1-N scores: "bce" (models.py:448-453) or "softmax_ce", the softmax
+        # cross-entropy over all entities (include/coper.h; 1vsAll / KvsAll-CE)
+        self.loss = md.get("loss", "bce")
+        if self.loss not in ("bce", "softmax_ce"):
+            raise ValueError("loss must be 'bce' or 'softmax_ce', not %r" % (self.loss,))
+        if self.loss == "softmax_ce" and self.use_negative_sampling:
+            raise NotImplementedError("loss='softmax_ce' normalises over all entities; sampled labels (num_labels) are "
+                                      "not supported - train with full 1-N labels (run_cpg --full-1n)")
         self.num_ent, self.num_rel = int(md["num_ent"]), int(md["num_rel"])
         self.ent_emb_size, self.rel_emb_size = int(md["ent_emb_size"]), int(md["rel_emb_size"])
         self.is_parameter_lookup = md.get("do_parameter_lookup", False)
@@ -765,6 +779,9 @@ class ConvE:
             dense = batch["e2_multi"]
             if not (isinstance(dense, torch.Tensor) and dense.is_cuda):
                 dense = torch.as_tensor(np.asarray(dense), dtype=torch.float32).to(self.dev, non_blocking=True)
+            if self.loss == "softmax_ce":         # global positive counts of the rows (not the shard's)
+                b.rowptr[0] = 0
+                b.rowptr[1:].copy_(torch.cumsum((dense != 0).sum(1), 0))
             if s.world > 1:
                 dense = dense[:, s.lo:s.hi].contiguous()
             dense = dense.contiguous()
@@ -1001,31 +1018,39 @@ class ConvE:
         self._side_pending = True
 
     def _scorer_backward(self, bg, b, inv_count):
-        """Scorer + BCE loss + dq / dE / dbias for the bg.B queries, then the entity-sharded scorer's exchange and the
-        mean loss.  Returns whether the relation gradient was cleared (on the side stream, for the scatter)."""
+        """Scorer + loss (BCE or softmax cross-entropy) + dq / dE / dbias for the bg.B queries, then the entity-sharded
+        scorer's exchange and the mean loss.  Returns whether the relation gradient was cleared (on the side stream, for
+        the scatter)."""
         g, Ns, d = self.grads, self.shard.rows, self.ent_emb_size
         rel_cleared = loss_done = False
+        ce = self.loss == "softmax_ce"
+        # the loss is a mean over B*N logits (BCE) or over B queries (CE)
+        loss_div = float(bg.B) if ce else float(bg.B) * float(self.num_ent)
+        if ce:
+            inv_count = 1.0 / float(bg.B)
+            fn, args = "coper_score1n_ce_fwd_bwd", self._ce_args(bg)
+        else:
+            fn = "coper_score1n_bce_fwd_bwd"
+            args = (ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
+                    ptr(bg.bits if self.prec == 0 else bg.bitsT), bg.B, Ns, d, self._pos, self._neg, inv_count)
         if self.use_negative_sampling:
             self._sampled_scorer(bg)
         elif self._norm_fused_now:
-            call("coper_score1n_bce_fwd_bwd_norm", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
-                 ptr(bg.bitsT), bg.B, Ns, d, self._pos, self._neg, inv_count, ptr(bg.loss_sum),
-                 ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), None, ptr(g["pred_bias"]), ptr(self.dE_sumsq), ptr(bg.ws),
-                 bg.ws_bytes, self.prec)
+            call(fn + "_norm", *args, ptr(bg.loss_sum), ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), None,
+                 ptr(g["pred_bias"]), ptr(self.dE_sumsq), ptr(bg.ws), bg.ws_bytes, self.prec)
+            ic_dE = _lib.load().coper_score1n_ce_dE_inv_count(inv_count, self.num_ent, self.prec) if ce else inv_count
             with self._on_side():
                 if self.rel_emb is not None:     # cleared here, off the main chain, for the scatter after the join
                     g["rel_emb"].zero_()
                     self.grad_sq["rel_emb"].zero_()
                     rel_cleared = True
-                call("coper_score1n_bce_dE", ptr(self._grad_buf(bg)), bg.B, Ns, d, inv_count, ptr(g["ent_emb"]),
+                call("coper_score1n_bce_dE", ptr(self._grad_buf(bg)), bg.B, Ns, d, ic_dE, ptr(g["ent_emb"]),
                      ptr(self.dE_sumsq), ptr(g["pred_bias"]), ptr(bg.ws), bg.ws_bytes, self.prec)
                 if self.world == 1:              # the mean loss the caller reads (models.py:451)
-                    torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
+                    torch.div(bg.loss_sum, loss_div, out=bg.loss_mean)
                     loss_done = True
         else:
-            call("coper_score1n_bce_fwd_bwd", ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias),
-                 ptr(bg.bits if self.prec == 0 else bg.bitsT), bg.B, Ns, d, self._pos, self._neg, inv_count,
-                 ptr(bg.loss_sum), ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), ptr(g["ent_emb"]),
+            call(fn, *args, ptr(bg.loss_sum), ptr(self._grad_buf(bg)), bg.ld, ptr(bg.dq), ptr(g["ent_emb"]),
                  ptr(g["pred_bias"]), ptr(bg.ws), bg.ws_bytes, self.prec)
         # entity-sharded scorer: every rank scored all B queries against its rows -> sum the partial loss and
         # the partial dq = G_shard . E_shard (SURVEY §8e step 4); dE / dbias stay local.
@@ -1034,8 +1059,19 @@ class ConvE:
         else:
             sharding.reduce_scorer_partials(b.loss_sum, b.dq, self.world, self.group)
         if not loss_done and not self.use_negative_sampling:
-            torch.div(bg.loss_sum, float(bg.B) * float(self.num_ent), out=bg.loss_mean)
+            torch.div(bg.loss_sum, loss_div, out=bg.loss_mean)
         return rel_cleared
+
+    def _ce_args(self, bg):
+        """Softmax cross-entropy: the log-sum-exp pass over this rank's rows, the exchange of the per-rank pairs and the
+        fixed-order finalise (bit-identical lse on every rank), then the CE call's leading arguments."""
+        Ns, d = self.shard.rows, self.ent_emb_size
+        head = (ptr(bg.q), ptr(self.ent_emb), ptr(self.E_prep), ptr(self.pred_bias))
+        call("coper_score1n_lse", *head, bg.B, Ns, d, ptr(bg.ml), ptr(bg.ws), bg.ws_bytes, self.prec)
+        parts = sharding.combine_lse(bg.ml, self.world, self.group, out=bg.ml_all)
+        call("coper_lse_finalize", ptr(parts), parts.shape[0], bg.B, ptr(bg.lse))
+        return head + (ptr(bg.bits if self.prec == 0 else bg.bitsT), ptr(bg.rowptr), ptr(bg.lse), bg.B, Ns, d,
+                       self.num_ent, self.label_smoothing_epsilon, 1.0 / float(bg.B))
 
     def _fc_backward(self, b):
         """FC block and CPG-FC backward, then the FC generators' context nets.  Returns the all-reduce of the big

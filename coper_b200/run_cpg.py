@@ -61,6 +61,8 @@ def model_name_of(cfg, model_descr, dataset_name, use_cpg, clean):
         cfg.context.context_rel_dropout)
     if use_cpg:
         name += "-context_batchnorm_{}".format(cfg.context.context_rel_use_batch_norm)
+    if cfg.model.get("loss", "bce") != "bce":
+        name += "-loss_{}".format(cfg.model.loss)
     if clean:
         name += "-CLEAN"
     return name
@@ -77,6 +79,9 @@ def main(argv=None):
     ap.add_argument("--full-1n", action="store_true", help="train with full 1-N labels (num_labels: null)")
     ap.add_argument("--device-sampling", action="store_true",
                     help="sampled-label configs: draw the [B, num_labels] ids / labels on the GPU (coper_sample_labels)")
+    ap.add_argument("--loss", default="bce", choices=["bce", "softmax_ce"],
+                    help="training objective: the reference's label-smoothed sigmoid BCE, or the softmax cross-entropy "
+                         "over all entities (needs full 1-N labels: --full-1n on a sampled-label config)")
     ap.add_argument("--max-steps", type=int, default=None)
     ap.add_argument("--eval-batches", type=int, default=None, help="cap the number of eval batches (synthetic runs)")
     ap.add_argument("--prec", default="fp16x3", choices=["fp32", "tf32x3", "fp16x3", "bf16"])
@@ -129,6 +134,11 @@ def main(argv=None):
     cfg = configs.load_config(args.config) if args.config else configs.load_config(dataset_name, args.model_type)
     if args.full_1n or args.synthetic:
         cfg.training.num_labels = None
+    if args.loss != "bce":
+        if cfg.training.get("num_labels") is not None:
+            ap.error("--loss %s normalises over all entities: this configuration samples num_labels = %s labels per "
+                     "query; add --full-1n" % (args.loss, cfg.training.num_labels))
+        cfg.model.loss = args.loss
     if args.max_steps is not None:
         cfg.training.max_steps = args.max_steps
 

@@ -9,6 +9,8 @@ collective on a tiny tensor; dE / dbias / optimizer state of the table never lea
 
   exchange_rows          all-reduce(sum) of the zero-masked [B, d] gather -> every rank has E[e1] exactly
   reduce_scorer_partials all-reduce(sum) of the partial loss (fp64) and the partial dq = G_shard . E_shard
+  combine_lse            all-gather of the per-shard log-sum-exp pairs [B, 2] (softmax cross-entropy): every rank then
+                         finalises the same lse over all entities (coper_lse_finalize, fixed order)
   reduce_sharded_sumsq   all-reduce(sum) of the squared-norm partials of the sharded gradients (global-norm clip)
   reduce_gold_and_counts all-reduce(sum) of the owner-provided gold logits, then of the integer rank counts
   gather_topk            all-gather of the per-shard top-k lists [B, k] (ConvE.predict_topk merges them on device)
@@ -125,6 +127,17 @@ def reduce_scorer_partials(loss_sum: torch.Tensor, dq: torch.Tensor, world: int,
         _all_reduce(loss_sum, group)
         _all_reduce(dq, group)
     return loss_sum, dq
+
+
+def combine_lse(ml: torch.Tensor, world: int, group=None, out=None) -> torch.Tensor:
+    """ml [B, 2]: (max, sum exp(s - max)) of every query over this rank's entity rows -> every rank's pairs [P, B, 2]
+    in rank order (``out``: optional [P, B, 2] buffer).  Without an active group: this rank's pairs, [1, B, 2]."""
+    if not _active(world, group):
+        return ml.unsqueeze(0)
+    if out is None:
+        out = ml.new_empty((dist.get_world_size(group),) + tuple(ml.shape))
+    _all_gather(out.view(-1, ml.shape[-1]), ml.contiguous(), group)
+    return out
 
 
 def reduce_sharded_sumsq(sumsq_sharded: torch.Tensor, world: int, group=None) -> torch.Tensor:

@@ -264,6 +264,47 @@ int coper_score1n_bce_fwd_bwd_norm(const float* q, const float* E, const void* E
 int coper_score1n_bce_dE(const void* G, int B, int64_t Ns, int d, float inv_count, float* dE, double* dE_sumsq,
                          float* dbias, void* workspace, size_t workspace_bytes, int prec, coper_stream_t stream);
 
+/* Softmax cross-entropy over all entities ("1vsAll" with one positive per row, "KvsAll-CE" with several): the opt-in
+ * second objective of the 1-N scorer (ConvE loss="softmax_ce").  Query b has the GLOBAL positive set P_b (the staged CSR
+ * row pointers: n_b = rowptr[b+1] - rowptr[b], never this shard's bits), eps = label smoothing, N = num_ent:
+ *   t_bn  = (1-eps) [n in P_b] / max(n_b, 1) + eps / N      (a distribution: sums to tau_b = eps + (1-eps) [n_b > 0])
+ *   lse_b = log sum_{n<N} exp(s_bn)                          (over every entity of every shard)
+ *   loss  = (1/B) sum_b sum_n t_bn (lse_b - s_bn)
+ *   G_bn  = (tau_b exp(s_bn - lse_b) - t_bn) / B             (exact dloss/ds, also for a row without positives)
+ * (The BCE objective smooths with +1/N on top of (1-eps), models.py:450; here the smoothing mass is eps/N so that the
+ * target stays a distribution.)
+ *   coper_score1n_lse: ml [B, 2] = (m_b, l_b) = (max_n s_bn, sum_n exp(s_bn - m_b)) over this rank's Ns rows; the
+ *       logits never leave the tensor memory / registers.  workspace: coper_score1n_lse_workspace_bytes (256-byte
+ *       aligned; 0 = unsupported precision).  Tensor-pipe engines: B <= 128 x the SM count (COPER_ERR_UNSUPPORTED);
+ *       their partials take 4 R B pairs (R <= SM count / ceil(B / 128)).  The fp32 engine keeps one pair per
+ *       (128-entity tile, query): ceil(Ns / 128) * B * 8 bytes (2.6 GB at Ns = 10 M, B = 4096), combined by one thread
+ *       per query - a parity path, not sized for the largest tables.
+ *   coper_lse_finalize: parts [P, B, 2] (every rank's ml, rank order) -> lse [B] = m + log sum_r l_r exp(m_r - m),
+ *       m = max_r m_r, in a fixed order with fp64 sums: every rank computes a bit-identical lse.  P = 1 on one GPU.
+ *   coper_score1n_ce_fwd_bwd(_norm): the BCE entry points' contract (label bits, G, ldG, workspace =
+ *       coper_score1n_bce_workspace_bytes, G bytes = coper_score1n_bce_G_bytes, E_prepared, dE == NULL split form) with
+ *       the CE loss: loss_sum = sum over this rank's rows of t (lse - s) (the caller divides by B), G = (tau exp(s - lse)
+ *       - t) * inv_count (inv_count = 1/B), dq = G.E, dE = G^T.q, dbias = sum_b G.  rowptr int32 [B + 1], lse [B] from
+ *       coper_lse_finalize.  Split form: then coper_score1n_bce_dE with inv_count = coper_score1n_ce_dE_inv_count
+ *       (inv_count, num_ent, prec) (fp16x3 carries G times 2^k, k = clamp(ceil(log2 num_ent), 10, 15); for num_ent
+ *       above ~2^18 the ~1/N entries still leave the lo plane in fp16 subnormals: ~1e-5 relative per element at 10 M
+ *       entities).  The bf16 engine runs the unfused scorer + dq GEMM (no single-kernel CE path). */
+size_t coper_score1n_lse_workspace_bytes(int B, int64_t Ns, int d, int prec);
+int coper_score1n_lse(const float* q, const float* E, const void* E_prepared, const float* bias, int B, int64_t Ns, int d,
+                      float* ml, void* workspace, size_t workspace_bytes, int prec, coper_stream_t stream);
+int coper_lse_finalize(const float* parts, int P, int B, float* lse, coper_stream_t stream);
+float coper_score1n_ce_dE_inv_count(float inv_count, int64_t num_ent, int prec);
+int coper_score1n_ce_fwd_bwd(const float* q, const float* E, const void* E_prepared, const float* bias,
+                             const uint32_t* label_bits, const int32_t* rowptr, const float* lse, int B, int64_t Ns, int d,
+                             int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G, int64_t ldG,
+                             float* dq, float* dE, float* dbias, void* workspace, size_t workspace_bytes, int prec,
+                             coper_stream_t stream);
+int coper_score1n_ce_fwd_bwd_norm(const float* q, const float* E, const void* E_prepared, const float* bias,
+                                  const uint32_t* label_bits, const int32_t* rowptr, const float* lse, int B, int64_t Ns,
+                                  int d, int64_t num_ent, float eps, float inv_count, double* loss_sum, void* G,
+                                  int64_t ldG, float* dq, float* dE, float* dbias, double* dE_sumsq, void* workspace,
+                                  size_t workspace_bytes, int prec, coper_stream_t stream);
+
 /* a8 / SURVEY §8f-2 — SAMPLED-label scorer (models.py:438-443), loss (:448-453) and gradients: what the shipped
  * big-dataset configs train with (training.num_labels = 100 / 1000).  lookup int32 [B, L] entity ids
  * (batch['lookup_values'], models.py:165), labels fp32 [B, L] (batch['e2_multi'] in sampled mode):
